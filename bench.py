@@ -2,6 +2,7 @@
 """bench.py — simplex pivots/sec and B&B nodes/sec on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload batched|large]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 A step is one pass of the hot path over one batch of synthetic input:
@@ -15,6 +16,13 @@ only provides the barrier and the max-over-ranks of the timings.
 
 --impl reference: the reference's own CPU implementation of the path.  The C# binary cannot run
 here (no .NET); the timed code is the C++ restatement in oracle/ on all host threads.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the timed path returned in its last step
+as DIR/<name>.npy (float64; int32 results are exact in it).  Inputs are seeded, so two builds run with
+the same arguments can be compared array for array.  batched: status, n_pivots, basis, x, z of every
+LP and the final tableaux of a fixed sample of DUMP_LPS LPs (`tableau`, their indices in
+`tableau_index`).  large: basis, x, z and the objective row plus a fixed sample of DUMP_ROWS rows of
+the tableau (`tableau`, `tableau_index`).
 """
 import argparse
 import json
@@ -35,6 +43,41 @@ BNB_INSTANCES = 512             # C4 instances per GPU in the bnb_simplex sectio
 KNAP_INSTANCES = 2368           # C5 instances per GPU in the bnb_knapsack section (16 per SM: one warp each)
 KNAP_INSTANCES_FRACTIONAL = 148
 POOLED = dict(seed=12, batch=4096)  # Mode B: one hard 60 x 120 instance (2.2e5 nodes), rounds of 4096 open nodes
+DUMP_LPS = 256                  # --dump-outputs: batched tableaux kept (26 MB of the 411 MB)
+DUMP_ROWS = 256                 # --dump-outputs: large-tableau constraint rows kept (25 MB of the 403 MB)
+DUMP_LIMIT = 64 << 20           # --dump-outputs: bytes written at most
+DUMP_SEED = 20261020            # the sample is the same in every run, so dumps compare element for element
+
+
+def sample_index(count, k):
+    """A fixed, seeded, sorted choice of k of range(count) (all of it when count <= k)."""
+    if count <= k:
+        return np.arange(count)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(count, k, replace=False))
+
+
+def dump_outputs(dirname, arrays):
+    """Each array as <dirname>/<name>.npy in float64."""
+    out = {k: np.ascontiguousarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in out.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes, more than {DUMP_LIMIT}")
+    os.makedirs(dirname, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(dirname, k + ".npy"), v)
+
+
+def dump_batched(dirname, res, tableaux):
+    """`res`: status, n_pivots, basis, x, z of every LP; `tableaux(idx)` returns the final tableaux of LPs idx."""
+    idx = sample_index(len(res["status"]), DUMP_LPS)
+    dump_outputs(dirname, dict(res, tableau=tableaux(idx), tableau_index=idx))
+
+
+def dump_large(dirname, T, basis, x, z):
+    """The large LP's state: basis, x, z, and the objective row plus DUMP_ROWS sampled constraint rows of T."""
+    m = T.shape[0] - 1
+    idx = np.append(sample_index(m, DUMP_ROWS), m)
+    dump_outputs(dirname, dict(basis=basis, x=x, z=[z], tableau=T[idx], tableau_index=idx))
 
 
 def load_peaks():
@@ -182,6 +225,11 @@ def run_reference(args):
         value = total / sum(times)
         used, sample = 1, f"{per_step} pivots per step of the 4096x8192 tableau (single tableau: one thread, as upstream)"
         cfg = {"workload": "C3 single large dense LP 4096x8192, window of pivots", **C3}
+        if args.dump_outputs:
+            x = np.zeros(n)
+            in_x = basis < n
+            x[basis[in_x]] = T[:m, -1][in_x]
+            dump_large(args.dump_outputs, T, basis, x, T[m, -1])
     else:
         A, b, c = workloads.batch_c2(**C2, seed=1)
         times, piv = [], 0
@@ -195,6 +243,9 @@ def run_reference(args):
         value = piv / sum(times)
         used, sample = cores, "full 4096-LP batch per step, arithmetic loop only (no per-iteration text formatting)"
         cfg = {"workload": "C2 batched dense LPs: 4096 x (64 constraints x 128 vars)", **C2}
+        if args.dump_outputs:
+            dump_batched(args.dump_outputs, {k: r[k] for k in ("status", "n_pivots", "basis", "x", "z")},
+                         lambda idx: r["tableau"][idx])
     line = {
         "impl": "reference", "metric": "simplex pivots/sec", "value": value, "unit": "pivots/s", "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * sum(times) / len(times),
@@ -266,7 +317,7 @@ def run_ours(args):
     sampler = ClockSampler(local_rank)
 
     # ---------------- config 3: large tableau (value when --workload large, else a section) ------
-    def bench_large(steps, warmup, per_step):
+    def bench_large(steps, warmup, per_step, dump=None):
         import ctypes as C
         A, b, c = workloads.large_c3(**C3, seed=7 + rank)
         dA, db, dc = (torch.from_numpy(v).to(dev) for v in (A, b, c))
@@ -301,6 +352,8 @@ def run_ours(args):
         done = per_step * steps
         if st != F.RUNNING:
             raise SystemExit(f"large LP finished early (status {st}) inside the timed window")
+        if dump:  # before lpx_session_profile, which pivots the session further
+            dump_large(dump, s.tableau(), *s.solution())
         # the two kernels of a block, timed separately with CUDA events on the session stream
         us = (C.c_double * 3)()
         F.lib().lpx_session_profile.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
@@ -330,7 +383,7 @@ def run_ours(args):
                                   "equivalent_GBs": per_pivot_equiv, "x_of_per_pivot_bound": per_pivot_equiv / hbm_peak}})
 
     # ---------------- config 2: batched --------------------------------------------------------
-    def bench_batched(steps, warmup):
+    def bench_batched(steps, warmup, dump=None):
         A, b, c = workloads.batch_c2(**C2, seed=1 + rank)
         count, m, n = A.shape
         rows, cols = m + 1, n + m + 1
@@ -414,6 +467,10 @@ def run_ours(args):
                         "unit": "GB/s", "algorithmic_bytes_per_launch": hbm_bytes, "peak_source": peak_kind,
                         "note": "inputs read once + final tableaux/x/basis written once; the tableau lives on-chip "
                                 "across all pivots, so this kernel is not HBM-bound"}}
+        if dump:  # the device buffers still hold the last timed step: the e2e calls have their own
+            res = dict(status=st, n_pivots=npv, basis=basis, x=x, z=z)
+            dump_batched(dump, {k: v.cpu().numpy() for k, v in res.items()},
+                         lambda idx: T[torch.from_numpy(idx).to(dev)].cpu().numpy())
         return dict(value=value, ms_per_step=total_ms / steps, launches=launches, clocks=clocks, pivots_per_step=pivots,
                     e2e={"value": e2e_value, "unit": "pivots/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
                          "ms_per_step": 1e3 * e2e_s / steps}, roofline=roof, host=(A, b, c))
@@ -602,9 +659,10 @@ def run_ours(args):
                 "host_cores_available": os.cpu_count(),
                 "note": "C++ restatement (oracle/) of the C# loops, not the C# binary (no .NET toolchain here)"}
 
+    dump = args.dump_outputs if rank == 0 else None
     if args.workload == "large":
         per_step = int(os.environ.get("LPX_BENCH_PERSTEP", "128"))
-        L = bench_large(args.steps, args.warmup, per_step)
+        L = bench_large(args.steps, args.warmup, per_step, dump)
         line = {"metric": "simplex pivots/sec", "value": L["value"], "unit": "pivots/s", "n_gpus": world,
                 "steps": args.steps, "warmup": args.warmup, "ms_per_step": L["ms_per_step"], "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
@@ -616,7 +674,7 @@ def run_ours(args):
                         "note": "the tableau is resident in HBM for the whole session; only 16 bytes of status "
                                 "cross PCIe per step"}}
     else:
-        Bm = bench_batched(args.steps, args.warmup)
+        Bm = bench_batched(args.steps, args.warmup, dump)
         host = Bm.pop("host")
         if not args.no_extras:
             try:
@@ -687,7 +745,10 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="batched", choices=["batched", "large"])
     ap.add_argument("--no-extras", action="store_true", help="skip the configs 3-5 sections")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     with OneJsonLine() as guard:
         line = run_reference(args) if args.impl == "reference" else run_ours(args)
