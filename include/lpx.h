@@ -284,6 +284,43 @@ int lpx_revised_solve(int m, int n, int sense, const double* A, const int* rel, 
                       int history_cap);
 size_t lpx_revised_history_stride(int m, int n);
 
+/* ---- Sensitivity analysis of an optimal Primal Simplex result — NOT the reference's ---------------------- */
+/* The reference's SensitivityAnalysis reads the objective row as tableau row 0, while its PrimalSimplex and this
+ * engine put the z-row last, so this report is defined here and checked against oracle/orc_sensitivity.cpp bit for
+ * bit and against an independent LP solver.  Input: the final tableau of a Primal Simplex solve with status
+ * LPX_OPTIMAL (m' rows after EQ expansion, W = n + m' + 1 columns), its basis, and the model's sense, rel, b, c.
+ * EPS = 1e-9.  The slack of constraint i is column n + i1 of its expanded row i1; an EQ row i expands to rows i1
+ * (a.x <= b) and i2 = i1 + 1 (-a.x <= -b).  z = T[m'], beta_r = T[r][W-1]; "non-basic" = not listed in basis.
+ *   shadow[i]  = T[m'][n+i1]  (EQ: T[m'][n+i1] - T[m'][n+i2]), negated for Min: d(objective as written)/d b_i.
+ *                (z itself stays as the solve returns it, the maximum of -c.x for Min.)
+ *   slack[i]   = beta_r if slack column n+i1 is basic in row r, else +0.
+ *   rhs range  : g = column n+i1 (EQ: column n+i1 minus column n+i2), q_r = beta_r / g_r;
+ *                lo = b_i + max{-q_r : g_r > EPS}, hi = b_i + min{-q_r : g_r < -EPS}; an empty side is -inf / +inf.
+ *   reduced[j] = T[m'][j] (>= 0 at an optimum for both senses).
+ *   cost range : non-basic j: Max (-inf, c_j + d_j], Min [c_j - d_j, +inf).  Basic j in row r, over non-basic
+ *                columns k < W-1 with alpha = T[r][k]: dlo = max{-(d_k/alpha) : alpha > EPS},
+ *                dhi = min{-(d_k/alpha) : alpha < -EPS}; Max [c_j + dlo, c_j + dhi], Min [c_j - dhi, c_j - dlo].
+ * Ties in every max / min: -0.0 equals +0.0 and the lowest row / column index wins (its own value is used).
+ * Instances whose status is not LPX_OPTIMAL get a record of NaNs.
+ * Scope: results of the Primal Simplex entry points.  GE rows never reach OPTIMAL there; lpx_dual_solve results are
+ * excluded, because that solver treats a.x >= b (b > 0) as a.x <= b and its tableau does not describe the model.
+ * One record per LP, lpx_sensitivity_stride(m, n) = 4m + 3n doubles:
+ *   shadow[m] | slack[m] | rhs_lo[m] | rhs_hi[m] | reduced[n] | cost_lo[n] | cost_hi[n]  */
+size_t lpx_sensitivity_stride(int m, int n);
+/* From final tableaux already on the device: the outputs of lpx_primal_solve_batched_dev, same pointer
+ * conventions (all device pointers, rel included), asynchronous on `stream`.  report: count x stride. */
+int lpx_sensitivity_batched_dev(int count, int m, int n, int sense, const int* rel, const double* b, const double* c,
+                                const int* status, const int* basis, const double* tableau, double* report, void* stream);
+/* Host buffers: lpx_primal_solve_batched plus the reports (count x stride); any output but status and report may
+ * be NULL.  The tableaux stay on the device: nothing but status / n_pivots / basis / x / z / report crosses PCIe. */
+int lpx_primal_solve_sensitivity_batched(int count, int m, int n, int sense, const double* A, const int* rel,
+                                         const double* b, const double* c, const lpx_options* opt, int* status,
+                                         int* n_pivots, int* basis, double* x, double* z, double* report,
+                                         long long* total_pivots);
+/* Large LP whose tableau lives in HBM; report is a host buffer of one stride (NaNs unless the session's status,
+ * as of its last step / sync, is LPX_OPTIMAL). */
+int lpx_session_sensitivity(lpx_session* s, double* report);
+
 /* ---- measurement helpers (bench.py) --------------------------------------------------------- */
 /* Unfused FP64 rate (separate DMUL and DADD, the only arithmetic the bit-exactness contract
  * allows) in TFLOP/s: the roofline denominator of the on-chip batched kernels. */

@@ -30,7 +30,8 @@ EXPORTS = [
     "lpx_bnb_knapsack_batched", "lpx_comm_unique_id", "lpx_comm_init", "lpx_comm_allreduce_max",
     "lpx_comm_allgather", "lpx_comm_destroy", "lpx_comm_world", "lpx_comm_rank", "lpx_kernel_launches",
     "lpx_reset_counters", "lpx_revised_solve", "lpx_revised_history_stride", "lpx_measure_fp64_rate", "lpx_measure_latencies", "lpx_session_profile", "lpx_session_debug_stamps",
-    "lpx_bnb_last_stats", "lpx_bnb_pooled",
+    "lpx_bnb_last_stats", "lpx_bnb_pooled", "lpx_sensitivity_stride", "lpx_sensitivity_batched_dev",
+    "lpx_primal_solve_sensitivity_batched", "lpx_session_sensitivity",
 ]
 
 
@@ -128,6 +129,11 @@ def lib():
                                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                C.c_void_p]
+    L.lpx_sensitivity_stride.restype = C.c_size_t
+    L.lpx_sensitivity_stride.argtypes = [C.c_int, C.c_int]
+    L.lpx_sensitivity_batched_dev.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 8
+    L.lpx_primal_solve_sensitivity_batched.argtypes = L.lpx_primal_solve_batched.argtypes
+    L.lpx_session_sensitivity.argtypes = [C.c_void_p, C.c_void_p]
     L.lpx_bnb_simplex_batched.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]

@@ -137,6 +137,55 @@ def primal_solve_batched_dev(count, m, n, sense, dA, drel, db, dc, dstatus, dnpi
     F.check(rc)
 
 
+SENSITIVITY_FIELDS = ("shadow", "slack", "rhs_lo", "rhs_hi", "reduced", "cost_lo", "cost_hi")
+
+
+def sensitivity_stride(m, n):
+    return int(F.lib().lpx_sensitivity_stride(m, n))
+
+
+def split_sensitivity(report, m, n):
+    """Named views of sensitivity records (include/lpx.h): shadow, slack, rhs_lo, rhs_hi (m each), reduced,
+    cost_lo, cost_hi (n each); `report` is one record or (count, stride)."""
+    out, o = {}, 0
+    for name, k in zip(SENSITIVITY_FIELDS, (m, m, m, m, n, n, n)):
+        out[name] = report[..., o:o + k]
+        o += k
+    return out
+
+
+def primal_solve_sensitivity_batched(A, b, c, rel=None, sense=0, max_iterations=10000, kernel=F.KERNEL_AUTO,
+                                     threads=0, reg_variant=0):
+    """primal_solve_batched without the tableaux, plus the sensitivity report of every OPTIMAL instance
+    (NaN records for the others), computed on the GPU next to the tableaux: `report` (count, 4m + 3n) and its
+    named (count, .) views."""
+    A, b, c, rel = _prep(A, b, c, rel)
+    count, m, n = A.shape
+    rows, _ = tableau_dims(m, n, rel)
+    opt = F.make_options(max_iterations, kernel, threads, reg_variant=reg_variant)
+    status = np.zeros(count, dtype=np.int32)
+    npiv = np.zeros(count, dtype=np.int32)
+    basis = np.zeros((count, rows - 1), dtype=np.int32)
+    x = np.zeros((count, n))
+    z = np.zeros(count)
+    report = np.zeros((count, sensitivity_stride(m, n)))
+    total = C.c_longlong()
+    rc = F.lib().lpx_primal_solve_sensitivity_batched(count, m, n, sense, F.ptr(A), F.ptr(rel), F.ptr(b), F.ptr(c),
+                                                      C.byref(opt), F.ptr(status), F.ptr(npiv), F.ptr(basis),
+                                                      F.ptr(x), F.ptr(z), F.ptr(report), C.byref(total))
+    F.check(rc)
+    return dict(status=status, n_pivots=npiv, basis=basis, x=x, z=z, total_pivots=total.value, report=report,
+                **split_sensitivity(report, m, n))
+
+
+def sensitivity_batched_dev(count, m, n, sense, drel, db, dc, dstatus, dbasis, dtableau, dreport, stream):
+    """lpx_sensitivity_batched_dev on the outputs of primal_solve_batched_dev: raw device pointers (ints),
+    asynchronous on `stream`; dreport receives count x sensitivity_stride(m, n) doubles."""
+    rc = F.lib().lpx_sensitivity_batched_dev(count, m, n, sense, F.ptr(drel), F.ptr(db), F.ptr(dc), F.ptr(dstatus),
+                                             F.ptr(dbasis), F.ptr(dtableau), F.ptr(dreport), F.ptr(stream or 0))
+    F.check(rc)
+
+
 class Session:
     """Large single LP whose tableau lives in HBM (lpx_session_*)."""
 
@@ -188,6 +237,13 @@ class Session:
         z = C.c_double()
         F.check(F.lib().lpx_session_read_solution(self._h, F.ptr(basis), F.ptr(x), C.cast(C.byref(z), C.c_void_p)))
         return basis, x, z.value
+
+    def sensitivity(self):
+        """Sensitivity report of the session's tableau (NaNs unless its status is OPTIMAL): `report` and its
+        named views."""
+        rep = np.zeros(sensitivity_stride(self.m, self.n))
+        F.check(F.lib().lpx_session_sensitivity(self._h, F.ptr(rep)))
+        return dict(report=rep, **split_sensitivity(rep, self.m, self.n))
 
     def pivots(self, cap):
         p = np.full((max(cap, 1), 2), -1, dtype=np.int32)

@@ -87,6 +87,19 @@ namespace Linear_Programming_Solver.Models
             int[] basis, int[] nonbasic, double[] xB, double[] Binv, double[] x, double[] history, int history_cap);
         [DllImport(Lib)] public static extern UIntPtr lpx_revised_history_stride(int m, int n);
 
+        // Sensitivity report of optimal Primal Simplex results (include/lpx.h; not the reference's SensitivityAnalysis,
+        // which reads the z-row from tableau row 0): lpx_sensitivity_stride doubles per LP,
+        // shadow[m] | slack[m] | rhs_lo[m] | rhs_hi[m] | reduced[n] | cost_lo[n] | cost_hi[n], NaNs unless OPTIMAL.
+        [DllImport(Lib)] public static extern UIntPtr lpx_sensitivity_stride(int m, int n);
+        [DllImport(Lib)]
+        public static extern int lpx_sensitivity_batched_dev(int count, int m, int n, int sense, IntPtr rel, IntPtr b,
+            IntPtr c, IntPtr status, IntPtr basis, IntPtr tableau, IntPtr report, IntPtr stream);
+        [DllImport(Lib)]
+        public static extern int lpx_primal_solve_sensitivity_batched(int count, int m, int n, int sense, double[] A,
+            int[] rel, double[] b, double[] c, ref LpxOptions opt, int[] status, int[] n_pivots, int[] basis,
+            double[] x, double[] z, double[] report, out long total_pivots);
+        [DllImport(Lib)] public static extern int lpx_session_sensitivity(IntPtr session, double[] report);
+
         [DllImport(Lib)]
         public static extern int lpx_primal_solve_batched(int count, int m, int n, int sense, double[] A, int[] rel,
             double[] b, double[] c, ref LpxOptions opt, int[] status, int[] n_pivots, int[] basis, double[] x,

@@ -318,6 +318,116 @@ static int batched_dev_launch(int count, int m, int n, int sense, const double* 
     return cta_launch(B, count, o.kernel, o.threads, stream, nullptr);
 }
 
+// lpx_primal_solve_batched(_sensitivity): host buffers through a three-stream chunk pipeline.  report (nullable):
+// the sensitivity records, computed per chunk on the compute stream from the chunk's tableaux, which then stay
+// in a device workspace unless `tableau` asks for them too.
+static int primal_batched_pipeline(int count, int m, int n, int sense, const double* A, const int* rel,
+                                   const double* b, const double* c, const lpx_options* opt, int* status,
+                                   int* n_pivots, int* basis, double* x, double* z, double* tableau, double* report,
+                                   long long* total_pivots) {
+    int rc = check_problem(m, n, sense, A, rel, b, c);
+    if (rc != LPX_OK) return rc;
+    if ((rc = ensure_device()) != LPX_OK) return rc;
+    Runtime& r = rt();
+    std::lock_guard<std::recursive_mutex> lk(r.mu);
+    if (total_pivots) *total_pivots = 0;
+    if (count == 0) return LPX_OK;
+    const int mm = expanded_rows(m, rel);
+    const size_t tsize = (size_t)(mm + 1) * (n + mm + 1);
+    const size_t cnt = (size_t)count;
+
+    double* dA = ws_dev_as<double>(WS_A, cnt * m * n);
+    double* db = ws_dev_as<double>(WS_B, cnt * m);
+    double* dc = ws_dev_as<double>(WS_C, cnt * n);
+    int* drel = ws_dev_as<int>(WS_REL, m);
+    int* dstat = ws_dev_as<int>(WS_STATUS, cnt);
+    int* dnp = ws_dev_as<int>(WS_NPIV, cnt);
+    int* dbasis = ws_dev_as<int>(WS_BASIS, cnt * mm);
+    double* dx = ws_dev_as<double>(WS_X, cnt * n);
+    double* dz = ws_dev_as<double>(WS_Z, cnt);
+    double* dT = (tableau || report) ? ws_dev_as<double>(WS_TABLEAU, cnt * tsize) : nullptr;
+    const size_t rstride = lpx_sensitivity_stride(m, n);
+    double* dR = report ? ws_dev_as<double>(WS_SENS, cnt * rstride) : nullptr;
+    unsigned long long* dtot = ws_dev_as<unsigned long long>(WS_TOTAL, 1);
+    if (!dA || !db || !dc || !drel || !dstat || !dnp || !dbasis || !dx || !dz || ((tableau || report) && !dT) ||
+        (report && !dR) || !dtot)
+        return LPX_E_CUDA;
+    if (rel) LPX_CUDA(cudaMemcpyAsync(drel, rel, (size_t)m * 4, cudaMemcpyHostToDevice, r.h2d));
+    LPX_CUDA(cudaMemsetAsync(dtot, 0, 8, r.h2d));
+
+    // Three-stage pipeline over chunks of the batch: H2D | solve | D2H on three streams, so that
+    // PCIe traffic in both directions overlaps the kernels.  The result copy is the long pole (the
+    // tableaux are 1.5x the inputs), so large batches ramp the chunk size up — 1, 2, 4, 5, 5, ... 32nds —
+    // and the first results start down the link after a 32nd of the upload instead of an 8th.
+    const int chunks = count >= 1024 ? 8 : (count >= 64 ? 4 : 1);
+    static const int ramp[9] = {0, 1, 3, 7, 12, 17, 22, 27, 32};
+    auto bound = [&](int k) -> size_t { return chunks == 8 ? cnt * ramp[k] / 32 : cnt * k / chunks; };
+    struct Events {  // destroyed on every return path, the LPX_CUDA early returns included
+        std::vector<cudaEvent_t> ev;
+        ~Events() {
+            for (cudaEvent_t e : ev) cudaEventDestroy(e);
+        }
+        int add(cudaEvent_t* out) {
+            LPX_CUDA(cudaEventCreateWithFlags(out, cudaEventDisableTiming));
+            ev.push_back(*out);
+            return LPX_OK;
+        }
+    } events;
+    std::vector<cudaEvent_t> up(chunks), done(chunks);
+    for (int k = 0; k < chunks; k++) {
+        if ((rc = events.add(&up[k])) != LPX_OK) return rc;
+        if ((rc = events.add(&done[k])) != LPX_OK) return rc;
+    }
+    lpx_options o;
+    lpx_default_options(&o);
+    if (opt) o = *opt;
+    bool all_le = true;
+    if (rel)
+        for (int i = 0; i < m; i++) all_le = all_le && rel[i] == 0;
+    int result = LPX_OK;
+    for (int k = 0; k < chunks && result == LPX_OK; k++) {
+        const size_t lo = bound(k), hi = bound(k + 1), len = hi - lo;
+        if (len == 0) continue;
+        LPX_CUDA(cudaMemcpyAsync(dA + lo * m * n, A + lo * m * n, len * m * n * 8, cudaMemcpyHostToDevice, r.h2d));
+        LPX_CUDA(cudaMemcpyAsync(db + lo * m, b + lo * m, len * m * 8, cudaMemcpyHostToDevice, r.h2d));
+        LPX_CUDA(cudaMemcpyAsync(dc + lo * n, c + lo * n, len * n * 8, cudaMemcpyHostToDevice, r.h2d));
+        LPX_CUDA(cudaEventRecord(up[k], r.h2d));
+        LPX_CUDA(cudaStreamWaitEvent(r.stream, up[k], 0));
+        result = batched_dev_launch((int)len, m, n, sense, dA + lo * m * n, rel ? drel : nullptr, mm, all_le, db + lo * m,
+                                    dc + lo * n, o, dstat + lo, dnp + lo, dbasis + lo * mm, dx + lo * n, dz + lo,
+                                    dT ? dT + lo * tsize : nullptr, dtot, r.stream);
+        if (result == LPX_OK && report)
+            result = sens_launch_batched((int)len, m, n, mm, sense, rel ? drel : nullptr, db + lo * m, dc + lo * n,
+                                         dstat + lo, dbasis + lo * mm, dT + lo * tsize, dR + lo * rstride, r.stream);
+        if (result != LPX_OK) break;
+        LPX_CUDA(cudaEventRecord(done[k], r.stream));
+        LPX_CUDA(cudaStreamWaitEvent(r.d2h, done[k], 0));
+        LPX_CUDA(cudaMemcpyAsync(status + lo, dstat + lo, len * 4, cudaMemcpyDeviceToHost, r.d2h));
+        if (n_pivots) LPX_CUDA(cudaMemcpyAsync(n_pivots + lo, dnp + lo, len * 4, cudaMemcpyDeviceToHost, r.d2h));
+        if (basis)
+            LPX_CUDA(cudaMemcpyAsync(basis + lo * mm, dbasis + lo * mm, len * mm * 4, cudaMemcpyDeviceToHost, r.d2h));
+        if (x) LPX_CUDA(cudaMemcpyAsync(x + lo * n, dx + lo * n, len * n * 8, cudaMemcpyDeviceToHost, r.d2h));
+        if (z) LPX_CUDA(cudaMemcpyAsync(z + lo, dz + lo, len * 8, cudaMemcpyDeviceToHost, r.d2h));
+        if (tableau)
+            LPX_CUDA(cudaMemcpyAsync(tableau + lo * tsize, dT + lo * tsize, len * tsize * 8, cudaMemcpyDeviceToHost,
+                                     r.d2h));
+        if (report)
+            LPX_CUDA(cudaMemcpyAsync(report + lo * rstride, dR + lo * rstride, len * rstride * 8, cudaMemcpyDeviceToHost,
+                                     r.d2h));
+    }
+    unsigned long long htot = 0;
+    if (result == LPX_OK) {
+        cudaError_t e = cudaStreamSynchronize(r.stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(&htot, dtot, 8, cudaMemcpyDeviceToHost, r.d2h);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(r.d2h);
+        if (e != cudaSuccess) result = cuda_fail(e, "batched pipeline sync", __FILE__, __LINE__);
+    } else {
+        cudaDeviceSynchronize();
+    }
+    if (total_pivots) *total_pivots = (long long)htot;
+    return result;
+}
+
 }  // namespace lpx
 
 using namespace lpx;
@@ -408,98 +518,20 @@ int lpx_primal_solve_batched(int count, int m, int n, int sense, const double* A
         set_error("lpx_primal_solve_batched: bad arguments");
         return LPX_E_BAD_ARGS;
     }
-    int rc = check_problem(m, n, sense, A, rel, b, c);
-    if (rc != LPX_OK) return rc;
-    if ((rc = ensure_device()) != LPX_OK) return rc;
-    Runtime& r = rt();
-    std::lock_guard<std::recursive_mutex> lk(r.mu);
-    if (total_pivots) *total_pivots = 0;
-    if (count == 0) return LPX_OK;
-    const int mm = expanded_rows(m, rel);
-    const size_t tsize = (size_t)(mm + 1) * (n + mm + 1);
-    const size_t cnt = (size_t)count;
+    return primal_batched_pipeline(count, m, n, sense, A, rel, b, c, opt, status, n_pivots, basis, x, z, tableau, nullptr,
+                                   total_pivots);
+}
 
-    double* dA = ws_dev_as<double>(WS_A, cnt * m * n);
-    double* db = ws_dev_as<double>(WS_B, cnt * m);
-    double* dc = ws_dev_as<double>(WS_C, cnt * n);
-    int* drel = ws_dev_as<int>(WS_REL, m);
-    int* dstat = ws_dev_as<int>(WS_STATUS, cnt);
-    int* dnp = ws_dev_as<int>(WS_NPIV, cnt);
-    int* dbasis = ws_dev_as<int>(WS_BASIS, cnt * mm);
-    double* dx = ws_dev_as<double>(WS_X, cnt * n);
-    double* dz = ws_dev_as<double>(WS_Z, cnt);
-    double* dT = tableau ? ws_dev_as<double>(WS_TABLEAU, cnt * tsize) : nullptr;
-    unsigned long long* dtot = ws_dev_as<unsigned long long>(WS_TOTAL, 1);
-    if (!dA || !db || !dc || !drel || !dstat || !dnp || !dbasis || !dx || !dz || (tableau && !dT) || !dtot)
-        return LPX_E_CUDA;
-    if (rel) LPX_CUDA(cudaMemcpyAsync(drel, rel, (size_t)m * 4, cudaMemcpyHostToDevice, r.h2d));
-    LPX_CUDA(cudaMemsetAsync(dtot, 0, 8, r.h2d));
-
-    // Three-stage pipeline over chunks of the batch: H2D | solve | D2H on three streams, so that
-    // PCIe traffic in both directions overlaps the kernels.  The result copy is the long pole (the
-    // tableaux are 1.5x the inputs), so large batches ramp the chunk size up — 1, 2, 4, 5, 5, ... 32nds —
-    // and the first results start down the link after a 32nd of the upload instead of an 8th.
-    const int chunks = count >= 1024 ? 8 : (count >= 64 ? 4 : 1);
-    static const int ramp[9] = {0, 1, 3, 7, 12, 17, 22, 27, 32};
-    auto bound = [&](int k) -> size_t { return chunks == 8 ? cnt * ramp[k] / 32 : cnt * k / chunks; };
-    struct Events {  // destroyed on every return path, the LPX_CUDA early returns included
-        std::vector<cudaEvent_t> ev;
-        ~Events() {
-            for (cudaEvent_t e : ev) cudaEventDestroy(e);
-        }
-        int add(cudaEvent_t* out) {
-            LPX_CUDA(cudaEventCreateWithFlags(out, cudaEventDisableTiming));
-            ev.push_back(*out);
-            return LPX_OK;
-        }
-    } events;
-    std::vector<cudaEvent_t> up(chunks), done(chunks);
-    for (int k = 0; k < chunks; k++) {
-        if ((rc = events.add(&up[k])) != LPX_OK) return rc;
-        if ((rc = events.add(&done[k])) != LPX_OK) return rc;
+int lpx_primal_solve_sensitivity_batched(int count, int m, int n, int sense, const double* A, const int* rel,
+                                         const double* b, const double* c, const lpx_options* opt, int* status,
+                                         int* n_pivots, int* basis, double* x, double* z, double* report,
+                                         long long* total_pivots) {
+    if (count < 0 || !status || !report) {
+        set_error("lpx_primal_solve_sensitivity_batched: bad arguments");
+        return LPX_E_BAD_ARGS;
     }
-    lpx_options o;
-    lpx_default_options(&o);
-    if (opt) o = *opt;
-    bool all_le = true;
-    if (rel)
-        for (int i = 0; i < m; i++) all_le = all_le && rel[i] == 0;
-    int result = LPX_OK;
-    for (int k = 0; k < chunks && result == LPX_OK; k++) {
-        const size_t lo = bound(k), hi = bound(k + 1), len = hi - lo;
-        if (len == 0) continue;
-        LPX_CUDA(cudaMemcpyAsync(dA + lo * m * n, A + lo * m * n, len * m * n * 8, cudaMemcpyHostToDevice, r.h2d));
-        LPX_CUDA(cudaMemcpyAsync(db + lo * m, b + lo * m, len * m * 8, cudaMemcpyHostToDevice, r.h2d));
-        LPX_CUDA(cudaMemcpyAsync(dc + lo * n, c + lo * n, len * n * 8, cudaMemcpyHostToDevice, r.h2d));
-        LPX_CUDA(cudaEventRecord(up[k], r.h2d));
-        LPX_CUDA(cudaStreamWaitEvent(r.stream, up[k], 0));
-        result = batched_dev_launch((int)len, m, n, sense, dA + lo * m * n, rel ? drel : nullptr, mm, all_le, db + lo * m,
-                                    dc + lo * n, o, dstat + lo, dnp + lo, dbasis + lo * mm, dx + lo * n, dz + lo,
-                                    dT ? dT + lo * tsize : nullptr, dtot, r.stream);
-        if (result != LPX_OK) break;
-        LPX_CUDA(cudaEventRecord(done[k], r.stream));
-        LPX_CUDA(cudaStreamWaitEvent(r.d2h, done[k], 0));
-        LPX_CUDA(cudaMemcpyAsync(status + lo, dstat + lo, len * 4, cudaMemcpyDeviceToHost, r.d2h));
-        if (n_pivots) LPX_CUDA(cudaMemcpyAsync(n_pivots + lo, dnp + lo, len * 4, cudaMemcpyDeviceToHost, r.d2h));
-        if (basis)
-            LPX_CUDA(cudaMemcpyAsync(basis + lo * mm, dbasis + lo * mm, len * mm * 4, cudaMemcpyDeviceToHost, r.d2h));
-        if (x) LPX_CUDA(cudaMemcpyAsync(x + lo * n, dx + lo * n, len * n * 8, cudaMemcpyDeviceToHost, r.d2h));
-        if (z) LPX_CUDA(cudaMemcpyAsync(z + lo, dz + lo, len * 8, cudaMemcpyDeviceToHost, r.d2h));
-        if (tableau)
-            LPX_CUDA(cudaMemcpyAsync(tableau + lo * tsize, dT + lo * tsize, len * tsize * 8, cudaMemcpyDeviceToHost,
-                                     r.d2h));
-    }
-    unsigned long long htot = 0;
-    if (result == LPX_OK) {
-        cudaError_t e = cudaStreamSynchronize(r.stream);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(&htot, dtot, 8, cudaMemcpyDeviceToHost, r.d2h);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(r.d2h);
-        if (e != cudaSuccess) result = cuda_fail(e, "batched pipeline sync", __FILE__, __LINE__);
-    } else {
-        cudaDeviceSynchronize();
-    }
-    if (total_pivots) *total_pivots = (long long)htot;
-    return result;
+    return primal_batched_pipeline(count, m, n, sense, A, rel, b, c, opt, status, n_pivots, basis, x, z, nullptr, report,
+                                   total_pivots);
 }
 
 }  // extern "C"

@@ -17,6 +17,7 @@ enum Slot {
     WS_HISTORY, WS_NHIST, WS_SCRATCH, WS_TOTAL, WS_NODE_INST, WS_NODE_OFF, WS_NODE_CNT, WS_NODE_MODE, WS_EX_VAR,
     WS_EX_REL, WS_EX_RHS, WS_KN_ITEMS, WS_KN_ASSIGN, WS_KN_OUT, WS_KN_AUX, WS_KN_EXACT, WS_MISC0, WS_MISC1, WS_MISC2,
     WS_PL_IN, WS_PL_OUT, WS_PL_ALL,  // pooled-tree B&B: node descriptors, own results, everybody's results
+    WS_SENS,  // sensitivity reports of lpx_primal_solve_sensitivity_batched
     WS_BB_SET0,  // pipelined B&B: descriptors, results, scratch of each of LPX_BB_SETS evaluation sets
     WS_COUNT = WS_BB_SET0 + 3 * 4
 };

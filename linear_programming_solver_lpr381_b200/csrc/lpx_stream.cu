@@ -14,6 +14,7 @@
 // row starts on a 128-byte line and double2 accesses are aligned; pad columns hold zeros.
 #include <algorithm>
 #include <cstring>
+#include <limits>
 #include <vector>
 
 #include "lpx_common.cuh"
@@ -487,8 +488,15 @@ struct lpx_session {
     lpx_options opt{};
     cudaStream_t stream = nullptr;
     bool own_stream = false;
-    void* buffers[24] = {};
+    void* buffers[32] = {};
     int nbuf = 0;
+    // sensitivity report: copies of b and c, the constraint -> slack row map, and (on first use) the work buffers
+    double* sens_b = nullptr;
+    double* sens_c = nullptr;
+    int* sens_rmap = nullptr;
+    int* sens_rowof = nullptr;
+    void* sens_partial = nullptr;
+    double* sens_report = nullptr;
     dim3 grid_update;
     dim3 grid_block;
     bool la_cluster = false;  // look-ahead on a thread-block cluster (else one CTA)
@@ -693,11 +701,12 @@ static lpx_session* session_create(int m, int n, int sense, const double* dA, co
     s->own_stream = true;
 
     // row map of the EQ expansion, and the first '>=' row, both known from rel on the host
-    std::vector<int> rsrc, rsgn;
+    std::vector<int> rsrc, rsgn, rmap;
     int first_ge = INT_MAX;
     for (int r = 0; r < m; r++) {
         const int rl = rel ? rel[r] : 0;
         if (rl == 1 && first_ge == INT_MAX) first_ge = r;
+        rmap.push_back(rl == 2 ? -(int)rsrc.size() - 1 : (int)rsrc.size());
         rsrc.push_back(r);
         rsgn.push_back(0);
         if (rl == 2) {
@@ -805,8 +814,11 @@ static lpx_session* session_create(int m, int n, int sense, const double* dA, co
         P.npartial = 0;
     int* drsrc = (int*)sess_alloc(s, (size_t)mm * 4);
     int* drsgn = (int*)sess_alloc(s, (size_t)mm * 4);
+    s->sens_b = (double*)sess_alloc(s, (size_t)m * 8);
+    s->sens_c = (double*)sess_alloc(s, (size_t)n * 8);
+    s->sens_rmap = (int*)sess_alloc(s, (size_t)m * 4);
     if (!P.T || !P.colbuf || !P.rhsbuf || !P.prow || !P.ratio || !P.basis || !P.pivlog || !P.ctl || !P.partial || !P.Fbuf ||
-        !P.Pbuf || !P.Lbuf || !drsrc || !drsgn) {
+        !P.Pbuf || !P.Lbuf || !drsrc || !drsgn || !s->sens_b || !s->sens_c || !s->sens_rmap) {
         sess_free(s);
         return nullptr;
     }
@@ -814,6 +826,9 @@ static lpx_session* session_create(int m, int n, int sense, const double* dA, co
     bool ok = true;
     ok = ok && cudaMemcpyAsync(drsrc, rsrc.data(), (size_t)mm * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
     ok = ok && cudaMemcpyAsync(drsgn, rsgn.data(), (size_t)mm * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(s->sens_b, db, (size_t)m * 8, cudaMemcpyDeviceToDevice, st) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(s->sens_c, dc, (size_t)n * 8, cudaMemcpyDeviceToDevice, st) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(s->sens_rmap, rmap.data(), (size_t)m * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
     ok = ok && cudaMemsetAsync(P.colbuf, 0, (size_t)2 * P.colstride * 8, st) == cudaSuccess;
     ok = ok && cudaMemsetAsync(P.rhsbuf, 0, (size_t)P.colstride * 8, st) == cudaSuccess;
     if (ok) {
@@ -1083,6 +1098,40 @@ int lpx_session_read_tableau(lpx_session* s, double* tableau) {
     }
     LPX_CUDA(cudaMemcpy2DAsync(tableau, (size_t)s->P.width * 8, Tcur, (size_t)s->P.ld * 8, (size_t)s->P.width * 8,
                                s->P.rows, cudaMemcpyDeviceToHost, s->stream));
+    LPX_CUDA(cudaStreamSynchronize(s->stream));
+    return LPX_OK;
+}
+
+int lpx_session_sensitivity(lpx_session* s, double* report) {
+    if (!s || !report) {
+        set_error("lpx_session_sensitivity: bad arguments");
+        return LPX_E_BAD_ARGS;
+    }
+    std::lock_guard<std::recursive_mutex> lk(rt().mu);
+    const StreamParams& P = s->P;
+    const size_t stride = lpx_sensitivity_stride(s->m_in, s->n);
+    StreamCtl h;
+    LPX_CUDA(cudaMemcpyAsync(&h, P.ctl, sizeof h, cudaMemcpyDeviceToHost, s->stream));
+    LPX_CUDA(cudaStreamSynchronize(s->stream));
+    if (h.status != LPX_OPTIMAL) {
+        for (size_t e = 0; e < stride; e++) report[e] = std::numeric_limits<double>::quiet_NaN();
+        return LPX_OK;
+    }
+    if (!s->sens_report) {
+        s->sens_rowof = (int*)sess_alloc(s, (size_t)P.width * 4);
+        s->sens_partial = sess_alloc(s, sens_session_partial_bytes(s->m_in, P.m));
+        s->sens_report = (double*)sess_alloc(s, stride * 8);
+        if (!s->sens_rowof || !s->sens_partial || !s->sens_report) {
+            s->sens_report = nullptr;
+            return LPX_E_CUDA;
+        }
+    }
+    // the live tableau, as lpx_session_read_tableau finds it: z-row and RHS are kept in place in it
+    const double* Tcur = (s->pipe && pipe_current_buffer(s, h)) ? P.T1 : P.T;
+    int rc = sens_session_launch(s->m_in, s->n, P.m, (size_t)P.ld, s->sense, s->sens_rmap, s->sens_b, s->sens_c, P.basis,
+                                 Tcur, s->sens_rowof, s->sens_partial, s->sens_report, s->stream);
+    if (rc != LPX_OK) return rc;
+    LPX_CUDA(cudaMemcpyAsync(report, s->sens_report, stride * 8, cudaMemcpyDeviceToHost, s->stream));
     LPX_CUDA(cudaStreamSynchronize(s->stream));
     return LPX_OK;
 }

@@ -19,4 +19,16 @@ int reg_launch_batched(int count, int m, int n, int sense, const double* A, cons
 
 void set_bnb_instance(int k);
 
+// sensitivity report kernels (lpx_sens.cu).  Batched: compact tableaux, b / c / basis strided per LP, rel shared.
+int sens_launch_batched(int count, int m, int n, int mm, int sense, const int* rel, const double* b, const double* c,
+                        const int* status, const int* basis, const double* tableau, double* report,
+                        cudaStream_t stream);
+// Session: one OPTIMAL tableau with rows ld doubles apart; rmap[i] = expanded row of constraint i's slack,
+// -(row + 1) for an EQ constraint.  rowof: n + mm + 1 ints, partial: sens_session_partial_bytes(m, mm).
+#define LPX_SENS_CHUNK_ROWS 32
+size_t sens_session_partial_bytes(int m, int mm);
+int sens_session_launch(int m, int n, int mm, size_t ld, int sense, const int* rmap, const double* b, const double* c,
+                        const int* basis, const double* T, int* rowof, void* partial, double* report,
+                        cudaStream_t stream);
+
 }  // namespace lpx

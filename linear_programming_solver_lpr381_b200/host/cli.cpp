@@ -5,6 +5,8 @@
 //                                           Branch and Bound | Cutting Plane | Revised Cutting Plane | BranchAndBoundKnapsack | ...
 //   lpr381 --export "<algorithm>" [input]   the export file layout ("Linear Program:" / "Iterations:")
 //   lpr381 --crlf ...                       Environment.NewLine = "\r\n" (where the reference runs)
+//   lpr381 --sensitivity "Primal Simplex" [input]   appends this project's "Sensitivity Analysis" block (shadow
+//                                           prices, slacks, RHS / cost ranges; not the reference's text)
 #include <cstdio>
 #include <fstream>
 #include <iostream>
@@ -16,18 +18,25 @@ using namespace lpr381;
 
 int main(int argc, char** argv) {
     int arg = 1;
-    bool as_export = false;
+    bool as_export = false, sensitivity = false;
     for (; arg < argc; arg++) {
         const std::string a = argv[arg];
         if (a == "--export") as_export = true;
         else if (a == "--crlf") NewLine() = "\r\n";
+        else if (a == "--sensitivity") sensitivity = true;
         else break;
     }
     if (arg >= argc) {
-        std::fprintf(stderr, "usage: lpr381 [--export] [--crlf] \"<algorithm>\" [input.txt]\n");
+        std::fprintf(stderr, "usage: lpr381 [--export] [--crlf] [--sensitivity] \"<algorithm>\" [input.txt]\n"
+                             "  --sensitivity (\"Primal Simplex\" only): this project's sensitivity report, not the "
+                             "reference's\n");
         return 2;
     }
     const std::string algorithm = argv[arg++];
+    if (sensitivity && algorithm != "Primal Simplex") {
+        std::fprintf(stderr, "--sensitivity: only \"Primal Simplex\" results are analysed\n");
+        return 2;
+    }
     std::stringstream in;
     if (arg < argc) {
         std::ifstream f(argv[arg]);
@@ -42,8 +51,10 @@ int main(int argc, char** argv) {
     const std::string input = in.str();
     std::string box;  // iterationOutputTextBox
     UpdatePivot append = [&](const std::string& text, const Highlight&) { box += text; };
+    std::string sens_block;
     try {
         LPProblem problem = LPParser::ParseFromText(input);
+        if (sensitivity) sens_block = "\n\n" + SensitivityText(problem);
         SimplexResult result;
         // the dropdown routes "Branch and Bound Knapsack" to plain BranchAndBound upstream
         // (Form1.cs:263-270); the knapsack solver itself is reachable here under its class name
@@ -60,7 +71,10 @@ int main(int argc, char** argv) {
             result = LPSolver().Solve(problem, algorithm, append);
         box += "\n\nFinal Report:\n" + result.Report;
         box += "\n\nSummary:\n" + result.Summary;
+        box += sens_block;
     } catch (const LpException& e) {
+        // a model the solve rejects (e.g. a '>=' row) still gets its sensitivity block: the status message
+        if (!sens_block.empty()) std::cout << sens_block.substr(2);
         std::fprintf(stderr, "Error: %s\n", e.what());
         return 1;
     }

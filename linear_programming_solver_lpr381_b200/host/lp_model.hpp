@@ -120,6 +120,10 @@ struct LPController {
     static SimplexResult SolvePrimalSimplex(const LPProblem& problem);
 };
 
+// `lpr381 --sensitivity`: this project's sensitivity block for an optimal Primal Simplex result (sensitivity_host.cpp);
+// the status message instead when the solve does not end OPTIMAL.  Not the reference's SensitivityAnalysis text.
+std::string SensitivityText(const LPProblem& problem);
+
 // Environment.NewLine of the host ("\n"; the reference's Windows build uses "\r\n")
 std::string& NewLine();
 
