@@ -68,7 +68,9 @@ typedef struct lpx_options {
                              prep per pivot, 3 blocked with a one-CTA look-ahead, 4 blocked, not pipelined */
     int reg_variant;      /* register-resident kernel: 0 = default build (4 when n <= 128, else 2), 1 one CTA per SM
                              (all registers), 2 two CTAs per SM (two column slots in shared memory), 3 three CTAs per
-                             SM (four slots), 4 condensed tableau (non-basic columns only), three CTAs per SM */
+                             SM (four slots), 4 condensed tableau (non-basic columns only), three CTAs per SM, 8 row
+                             warps x 8 rows (two of four slots in shared memory), 5 the same with 4 row warps x 16
+                             rows (one of four slots in shared memory); 4 and 5 need n <= 128 */
     int stream_block;     /* streaming kernels: pivots applied per HBM pass (0 = default, max 16) */
     int stream_pass_variant; /* blocked pass: 0 auto, 1 two doubles per thread, 2 one double per thread,
                                 3 TMA-staged (cp.async.bulk + mbarrier pipeline) */

@@ -72,7 +72,7 @@ __global__ void __launch_bounds__((NW + 1) * 32, OCC) reg_simplex_kernel(const R
     __shared__ int s_nbvar[COND ? COLS : 1];       // COND: the variable held by each column slot
     constexpr int NT = (NW + 1) * 32;
     static_assert(ROWS >= 64 && ROWS <= 96, "the control warp holds the RHS of rows lane and lane+32");
-    __shared__ double s_f[ROWS];     // entering column = update factors
+    __shared__ __align__(16) double s_f[ROWS];  // entering column = update factors
     __shared__ double s_rhs[ROWS + 1];
     __shared__ double s_p[COLS];     // normalised pivot row
     __shared__ double s_raw[COLS];   // the leaving row before normalisation
@@ -130,7 +130,10 @@ __global__ void __launch_bounds__((NW + 1) * 32, OCC) reg_simplex_kernel(const R
         if (lane + 32 < m) rhs1 = bp[lane + 32];
     }
     // the reference's up-front check (PrimalSimplex.cs:73-76); '>=' rows cannot occur here
-    if (tid == 0) s_ctl[1] = LPX_RUNNING;
+    if (tid == 0) {
+        s_ctl[1] = LPX_RUNNING;
+        s_ctl[3] = 0;  // pivots done: kept here by lane 0 of the control warp, not in a register of every thread
+    }
     for (int i = tid; i < m; i += NT) s_basis[i] = n + i;
     if (COND)
         for (int j = tid; j < COLS; j += NT) s_nbvar[j] = j;
@@ -144,40 +147,47 @@ __global__ void __launch_bounds__((NW + 1) * 32, OCC) reg_simplex_kernel(const R
         // ChooseEntering on the objective row (control warp): most negative entry below -1e-9,
         // lowest column on ties, NaN never wins.  Two REDUX minima on the value key, one on the
         // column index.
-        auto choose_entering = [&](int next_iter) {
-            unsigned long long kk[C], kl = ~0ULL;
+        // The keys are computed twice rather than kept in an array: the control warp shares the register budget
+        // with the row warps' tableau.
+        auto choose_entering = [&]() {
+            auto key = [&](int c) {
+                const double zv = T_GET(0, c);
+                return zv < -LPX_EPS ? dkey(zv) : ~0ULL;
+            };
+            unsigned long long kl = ~0ULL;
 #pragma unroll
             for (int c = 0; c < C; c++) {
-                const double zv = T_GET(0, c);
-                kk[c] = zv < -LPX_EPS ? dkey(zv) : ~0ULL;
-                kl = kk[c] < kl ? kk[c] : kl;
+                const unsigned long long kc = key(c);
+                kl = kc < kl ? kc : kl;
             }
             const unsigned long long K = warp_min_u64(kl);
+            int ln;  // the lane index read afresh: held across the pivot loop it costs a register the row warps need
+            asm volatile("mov.u32 %0, %%laneid;" : "=r"(ln));
             int jl = INT_MAX;
 #pragma unroll
             for (int c = C - 1; c >= 0; c--)
-                if (kk[c] == K) {
-                    if (COND) jl = min(jl, (s_nbvar[lane + 32 * c] << 8) | (lane + 32 * c));  // lowest VARIABLE wins
-                    else jl = lane + 32 * c;
+                if (key(c) == K) {
+                    if (COND) jl = min(jl, (s_nbvar[ln + 32 * c] << 8) | (ln + 32 * c));  // lowest VARIABLE wins
+                    else jl = ln + 32 * c;
                 }
             int j = __reduce_min_sync(0xffffffffu, jl);
             if (COND) j &= 255;
             // one word tells every warp how the next pass starts: the column, -1 = optimal, -2 = the
             // reference's iteration limit, which it tests BEFORE looking for an entering column
-            if (lane == 0) s_ctl[0] = next_iter > B.max_iter ? -2 : (K == ~0ULL ? -1 : j);
+            if (lane == 0) s_ctl[0] = s_ctl[3] + 1 > B.max_iter ? -2 : (K == ~0ULL ? -1 : j);
         };
-        if (ctl) choose_entering(1);
+        if (ctl) choose_entering();
 
         // One pivot = five short phases separated by block barriers.  Latency, not throughput,
         // bounds it, so the narrow decisions (entering column, ratios, leaving row, RHS) run in the
         // control warp only — the row warps neither repeat them nor compete for issue slots — and
         // every division is done by a different thread.
-        int iter = 1;
         // DBG build: lane 0 of four warps records its ARRIVAL time at each barrier of pivots 4..7
         const int dslot = w == 0 ? 0 : w == 5 ? 1 : w == NW - 1 ? 2 : ctl ? 3 : -1;
+        int dbg_piv = 0;
 #define REG_STAMP(k)                                                                                  \
-    if (DBG && B.dbg && p == 0 && lane == 0 && dslot >= 0 && iter >= 4 && iter < 8)                    \
-        B.dbg[((iter - 4) * 4 + dslot) * 8 + (k)] = clock64();
+    if (DBG && B.dbg && p == 0 && lane == 0 && dslot >= 0 && dbg_piv >= 3 && dbg_piv < 7)             \
+        B.dbg[((dbg_piv - 3) * 4 + dslot) * 8 + (k)] = clock64();
         while (true) {
             __syncthreads();  // (A) s_ctl[0] holds the entering column; all updates are done
             const int e = s_ctl[0];
@@ -215,7 +225,7 @@ __global__ void __launch_bounds__((NW + 1) * 32, OCC) reg_simplex_kernel(const R
                 a1 = s_f[lane + 32];
                 const double nan = __longlong_as_double(0x7ff8000000000000LL);  // = not eligible
                 const double r0 = (lane < m && a0 > LPX_EPS) ? __ddiv_rn(rhs0, a0) : nan;
-                const double r1 = (lane + 32 < m && a1 > LPX_EPS) ? __ddiv_rn(rhs1, a1) : nan;
+                const double r1 = (lane < m - 32 && a1 > LPX_EPS) ? __ddiv_rn(rhs1, a1) : nan;  // lane + 32 < m
                 const int row = warp_margin_scan64(m, LPX_MARGIN_PRIMAL, r0, r1);
                 if (lane == 0) s_ctl[2] = row;
             }
@@ -273,10 +283,11 @@ __global__ void __launch_bounds__((NW + 1) * 32, OCC) reg_simplex_kernel(const R
                     }
                     __syncwarp();
                 }
-                choose_entering(iter + 1);
+                if (lane == 0) s_ctl[3]++;
+                choose_entering();
                 const double u0 = __dsub_rn(rhs0, __dmul_rn(a0, prhs)), u1 = __dsub_rn(rhs1, __dmul_rn(a1, prhs));
                 rhs0 = lane == lr ? prhs : u0;
-                rhs1 = lane + 32 == lr ? prhs : u1;
+                rhs1 = lane == lr - 32 ? prhs : u1;
                 zrhs = __dsub_rn(zrhs, __dmul_rn(fz, prhs));
                 if (!COND && lane == 0) s_basis[lr] = e;
             } else {
@@ -291,32 +302,36 @@ __global__ void __launch_bounds__((NW + 1) * 32, OCC) reg_simplex_kernel(const R
                     REG_ZERO(0) else REG_ZERO(1) else REG_ZERO(2) else REG_ZERO(3) else REG_ZERO(4) else REG_ZERO(5) else REG_ZERO(6) else REG_ZERO(7)
 #undef REG_ZERO
                 }
-                if (CS != 0) {
+                // rows outside, slots inside: the C pivot-row entries stay in registers and each factor is
+                // read where it is used (two rows per broadcast LDS.128), so that a 16-row warp never holds
+                // all R factors at once; the shared-memory slot of a row is loaded and stored exactly once
+                double pc[C];
 #pragma unroll
-                    for (int r = 0; r < R; r++) f[r] = s_f[w * R + r];
+                for (int c = 0; c < C; c++) pc[c] = s_p[lane + 32 * c];
+#pragma unroll
+                for (int r = 0; r < R; r++) {
+                    const double fr = CS == 0 ? f[r] : s_f[w * R + r];
+#pragma unroll
+                    for (int c = 0; c < C; c++) T_SET(r, c, __dsub_rn(T_GET(r, c), __dmul_rn(fr, pc[c])));
                 }
+                // the leaving row becomes the normalised pivot row; its index is read again rather than held
+                // across barrier (E) in a register the update needs
+                const int rlp = s_ctl[2] - w * R;
+                if (rlp >= 0 && rlp < R) {
 #pragma unroll
-                for (int c = 0; c < C; c++) {
-                    const double pc = s_p[lane + 32 * c];
+                    for (int r = 0; r < R; r++)
+                        if (r == rlp) {
 #pragma unroll
-                    for (int r = 0; r < R; r++) T_SET(r, c, __dsub_rn(T_GET(r, c), __dmul_rn(f[r], pc)));
-                }
-                if (w == wl) {  // the leaving row becomes the normalised pivot row
-#pragma unroll
-                    for (int c = 0; c < C; c++) {
-                        const double pc = s_p[lane + 32 * c];
-#pragma unroll
-                        for (int r = 0; r < R; r++)
-                            if (r == rl) T_SET(r, c, pc);
-                    }
+                            for (int c = 0; c < C; c++) T_SET(r, c, pc[c]);
+                        }
                 }
             }
             REG_STAMP(4)
-            n_piv++;
-            iter++;
+            if (DBG) dbg_piv++;
         }
         __syncthreads();
 #undef REG_STAMP
+        n_piv = s_ctl[3];
 
         // ---- results ----------------------------------------------------------------------------
         if (ctl) {
@@ -329,12 +344,14 @@ __global__ void __launch_bounds__((NW + 1) * 32, OCC) reg_simplex_kernel(const R
             // variables' columns, the row's own basic variable = 1; then one coalesced copy
             double* To = B.tableau + (size_t)p * (m + 1) * width;
             double* rb = s_t + (size_t)(CS ? CS : 1) * (ROWS + 1) * 32 + (size_t)w * RBW;
+            // zeroed once: every row of the warp scatters its non-basic entries to the same places (by the same
+            // lane), so between rows only the unit of the row's basic variable has to be taken back out
+            for (int k = lane; k < RBW; k += 32) rb[k] = 0.0;
+            __syncwarp();
 #pragma unroll
             for (int r = 0; r < R; r++) {
                 const int i = ctl ? m : w * R + r;
                 if (ctl ? r == 0 : i < m) {
-                    for (int k = lane; k < RBW; k += 32) rb[k] = 0.0;
-                    __syncwarp();
 #pragma unroll
                     for (int c = 0; c < C; c++) {
                         const int j = lane + 32 * c;
@@ -344,6 +361,7 @@ __global__ void __launch_bounds__((NW + 1) * 32, OCC) reg_simplex_kernel(const R
                     __syncwarp();
                     for (int j = lane; j < width - 1; j += 32) To[(size_t)i * width + j] = rb[j];
                     __syncwarp();
+                    if (!ctl && lane == 0) rb[s_basis[i]] = 0.0;
                 }
             }
             if (ctl) {
@@ -443,7 +461,7 @@ int reg_launch_batched(int count, int m, int n, int sense, const double* A, cons
     B.z = z;
     B.tableau = tableau;
     B.total_pivots = total_pivots;
-    // Builds: the condensed tableau at three CTAs per SM (reg_variant 4, the default for n <= 128); the full tableau
+    // Builds: the condensed tableau at three CTAs per SM (reg_variant 4, the default for n <= 128, and 5); the full tableau
     // with all six column slots in registers, one CTA per SM (1), four in registers + two in shared memory, two CTAs
     // per SM (2: 1.04 ms per 4096-LP batch, against 1.34 for 1), or two + four at three CTAs per SM (3: 1.19 ms).
     B.dbg = nullptr;
@@ -475,11 +493,17 @@ int reg_launch_batched(int count, int m, int n, int sense, const double* A, cons
     }
     // Default: the condensed build, three CTAs per SM (n <= 128 columns of A; wider problems keep the six-slot build).
     const int variant = opt.reg_variant ? opt.reg_variant : (n <= 128 ? 4 : 2);
-    if (variant == 4) {
-        if (n > 128) {
-            set_error("LPX_KERNEL_CTA_REG, reg_variant 4: the condensed build holds n <= 128 non-basic columns");
-            return LPX_E_CAPACITY;
-        }
+    if ((variant == 4 || variant == 5) && n > 128) {
+        set_error("LPX_KERNEL_CTA_REG, reg_variant 4 / 5: the condensed build holds n <= 128 non-basic columns");
+        return LPX_E_CAPACITY;
+    }
+    if (variant == 5) {
+        // 4 row warps x 16 rows, three of the four column slots in registers (128 registers, no spills) and one in
+        // shared memory, + one row buffer per warp: half the update's shared-memory traffic of build 4, but at 15
+        // warps per SM instead of 27 (0.780 ms per 4096-LP batch against 0.726 for build 4, DESIGN.md §9)
+        constexpr size_t smem5 = (size_t)1 * (4 * 16 + 1) * 32 * 8 + (size_t)5 * (128 + 64 + 32) * 8;
+        reg_simplex_kernel<4, 16, 3, 1, 3, false, true><<<count, 5 * 32, smem5, stream>>>(B);
+    } else if (variant == 4) {
         // 8 row warps x 8 rows, four column slots (two in registers, two in shared memory) + one row buffer per warp;
         // 72 registers, no spills (11 warps x 6 rows at 56 registers: 0.806 ms against 0.782 per 4096-LP batch)
         constexpr size_t smem4 = (size_t)2 * (8 * 8 + 1) * 32 * 8 + (size_t)9 * (128 + 64 + 32) * 8;
