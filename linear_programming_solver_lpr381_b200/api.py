@@ -50,11 +50,12 @@ def primal_solve(A, b, c, rel=None, sense=0, max_iterations=10000, kernel=F.KERN
     return out
 
 
-def dual_solve(A, b, c, rel=None, sense=0, max_iterations=10000, kernel=F.KERNEL_AUTO, history=0, pivots_cap=10200):
+def dual_solve(A, b, c, rel=None, sense=0, max_iterations=10000, kernel=F.KERNEL_AUTO, threads=0, history=0,
+               pivots_cap=10200):
     A, b, c, rel = _prep(A, b, c, rel)
     m, n = A.shape
     rows, cols = tableau_dims(m, n, rel)
-    opt = F.make_options(max_iterations, kernel)
+    opt = F.make_options(max_iterations, kernel, threads)
     status, npiv, silent = C.c_int(), C.c_int(), C.c_int()
     pivots = np.full((pivots_cap, 2), -1, dtype=np.int32)
     basis = np.zeros(rows - 1, dtype=np.int32)
@@ -262,11 +263,11 @@ class Session:
             pass
 
 
-def bnb_simplex_batched(A, b, c, rel=None, sense=0, max_iterations=10000, kernel=F.KERNEL_AUTO, on_node=None,
-                        want_history=False):
+def bnb_simplex_batched(A, b, c, rel=None, sense=0, max_iterations=10000, kernel=F.KERNEL_AUTO, threads=0,
+                        on_node=None, want_history=False):
     A, b, c, rel = _prep(A, b, c, rel)
     count, m, n = A.shape
-    opt = F.make_options(max_iterations, kernel)
+    opt = F.make_options(max_iterations, kernel, threads)
     found = np.zeros(count, dtype=np.int32)
     best_z = np.zeros(count)
     best_x = np.zeros((count, n))
@@ -314,12 +315,12 @@ def bnb_simplex(A, b, c, rel=None, sense=0, trace=False, want_history=False, **k
     return out
 
 
-def bnb_pooled(A, b, c, rel=None, sense=0, batch=64, node_cap=1 << 20):
+def bnb_pooled(A, b, c, rel=None, sense=0, batch=64, node_cap=1 << 20, threads=0):
     """Mode B, the pooled tree (lpx_bnb_pooled) — NOT the reference's tree.  After lpx_comm_init every rank must
     make the same call; every rank returns the same result."""
     A, b, c, rel = _prep(A, b, c, rel)
     m, n = A.shape
-    opt = F.make_options()
+    opt = F.make_options(threads=threads)
     found = C.c_int()
     best_z = C.c_double()
     best_x = np.zeros(n)

@@ -217,7 +217,8 @@ struct Driver {
         double* d_z = ws_dev_as<double>(WS_Z, cnt);
         int* d_piv = pivots_cap ? ws_dev_as<int>(WS_PIVOTS, (size_t)cnt * pivots_cap * 2) : nullptr;
         double* d_hist = history_cap ? ws_dev_as<double>(WS_HISTORY, (size_t)cnt * history_cap * tsize) : nullptr;
-        const bool fits = cta_fits_smem(max_rows, max_width);
+        // a forced global-memory tableau needs working storage also where the tableau would fit shared memory
+        const bool fits = cta_fits_smem(max_rows, max_width) && opt.kernel != LPX_KERNEL_CTA_GLOBAL;
         double* d_scratch = fits ? nullptr : ws_dev_as<double>(WS_SCRATCH, (size_t)cnt * tsize);
         int* h_stat = ws_pin_as<int>(WS_STATUS, (size_t)cnt * 6);
         double* h_x = ws_pin_as<double>(WS_X, (size_t)cnt * n);
@@ -531,7 +532,9 @@ struct Driver {
             B.max_iter = opt.max_iterations;
             B.max_rows = max_rows;
             B.max_width = max_width;
-            if (!cond && kind == 1 && cta_cluster_size_for(max_rows, max_width) == 0) {  // beyond a 4-CTA cluster
+            // beyond a 4-CTA cluster, or a forced global-memory tableau (either kind of node)
+            if (!cond && ((kind == 1 && cta_cluster_size_for(max_rows, max_width) == 0) ||
+                          opt.kernel == LPX_KERNEL_CTA_GLOBAL)) {
                 double* sc = (double*)ws_dev(s_scr, (size_t)cnt * tsize * 8);
                 if (!sc) return LPX_E_CUDA;
                 B.scratch = sc;

@@ -141,7 +141,10 @@ def test_c3_full_size_first_pivots(lpx, orc):
     s.close()
 
 
-@pytest.mark.parametrize("protocol,kblock,pass_variant", [(0, 0, 0), (0, 0, 3), (0, 16, 0), (4, 0, 3)])
+# pass variants 1 and 2 are the LDG/STG block passes, stream_update_block_kernel<8, 2, 4>, <8, 1, 4>, <16, 2, 2> and
+# <16, 1, 4> (lpx_stream.cu:581-587); protocol 0 with kblock <= 8 takes the pipelined kernel whatever the variant
+@pytest.mark.parametrize("protocol,kblock,pass_variant", [(0, 0, 0), (0, 0, 3), (0, 16, 0), (4, 0, 3), (4, 3, 1),
+                                                          (4, 8, 2), (0, 16, 1), (4, 11, 2)])
 def test_c3_full_size_pipelined_blocks(lpx, orc, protocol, kblock, pass_variant):
     """4096 x 8192 through the production protocols over >= 8 look-ahead blocks, stepped in uneven
     chunks (so blocks are cut short and the Fbuf/Pbuf/Lbuf halves and the ping-pong tableau buffers
@@ -164,13 +167,19 @@ def test_c3_full_size_pipelined_blocks(lpx, orc, protocol, kblock, pass_variant)
     s.close()
 
 
-@pytest.mark.parametrize("kblock", [0, 3, 16])
-def test_tma_staged_pass(lpx, orc, kblock):
-    """pass_variant 3: the blocked HBM pass staged through shared memory by cp.async.bulk."""
+# (kblock, pass_variant, protocol); the ids of the TMA-staged cases stay the kblock alone
+BLOCK_PASSES = [pytest.param(k, 3, 0, id=str(k)) for k in (0, 3, 16)] + \
+    [pytest.param(k, v, 4 if k <= 8 else 0, id=f"{k}-ldg{v}") for v in (1, 2) for k in (0, 3, 16)]
+
+
+@pytest.mark.parametrize("kblock,pass_variant,protocol", BLOCK_PASSES)
+def test_tma_staged_pass(lpx, orc, kblock, pass_variant, protocol):
+    """The blocked HBM pass: pass_variant 3 stages it through shared memory by cp.async.bulk, 1 and 2 are the
+    LDG/STG passes with two / one doubles per thread.  The small LPs give a row chunk of one row per CTA."""
     for (m, n, seed) in [(256, 512, 7), (100, 37, 3), (9, 700, 5)]:
         A, b, c = workloads.lp_integer(m, n, seed)
         want = orc.primal_solve(A, b, c)
-        s = lpx.Session(A, b, c, kblock=kblock, pass_variant=3)
+        s = lpx.Session(A, b, c, kblock=kblock, pass_variant=pass_variant, single_cta_select=protocol)
         st, tot = F.RUNNING, 0
         while st == F.RUNNING:
             st, tot = s.step(50)
@@ -186,7 +195,8 @@ def test_tma_staged_pass(lpx, orc, kblock):
         c = rng.integers(-2, 9, size=n).astype(float)
         rel = rng.choice([0, 0, 0, 2], size=m).astype(np.int32)
         want = orc.primal_solve(A, b, c, rel, 0, max_iterations=60)
-        s = lpx.Session(A, b, c, rel=rel, max_iterations=60, kblock=kblock, pass_variant=3)
+        s = lpx.Session(A, b, c, rel=rel, max_iterations=60, kblock=kblock, pass_variant=pass_variant,
+                        single_cta_select=protocol)
         st, tot = F.RUNNING, 0
         while st == F.RUNNING:
             st, tot = s.step(7)
