@@ -323,6 +323,65 @@ int lpx_primal_solve_sensitivity_batched(int count, int m, int n, int sense, con
  * as of its last step / sync, is LPX_OPTIMAL). */
 int lpx_session_sensitivity(lpx_session* s, double* report);
 
+/* ---- Re-optimization of an optimal Primal Simplex result — NOT the reference's ---------------------------- */
+/* What-if queries past the sensitivity ranges: change b, change c, add a constraint or add a variable, then re-solve
+ * warm from the final tableau of a Primal Simplex solve with status LPX_OPTIMAL, instead of from the slack basis.
+ * Checked against oracle/orc_reopt.cpp bit for bit and against an independent LP solver.  Notation as in the
+ * sensitivity section: m' rows after EQ expansion, W = n + m' + 1, the slack of constraint i is s1 = n + i1 (an EQ
+ * row also has s2 = n + i2), T[m'] is the z-row, the RHS the last column, max-form (Min costs negated as
+ * BuildTableau does).  FP64 with separate multiply / add / subtract; a term whose payload coefficient is zero
+ * (either sign) is SKIPPED, so an all-zero change returns the base's bits.  One call has one kind; each query has
+ * its own payload (lpx_reopt_payload_stride doubles) and names its base.
+ *   LPX_REOPT_RHS   payload db[m].  For i ascending with db_i != 0, on every row r (z-row included):
+ *                   T[r][W-1] += db_i * T[r][s1]; an EQ row also T[r][W-1] -= db_i * T[r][s2].
+ *                   Then Dual Simplex with the reference's rules (most negative RHS < -1e-9 leaves; min z_j / -a over
+ *                   a < -1e-9 with the 1e-12 margin scan enters; limit 10000), no silent pivots.  Shape unchanged.
+ *   LPX_REOPT_COST  payload dc[n], in the model's sense.  delta_j = dc_j (Max) or -dc_j (Min).  For j ascending with
+ *                   dc_j != 0: if j is basic in row r, z[k] += delta_j * T[r][k] for all k < W (RHS included); then
+ *                   z[j] -= delta_j.  Then Primal Simplex with the reference's rules (entering below -1e-9, ratio
+ *                   margin 1e-9, opt.max_iterations).  Shape unchanged.
+ *   LPX_REOPT_ROW   payload a[n], rel (0 LE / 1 GE, stored as a double), beta.  New row m' and new slack column
+ *                   n + m': the old RHS position becomes the slack column, the RHS moves right (the layout of the
+ *                   pooled tree's bound row).  Raw row: a, +0 in the old slack columns, beta; for GE every entry of it,
+ *                   zeros included, is negated.  +1 in the new slack column.  Then for r = 0 .. m'-1 ascending with
+ *                   j = basis[r] < n and a_j != 0: row[k] -= a~_j * T[r][k] over the old columns and the RHS (a~ = the
+ *                   raw row's a).  The old rows and the z-row get +0 in the new column.  Dual Simplex as for RHS.
+ *                   rows + 1, cols + 1; the new slack is basic in the new row.
+ *   LPX_REOPT_COL   payload a[m], c_new in the model's sense.  New decision variable at column n: old columns >= n and
+ *                   basis entries >= n shift by one.  Its entry starts at +0 in the constraint rows and at -c'_new in
+ *                   the z-row (c' = c for Max, -c for Min, as BuildTableau writes it); then on every row, for i
+ *                   ascending with a_i != 0: v += a_i * T[r][s1]; an EQ row also v -= a_i * T[r][s2].  Primal Simplex
+ *                   as for COST.  cols + 1; x has n + 1 entries.
+ * A query whose base is not LPX_OPTIMAL gets the base's status, 0 pivots and zeroed basis / x / z / tableau.
+ * Outcomes: RHS / ROW: LPX_OPTIMAL, LPX_INFEASIBLE, LPX_S_ITER_LIMIT; COST / COL: LPX_OPTIMAL, LPX_UNBOUNDED,
+ * LPX_S_ITER_LIMIT.  opt.kernel: AUTO (shared-memory tableau when it fits, else global memory), CTA_SMEM
+ * (LPX_E_CAPACITY when it does not fit) or CTA_GLOBAL; any other kernel, an unknown kind or a ROW rel other than 0 / 1
+ * is LPX_E_BAD_ARGS.  opt.threads is honoured. */
+#define LPX_REOPT_RHS  1
+#define LPX_REOPT_COST 2
+#define LPX_REOPT_ROW  3
+#define LPX_REOPT_COL  4
+/* doubles per query payload: m (RHS), n (COST), n + 2 (ROW), m + 1 (COL); 0 for an unknown kind */
+size_t lpx_reopt_payload_stride(int kind, int m, int n);
+/* rows / cols of a query's result tableau (rel: the base model's, host pointer, nullable = all LE) */
+int lpx_reopt_dims(int kind, int m, int n, const int* rel, int* rows, int* cols);
+/* Device pointers throughout (rel included; the outputs of lpx_primal_solve_batched_dev serve as the bases),
+ * asynchronous on `stream`.  base_status / base_basis / base_tableau: the bases, indexed by src[q] (nullable: query q
+ * uses base q).  payload: count x stride.  Per query: status, n_pivots (nullable), pivots (nullable, pivots_cap pairs),
+ * basis (nullable, rows - 1), x (nullable, n or n + 1 for COL), z (nullable), tableau (nullable, rows x cols as
+ * lpx_reopt_dims gives them; must not overlap the bases).  total_pivots: as in lpx_primal_solve_batched_dev. */
+int lpx_reoptimize_batched_dev(int kind, int count, int m, int n, int sense, const int* rel, const int* base_status,
+                               const int* base_basis, const double* base_tableau, const int* src, const double* payload,
+                               const lpx_options* opt, int* status, int* n_pivots, int* pivots, int pivots_cap,
+                               int* basis, double* x, double* z, double* tableau, unsigned long long* total_pivots,
+                               void* stream);
+/* Host buffers: one GPU Primal Simplex solve of the base (A, rel, b, c; opt.max_iterations and opt.threads apply to it,
+ * the kernel is chosen automatically) and `count` queries of one kind against its final tableau.  *base_status is
+ * the base's status.  Any per-query output may be NULL. */
+int lpx_reoptimize(int kind, int m, int n, int sense, const double* A, const int* rel, const double* b, const double* c,
+                   const lpx_options* opt, int count, const double* payload, int* base_status, int* status,
+                   int* n_pivots, int* pivots, int pivots_cap, int* basis, double* x, double* z, double* tableau);
+
 /* ---- measurement helpers (bench.py) --------------------------------------------------------- */
 /* Unfused FP64 rate (separate DMUL and DADD, the only arithmetic the bit-exactness contract
  * allows) in TFLOP/s: the roofline denominator of the on-chip batched kernels. */

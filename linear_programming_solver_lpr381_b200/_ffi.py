@@ -18,6 +18,7 @@ S_GE_ROW, S_NEG_RHS, S_ITER_LIMIT = -1, -2, -3
 E_BAD_ARGS, E_CUDA, E_CAPACITY, E_NCCL = -4, -5, -8, -9
 KERNEL_AUTO, KERNEL_CTA_SMEM, KERNEL_CTA_GLOBAL, KERNEL_STREAM, KERNEL_CTA_REG, KERNEL_CTA_CLUSTER = 0, 1, 2, 3, 4, 5
 BNB_WANT_HISTORY = 1
+REOPT_RHS, REOPT_COST, REOPT_ROW, REOPT_COL = 1, 2, 3, 4
 
 # every symbol include/lpx.h declares; tests check that the library exports all of them
 EXPORTS = [
@@ -31,7 +32,8 @@ EXPORTS = [
     "lpx_comm_allgather", "lpx_comm_destroy", "lpx_comm_world", "lpx_comm_rank", "lpx_kernel_launches",
     "lpx_reset_counters", "lpx_revised_solve", "lpx_revised_history_stride", "lpx_measure_fp64_rate", "lpx_measure_latencies", "lpx_session_profile", "lpx_session_debug_stamps",
     "lpx_bnb_last_stats", "lpx_bnb_pooled", "lpx_sensitivity_stride", "lpx_sensitivity_batched_dev",
-    "lpx_primal_solve_sensitivity_batched", "lpx_session_sensitivity",
+    "lpx_primal_solve_sensitivity_batched", "lpx_session_sensitivity", "lpx_reopt_payload_stride", "lpx_reopt_dims",
+    "lpx_reoptimize_batched_dev", "lpx_reoptimize",
 ]
 
 
@@ -134,6 +136,13 @@ def lib():
     L.lpx_sensitivity_batched_dev.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 8
     L.lpx_primal_solve_sensitivity_batched.argtypes = L.lpx_primal_solve_batched.argtypes
     L.lpx_session_sensitivity.argtypes = [C.c_void_p, C.c_void_p]
+    L.lpx_reopt_payload_stride.restype = C.c_size_t
+    L.lpx_reopt_payload_stride.argtypes = [C.c_int, C.c_int, C.c_int]
+    L.lpx_reopt_dims.argtypes = [C.c_int, C.c_int, C.c_int, C.c_void_p, _ip, _ip]
+    L.lpx_reoptimize_batched_dev.argtypes = ([C.c_int] * 5 + [C.c_void_p] * 9 + [C.c_void_p, C.c_int]
+                                             + [C.c_void_p] * 6)
+    L.lpx_reoptimize.argtypes = ([C.c_int] * 4 + [C.c_void_p] * 5 + [C.c_int] + [C.c_void_p] * 5 + [C.c_int]
+                                 + [C.c_void_p] * 4)
     L.lpx_bnb_simplex_batched.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]

@@ -187,6 +187,63 @@ def sensitivity_batched_dev(count, m, n, sense, drel, db, dc, dstatus, dbasis, d
     F.check(rc)
 
 
+REOPT_KINDS = {"rhs": F.REOPT_RHS, "cost": F.REOPT_COST, "row": F.REOPT_ROW, "col": F.REOPT_COL}
+
+
+def reopt_payload_stride(kind, m, n):
+    return int(F.lib().lpx_reopt_payload_stride(REOPT_KINDS.get(kind, kind), m, n))
+
+
+def reopt_dims(kind, m, n, rel=None):
+    rows, cols = C.c_int(), C.c_int()
+    rel = None if rel is None else np.ascontiguousarray(rel, dtype=np.int32)
+    F.check(F.lib().lpx_reopt_dims(REOPT_KINDS.get(kind, kind), m, n, F.ptr(rel), C.byref(rows), C.byref(cols)))
+    return rows.value, cols.value
+
+
+def reoptimize(kind, A, b, c, payload, rel=None, sense=0, max_iterations=10000, kernel=F.KERNEL_AUTO, threads=0,
+               pivots_cap=64, want_tableau=True):
+    """lpx_reoptimize: one GPU Primal Simplex solve of the base, then len(payload) what-if queries of one kind
+    ("rhs", "cost", "row", "col" or LPX_REOPT_*) re-solved warm from its final tableau (include/lpx.h).  payload:
+    (count, reopt_payload_stride) doubles.  Returns base_status and per query status, n_pivots, pivots (count, cap, 2;
+    -1 past the query's pivots), basis, x, z, tableau."""
+    kind = REOPT_KINDS.get(kind, kind)
+    A, b, c, rel = _prep(A, b, c, rel)
+    m, n = A.shape
+    stride = reopt_payload_stride(kind, m, n)
+    pay = np.ascontiguousarray(payload, dtype=np.float64).reshape(-1, stride)
+    count = pay.shape[0]
+    rows, cols = reopt_dims(kind, m, n, rel)
+    nx = n + 1 if kind == F.REOPT_COL else n
+    opt = F.make_options(max_iterations, kernel, threads)
+    base_status = C.c_int()
+    status = np.zeros(count, np.int32)
+    npiv = np.zeros(count, np.int32)
+    pivots = np.full((count, max(pivots_cap, 1), 2), -1, np.int32)
+    basis = np.zeros((count, rows - 1), np.int32)
+    x = np.zeros((count, nx))
+    z = np.zeros(count)
+    T = np.zeros((count, rows, cols)) if want_tableau else None
+    F.check(F.lib().lpx_reoptimize(kind, m, n, sense, F.ptr(A), F.ptr(rel), F.ptr(b), F.ptr(c), C.byref(opt), count,
+                                   F.ptr(pay), C.byref(base_status), F.ptr(status), F.ptr(npiv), F.ptr(pivots),
+                                   pivots_cap, F.ptr(basis), F.ptr(x), F.ptr(z), F.ptr(T)))
+    return dict(base_status=base_status.value, status=status, n_pivots=npiv, pivots=pivots, basis=basis, x=x, z=z,
+                tableau=T)
+
+
+def reoptimize_batched_dev(kind, count, m, n, sense, drel, dbase_status, dbase_basis, dbase_tableau, dsrc, dpayload,
+                           dstatus, dnpiv, dpivots, pivots_cap, dbasis, dx, dz, dtableau, dtotal, stream,
+                           max_iterations=10000, kernel=F.KERNEL_AUTO, threads=0):
+    """lpx_reoptimize_batched_dev: raw device pointers (ints, 0 / None for the nullable ones), asynchronous on
+    `stream`; the bases are outputs of primal_solve_batched_dev."""
+    opt = F.make_options(max_iterations, kernel, threads)
+    F.check(F.lib().lpx_reoptimize_batched_dev(
+        REOPT_KINDS.get(kind, kind), count, m, n, sense, F.ptr(drel), F.ptr(dbase_status), F.ptr(dbase_basis),
+        F.ptr(dbase_tableau), F.ptr(dsrc), F.ptr(dpayload), C.byref(opt), F.ptr(dstatus), F.ptr(dnpiv),
+        F.ptr(dpivots), pivots_cap, F.ptr(dbasis), F.ptr(dx), F.ptr(dz), F.ptr(dtableau), F.ptr(dtotal),
+        F.ptr(stream or 0)))
+
+
 class Session:
     """Large single LP whose tableau lives in HBM (lpx_session_*)."""
 

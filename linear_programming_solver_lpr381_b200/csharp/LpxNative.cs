@@ -100,6 +100,20 @@ namespace Linear_Programming_Solver.Models
             double[] x, double[] z, double[] report, out long total_pivots);
         [DllImport(Lib)] public static extern int lpx_session_sensitivity(IntPtr session, double[] report);
 
+        // Re-optimization of optimal Primal Simplex results (include/lpx.h; not the reference's): what-if queries that
+        // change b (kind 1) or c (2), add a constraint (3) or a variable (4), re-solved warm from the final tableau.
+        [DllImport(Lib)] public static extern UIntPtr lpx_reopt_payload_stride(int kind, int m, int n);
+        [DllImport(Lib)] public static extern int lpx_reopt_dims(int kind, int m, int n, int[] rel, out int rows, out int cols);
+        [DllImport(Lib)]
+        public static extern int lpx_reoptimize_batched_dev(int kind, int count, int m, int n, int sense, IntPtr rel,
+            IntPtr base_status, IntPtr base_basis, IntPtr base_tableau, IntPtr src, IntPtr payload, ref LpxOptions opt,
+            IntPtr status, IntPtr n_pivots, IntPtr pivots, int pivots_cap, IntPtr basis, IntPtr x, IntPtr z,
+            IntPtr tableau, IntPtr total_pivots, IntPtr stream);
+        [DllImport(Lib)]
+        public static extern int lpx_reoptimize(int kind, int m, int n, int sense, double[] A, int[] rel, double[] b,
+            double[] c, ref LpxOptions opt, int count, double[] payload, out int base_status, int[] status,
+            int[] n_pivots, int[] pivots, int pivots_cap, int[] basis, double[] x, double[] z, double[] tableau);
+
         [DllImport(Lib)]
         public static extern int lpx_primal_solve_batched(int count, int m, int n, int sense, double[] A, int[] rel,
             double[] b, double[] c, ref LpxOptions opt, int[] status, int[] n_pivots, int[] basis, double[] x,

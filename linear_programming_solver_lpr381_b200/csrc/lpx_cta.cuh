@@ -15,18 +15,28 @@
 
 namespace lpx {
 
-// Warm start of a pooled-tree B&B node (lpx_pooled.cu, Mode B — not the reference's tree): the node's tableau
-// is its parent's FINAL tableau plus one bound row on variable `var` (x_var <= val for side 0, x_var >= val for
-// side 1, written in the parent's non-basic variables) plus one slack column; Dual Simplex pivots follow.
-// T / basis may point into ANOTHER GPU's node pool (peer memory over NVLink); out_T / out_basis are local.
+// Warm start from a final tableau: the problem's working tableau is built from a SOURCE tableau by one edit of
+// kind `kind`, then the kind's loop runs.
+//   WARM_BOUND       a pooled-tree B&B node (lpx_pooled.cu, Mode B — not the reference's tree): the parent's FINAL
+//                    tableau plus one bound row on variable `var` (x_var <= val for side 0, x_var >= val for side 1,
+//                    written in the parent's non-basic variables) plus one slack column; Dual Simplex pivots follow.
+//                    T / basis may point into ANOTHER GPU's node pool (peer memory over NVLink); out_T / out_basis
+//                    are local.
+//   LPX_REOPT_*      a re-optimization query (lpx_reopt.cu; the edits are defined in include/lpx.h): the payload is
+//                    CtaBatch::reopt_payload + p * reopt_stride, the model's rel / m_in are CtaBatch::rel / m_in, and
+//                    a source that is not LPX_OPTIMAL (base_status) is not built: the problem gets that status.
+//                    RHS / ROW run the dual loop, COST / COL the primal loop.  out_T is the working storage of the
+//                    global-memory build (unused in shared memory); results go to CtaBatch::basis / tableau.
+enum { WARM_BOUND = 0 };  // the other kinds are LPX_REOPT_RHS .. LPX_REOPT_COL (1 .. 4)
 struct WarmNode {
-    const double* T;     // parent's compact tableau, rows x (n + rows)
-    const int* basis;    // parent's basis, rows - 1 entries
-    double* out_T;       // this node's final tableau, (rows + 1) x (n + rows + 1), compact
-    int* out_basis;      // rows entries
+    const double* T;     // source (parent's / base's) compact tableau, rows x (n_src + rows)
+    const int* basis;    // its basis, rows - 1 entries
+    double* out_T;       // this problem's final tableau, compact (WARM_BOUND: (rows + 1) x (n + rows + 1))
+    int* out_basis;      // WARM_BOUND: rows entries
     double val;
-    int rows;            // of the PARENT's tableau (constraint rows + objective row)
-    int var, side, pad;
+    int rows;            // of the SOURCE tableau (constraint rows + objective row)
+    int var, side, kind;
+    int base_status;     // status of the source; anything but LPX_OPTIMAL is passed through unsolved
 };
 
 struct CtaBatch {
@@ -72,7 +82,9 @@ struct CtaBatch {
     // (R/Models/Branch&Bound.cs:268-294), and the branching variable (:198-213), -1 if none
     int* node_flags;
     int* node_branch;
-    const WarmNode* warm;  // nullable: problem p is built from warm[p] instead of (A, b, c) and runs the dual loop
+    const WarmNode* warm;  // nullable: problem p is built from warm[p] instead of (A, b, c) and runs its kind's loop
+    const double* reopt_payload;  // LPX_REOPT_* warm records: problem p's payload at + p * reopt_stride
+    long long reopt_stride;
     long long* dbg;  // LPX_CTA_PROF=1: clock64() sums per phase of the LAST problem of the batch (8 slots)
 };
 
@@ -513,6 +525,96 @@ __device__ __forceinline__ void cta_node_epilogue(const CtaBatch& B, int p, int 
     __syncthreads();
 }
 
+// The working tableau of a re-optimization query (include/lpx.h, "Re-optimization"): rows x width at T (leading
+// dimension ld), built straight from the source tableau Ts (rows_s rows) with the edit of `kind`, in the definition's
+// order of terms; sbasis receives the query's basis.  n counts the query's decision variables (COL: one more than the
+// source).  rowof: n ints of shared scratch.  Ends with a block barrier.  Not inlined: the kernel's pivot loops keep
+// the register allocation they have without it.
+template <int THREADS>
+__device__ __noinline__ void cta_reopt_build(int kind, const double* Ts, const int* bs, int rows_s, int n, int m_in,
+                                             const int* rel, int sense, const double* pay, double* T, int ld, int rows,
+                                             int width, int* sbasis, int* rowof) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    constexpr int NW = THREADS / 32;
+    const int ms = rows_s - 1;                                // source constraint rows
+    const int ns = kind == LPX_REOPT_COL ? n - 1 : n;         // source decision variables
+    const int ws = ns + rows_s, rhs_s = ws - 1;               // source width and RHS column
+    auto src = [&](int i, int j) { return Ts[(size_t)i * ws + j]; };
+    // v + sum over constraints i ascending with d_i != 0 of d_i * T[r][s1] (EQ: - d_i * T[r][s2]), term by term
+    auto slack_terms = [&](double v, int r, const double* d) {
+        int i1 = 0;
+        for (int i = 0; i < m_in; i++) {
+            const bool eq = rel && rel[i] == 2;
+            const double di = d[i];
+            if (di != 0.0) {
+                v = __dadd_rn(v, __dmul_rn(di, src(r, ns + i1)));
+                if (eq) v = __dsub_rn(v, __dmul_rn(di, src(r, ns + i1 + 1)));
+            }
+            i1 += eq ? 2 : 1;
+        }
+        return v;
+    };
+    for (int i = tid; i < ms; i += THREADS) {
+        const int b = bs[i];
+        sbasis[i] = (kind == LPX_REOPT_COL && b >= ns) ? b + 1 : b;
+    }
+    if (kind == LPX_REOPT_ROW && tid == 0) sbasis[ms] = rhs_s;  // the new slack is basic in the new row
+    if (kind == LPX_REOPT_COST)
+        for (int j = tid; j < n; j += THREADS) rowof[j] = -1;
+    __syncthreads();
+    if (kind == LPX_REOPT_COST)
+        for (int i = tid; i < ms; i += THREADS)
+            if (sbasis[i] < n) rowof[sbasis[i]] = i;
+    __syncthreads();
+    const bool ge = kind == LPX_REOPT_ROW && pay[n] == 1.0;
+    for (int i = warp; i < rows; i += NW) {
+        double* Ti = T + (size_t)i * ld;
+        for (int j = lane; j < width; j += 32) {
+            double v;
+            if (kind == LPX_REOPT_RHS) {
+                v = j < rhs_s ? src(i, j) : slack_terms(src(i, rhs_s), i, pay);
+            } else if (kind == LPX_REOPT_COST) {
+                v = src(i, j);
+                if (i == ms)
+                    for (int q = 0; q < n; q++) {
+                        const double d = pay[q];
+                        if (d == 0.0) continue;
+                        const double delta = sense == 1 ? dneg(d) : d;
+                        if (rowof[q] >= 0) v = __dadd_rn(v, __dmul_rn(delta, src(rowof[q], j)));
+                        if (j == q) v = __dsub_rn(v, delta);
+                    }
+            } else if (kind == LPX_REOPT_ROW) {
+                if (i != ms) {  // an old row (i > ms: the objective row): the old RHS position becomes the new slack
+                    const int si = i < ms ? i : ms;
+                    v = j < rhs_s ? src(si, j) : (j == rhs_s ? 0.0 : src(si, rhs_s));
+                } else if (j == rhs_s) {
+                    v = 1.0;
+                } else {  // the raw row (GE: every entry negated, zeros included), then the basic columns eliminated
+                    const int k = j < rhs_s ? j : rhs_s;
+                    v = k < n ? pay[k] : (k == rhs_s ? pay[n + 1] : 0.0);
+                    if (ge) v = dneg(v);
+                    for (int r = 0; r < ms; r++) {
+                        const int b = sbasis[r];
+                        if (b >= n || pay[b] == 0.0) continue;
+                        v = __dsub_rn(v, __dmul_rn(ge ? dneg(pay[b]) : pay[b], src(r, k)));
+                    }
+                }
+            } else {  // LPX_REOPT_COL: the new column sits at ns, the old columns from ns on move right by one
+                if (j != ns) {
+                    v = src(i, j < ns ? j : j - 1);
+                } else {
+                    const double cn = sense == 1 ? dneg(pay[m_in]) : pay[m_in];
+                    v = slack_terms(i == ms ? dneg(cn) : 0.0, i, pay);
+                }
+            }
+            Ti[j] = v;
+        }
+    }
+    if (ld > width)
+        for (int i = tid; i < rows; i += THREADS) T[(size_t)i * ld + width] = 0.0;  // pad column
+    __syncthreads();
+}
+
 template <int THREADS, bool SMEM_T>
 __global__ void __launch_bounds__(THREADS) cta_simplex_kernel(const CtaBatch B) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -524,9 +626,12 @@ __global__ void __launch_bounds__(THREADS) cta_simplex_kernel(const CtaBatch B) 
     const int nex = B.node_extra_cnt ? B.node_extra_cnt[p] : 0;
     const int exo = B.node_extra_off ? B.node_extra_off[p] : 0;
     const bool warm = B.warm != nullptr;
-    const int mode = warm ? 1 : (B.node_mode ? B.node_mode[p] : B.mode);
+    const int kind = warm ? B.warm[p].kind : WARM_BOUND;
+    const int mode = warm ? (kind == LPX_REOPT_COST || kind == LPX_REOPT_COL ? 0 : 1)
+                          : (B.node_mode ? B.node_mode[p] : B.mode);
     const int n = B.n;
-    const int m = warm ? B.warm[p].rows : B.m_base + nex;  // a warm node has one constraint row more than its parent
+    // a bound row or an added row gives one constraint row more than the source
+    const int m = warm ? B.warm[p].rows - (kind == WARM_BOUND || kind == LPX_REOPT_ROW ? 0 : 1) : B.m_base + nex;
     const int rows = m + 1, width = n + m + 1, ld = SMEM_T ? ((width + 1) & ~1) : width;
     const int rhs = width - 1;
 
@@ -553,6 +658,8 @@ __global__ void __launch_bounds__(THREADS) cta_simplex_kernel(const CtaBatch B) 
         cta_row_map<THREADS>(B, bi, nex, exo, mode, rsrc, rsgn, ctl);
         __syncthreads();
         status = ctl[0];
+    } else if (B.warm[p].base_status != LPX_OPTIMAL) {
+        status = B.warm[p].base_status;
     }
 
     int n_piv = 0, n_silent = 0, n_hist = 0;
@@ -560,7 +667,7 @@ __global__ void __launch_bounds__(THREADS) cta_simplex_kernel(const CtaBatch B) 
     double* hist = B.history ? B.history + (size_t)p * B.history_stride : nullptr;
     const size_t tsize = (size_t)rows * width;
 
-    if (warm) {
+    if (status == LPX_RUNNING && warm && kind == WARM_BOUND) {
         // ---- parent's final tableau + bound row + slack column (lpx_pooled.cu; oracle/orc_pooled.cpp) -----
         const WarmNode wn = B.warm[p];
         const int mp = wn.rows - 1, wp = n + wn.rows, rhs_p = wp - 1;  // parent: constraint rows, width, RHS column
@@ -598,6 +705,12 @@ __global__ void __launch_bounds__(THREADS) cta_simplex_kernel(const CtaBatch B) 
         if (ld > width)
             for (int i = tid; i < rows; i += THREADS) T[(size_t)i * ld + width] = 0.0;  // pad column
         __syncthreads();
+    } else if (status == LPX_RUNNING && warm) {
+        // ---- a re-optimization query: the base's final tableau with one edit (lpx_reopt.cu) ---------------
+        const WarmNode& wn = B.warm[p];
+        cta_reopt_build<THREADS>(kind, wn.T, wn.basis, wn.rows, n, B.m_in, B.rel, B.sense,
+                                 B.reopt_payload + (size_t)p * B.reopt_stride, T, ld, rows, width, sbasis,
+                                 reinterpret_cast<int*>(prow));
     } else if (status == LPX_RUNNING) {
         // ---- BuildTableau -------------------------------------------------------------------
         for (int i = warp; i < rows; i += NW) {
@@ -795,7 +908,7 @@ __global__ void __launch_bounds__(THREADS) cta_simplex_kernel(const CtaBatch B) 
         // ---- FinalizeReport's numeric part (PrimalSimplex.cs:132-138) -------------------------
         if (B.basis)
             for (int i = tid; i < m; i += THREADS) B.basis[(size_t)p * B.basis_stride + i] = sbasis[i];
-        if (warm) {  // the final tableau and basis stay in the node pool for the node's own children
+        if (warm && kind == WARM_BOUND) {  // the final tableau and basis stay in the node pool for the node's own children
             for (int i = tid; i < m; i += THREADS) B.warm[p].out_basis[i] = sbasis[i];
             if (SMEM_T) cta_copy_out<THREADS>(B.warm[p].out_T, T, ld, rows, width);
         }

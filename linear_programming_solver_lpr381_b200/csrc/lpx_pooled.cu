@@ -373,7 +373,8 @@ extern "C" int lpx_bnb_pooled(int m, int n, int sense, const double* A, const in
             w.rows = par.rows;
             w.var = nd->var;
             w.side = nd->side;
-            w.pad = 0;
+            w.kind = WARM_BOUND;
+            w.base_status = LPX_OPTIMAL;
             my_max_rows = std::max(my_max_rows, nd->rows);
             any_big = any_big || !cta_fits_smem(nd->rows, n + nd->rows);
         }

@@ -18,6 +18,7 @@ enum Slot {
     WS_EX_REL, WS_EX_RHS, WS_KN_ITEMS, WS_KN_ASSIGN, WS_KN_OUT, WS_KN_AUX, WS_KN_EXACT, WS_MISC0, WS_MISC1, WS_MISC2,
     WS_PL_IN, WS_PL_OUT, WS_PL_ALL,  // pooled-tree B&B: node descriptors, own results, everybody's results
     WS_SENS,  // sensitivity reports of lpx_primal_solve_sensitivity_batched
+    WS_RO_REC, WS_RO_PAY, WS_RO_SRC, WS_RO_BASE_T, WS_RO_BASE_I,  // re-optimization: records, payloads, base
     WS_BB_SET0,  // pipelined B&B: descriptors, results, scratch of each of LPX_BB_SETS evaluation sets
     WS_COUNT = WS_BB_SET0 + 3 * 4
 };

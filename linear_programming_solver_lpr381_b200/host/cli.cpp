@@ -7,10 +7,13 @@
 //   lpr381 --crlf ...                       Environment.NewLine = "\r\n" (where the reference runs)
 //   lpr381 --sensitivity "Primal Simplex" [input]   appends this project's "Sensitivity Analysis" block (shadow
 //                                           prices, slacks, RHS / cost ranges; not the reference's text)
+//   lpr381 --what-if "<spec>" "Primal Simplex" [input]   repeatable: appends a "What-if" block, the optimum after
+//                                           each change, re-solved warm (whatif_host.cpp; not the reference's)
 #include <cstdio>
 #include <fstream>
 #include <iostream>
 #include <sstream>
+#include <vector>
 
 #include "lp_model.hpp"
 
@@ -18,23 +21,30 @@ using namespace lpr381;
 
 int main(int argc, char** argv) {
     int arg = 1;
-    bool as_export = false, sensitivity = false;
+    bool as_export = false, sensitivity = false, bad_what_if = false;
+    std::vector<std::string> what_if;
     for (; arg < argc; arg++) {
         const std::string a = argv[arg];
         if (a == "--export") as_export = true;
         else if (a == "--crlf") NewLine() = "\r\n";
         else if (a == "--sensitivity") sensitivity = true;
-        else break;
+        else if (a == "--what-if") {
+            if (++arg < argc) what_if.push_back(argv[arg]);
+            else bad_what_if = true;
+        } else break;
     }
-    if (arg >= argc) {
-        std::fprintf(stderr, "usage: lpr381 [--export] [--crlf] [--sensitivity] \"<algorithm>\" [input.txt]\n"
+    if (arg >= argc || bad_what_if) {
+        std::fprintf(stderr, "usage: lpr381 [--export] [--crlf] [--sensitivity] [--what-if \"<spec>\"]... \"<algorithm>\" "
+                             "[input.txt]\n"
                              "  --sensitivity (\"Primal Simplex\" only): this project's sensitivity report, not the "
-                             "reference's\n");
+                             "reference's\n"
+                             "  --what-if (\"Primal Simplex\" only): rhs <i> <b_i> | cost <j> <c_j> | row <constraint> | "
+                             "col <c> <a_1> .. <a_m>\n");
         return 2;
     }
     const std::string algorithm = argv[arg++];
-    if (sensitivity && algorithm != "Primal Simplex") {
-        std::fprintf(stderr, "--sensitivity: only \"Primal Simplex\" results are analysed\n");
+    if ((sensitivity || !what_if.empty()) && algorithm != "Primal Simplex") {
+        std::fprintf(stderr, "--sensitivity / --what-if: only \"Primal Simplex\" results are analysed\n");
         return 2;
     }
     std::stringstream in;
@@ -55,6 +65,7 @@ int main(int argc, char** argv) {
     try {
         LPProblem problem = LPParser::ParseFromText(input);
         if (sensitivity) sens_block = "\n\n" + SensitivityText(problem);
+        if (!what_if.empty()) sens_block += "\n\n" + WhatIfText(problem, what_if);
         SimplexResult result;
         // the dropdown routes "Branch and Bound Knapsack" to plain BranchAndBound upstream
         // (Form1.cs:263-270); the knapsack solver itself is reachable here under its class name
@@ -73,7 +84,7 @@ int main(int argc, char** argv) {
         box += "\n\nSummary:\n" + result.Summary;
         box += sens_block;
     } catch (const LpException& e) {
-        // a model the solve rejects (e.g. a '>=' row) still gets its sensitivity block: the status message
+        // a model the solve rejects (e.g. a '>=' row) still gets its sensitivity / what-if blocks: the status message
         if (!sens_block.empty()) std::cout << sens_block.substr(2);
         std::fprintf(stderr, "Error: %s\n", e.what());
         return 1;

@@ -123,6 +123,8 @@ struct LPController {
 // `lpr381 --sensitivity`: this project's sensitivity block for an optimal Primal Simplex result (sensitivity_host.cpp);
 // the status message instead when the solve does not end OPTIMAL.  Not the reference's SensitivityAnalysis text.
 std::string SensitivityText(const LPProblem& problem);
+// `lpr381 --what-if`: re-optimization queries against the optimal Primal Simplex result (whatif_host.cpp)
+std::string WhatIfText(const LPProblem& problem, const std::vector<std::string>& specs);
 
 // Environment.NewLine of the host ("\n"; the reference's Windows build uses "\r\n")
 std::string& NewLine();
