@@ -381,6 +381,18 @@ int lpx_reoptimize_batched_dev(int kind, int count, int m, int n, int sense, con
 int lpx_reoptimize(int kind, int m, int n, int sense, const double* A, const int* rel, const double* b, const double* c,
                    const lpx_options* opt, int count, const double* payload, int* base_status, int* status,
                    int* n_pivots, int* pivots, int pivots_cap, int* basis, double* x, double* z, double* tableau);
+/* A NEW session holding one what-if query against an optimal base session.  The base is not modified and may be
+ * stepped, read or re-queried afterwards; several query sessions of one base may be open at once.  kind / payload
+ * (host pointer, lpx_reopt_payload_stride(kind, m, n) doubles, m / n the base model's) are the definition above; the
+ * edit is applied to the base's current tableau and basis, and the query's results equal oracle/orc_reopt.cpp on them
+ * bit for bit.  RHS / ROW run the Dual Simplex rules (limit 10000) one pivot per HBM pass; COST / COL run the Primal
+ * Simplex rules with opt's max_iterations and stream protocol, as lpx_session_open does.  opt NULL: the base's options.
+ * NULL (lpx_last_error() says why) when the base's status, as of its last step / sync, is not LPX_OPTIMAL, for an
+ * unknown kind, a ROW rel other than 0 / 1, or a NULL base / payload.  The query is read with the session calls:
+ * step / sync run its loop, pivots count from 0, dims give its shape (ROW: rows + 1; ROW / COL: cols + 1),
+ * read_solution's x has n + 1 entries for COL.  lpx_session_sensitivity reports on the modified model (b + db, or
+ * c + dc) for RHS / COST queries and returns LPX_E_BAD_ARGS for ROW / COL queries.  Free with lpx_session_close. */
+lpx_session* lpx_session_reoptimize(const lpx_session* base, int kind, const double* payload, const lpx_options* opt);
 
 /* ---- measurement helpers (bench.py) --------------------------------------------------------- */
 /* Unfused FP64 rate (separate DMUL and DADD, the only arithmetic the bit-exactness contract

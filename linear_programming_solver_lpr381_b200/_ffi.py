@@ -33,7 +33,7 @@ EXPORTS = [
     "lpx_reset_counters", "lpx_revised_solve", "lpx_revised_history_stride", "lpx_measure_fp64_rate", "lpx_measure_latencies", "lpx_session_profile", "lpx_session_debug_stamps",
     "lpx_bnb_last_stats", "lpx_bnb_pooled", "lpx_sensitivity_stride", "lpx_sensitivity_batched_dev",
     "lpx_primal_solve_sensitivity_batched", "lpx_session_sensitivity", "lpx_reopt_payload_stride", "lpx_reopt_dims",
-    "lpx_reoptimize_batched_dev", "lpx_reoptimize",
+    "lpx_reoptimize_batched_dev", "lpx_reoptimize", "lpx_session_reoptimize",
 ]
 
 
@@ -143,6 +143,8 @@ def lib():
                                              + [C.c_void_p] * 6)
     L.lpx_reoptimize.argtypes = ([C.c_int] * 4 + [C.c_void_p] * 5 + [C.c_int] + [C.c_void_p] * 5 + [C.c_int]
                                  + [C.c_void_p] * 4)
+    L.lpx_session_reoptimize.restype = C.c_void_p
+    L.lpx_session_reoptimize.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
     L.lpx_bnb_simplex_batched.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]

@@ -296,6 +296,30 @@ class Session:
         F.check(F.lib().lpx_session_read_solution(self._h, F.ptr(basis), F.ptr(x), C.cast(C.byref(z), C.c_void_p)))
         return basis, x, z.value
 
+    def reoptimize(self, kind, payload, **opts):
+        """lpx_session_reoptimize: a new Session holding one what-if query ("rhs", "cost", "row", "col" or
+        LPX_REOPT_*) against this session, which must be OPTIMAL and is left unchanged.  payload:
+        reopt_payload_stride(kind, m, n) doubles.  opts (max_iterations, single_cta_select, kblock, pass_variant)
+        select the Primal Simplex protocol of COST / COL queries; none given: this session's options."""
+        kind = REOPT_KINDS.get(kind, kind)
+        pay = np.ascontiguousarray(payload, dtype=np.float64).ravel()
+        if kind in REOPT_KINDS.values() and pay.size != reopt_payload_stride(kind, self.m, self.n):
+            raise F.LpxError(F.E_BAD_ARGS, "payload has %d doubles, kind %d needs %d" % (
+                pay.size, kind, reopt_payload_stride(kind, self.m, self.n)))
+        opt = F.make_options(**opts) if opts else None
+        h = F.lib().lpx_session_reoptimize(self._h, kind, F.ptr(pay),
+                                           None if opt is None else C.cast(C.byref(opt), C.c_void_p))
+        if not h:
+            raise F.LpxError(F.E_BAD_ARGS, F.last_error())
+        q = Session.__new__(Session)
+        q._h = h
+        q.m = self.m + (kind == F.REOPT_ROW)
+        q.n = self.n + (kind == F.REOPT_COL)
+        r, cc = C.c_int(), C.c_int()
+        F.check(F.lib().lpx_session_dims(h, C.byref(r), C.byref(cc)))
+        q.rows, q.cols = r.value, cc.value
+        return q
+
     def sensitivity(self):
         """Sensitivity report of the session's tableau (NaNs unless its status is OPTIMAL): `report` and its
         named views."""

@@ -113,6 +113,9 @@ namespace Linear_Programming_Solver.Models
         public static extern int lpx_reoptimize(int kind, int m, int n, int sense, double[] A, int[] rel, double[] b,
             double[] c, ref LpxOptions opt, int count, double[] payload, out int base_status, int[] status,
             int[] n_pivots, int[] pivots, int pivots_cap, int[] basis, double[] x, double[] z, double[] tableau);
+        // One query against an OPTIMAL session: a new session (IntPtr.Zero on refusal); opt IntPtr.Zero = the base's options.
+        [DllImport(Lib)]
+        public static extern IntPtr lpx_session_reoptimize(IntPtr base_session, int kind, double[] payload, IntPtr opt);
 
         [DllImport(Lib)]
         public static extern int lpx_primal_solve_batched(int count, int m, int n, int sense, double[] A, int[] rel,

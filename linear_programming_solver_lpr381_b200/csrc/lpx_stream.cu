@@ -476,6 +476,7 @@ __global__ void __launch_bounds__(256, 4) stream_update_kernel(StreamParams P) {
 
 #include "lpx_stream_block.cuh"
 #include "lpx_stream_pipe.cuh"
+#include "lpx_stream_reopt.cuh"
 
 
 // ---- session object -----------------------------------------------------------------------------
@@ -494,6 +495,9 @@ struct lpx_session {
     double* sens_b = nullptr;
     double* sens_c = nullptr;
     int* sens_rmap = nullptr;
+    std::vector<int> rmap;  // host copy of sens_rmap: constraint i -> expanded row i1 (EQ: -i1 - 1)
+    bool sens_ok = true;    // false for ROW / COL re-optimization queries and their descendants
+    bool dual = false;      // Dual Simplex per-pivot protocol (RHS / ROW re-optimization queries)
     int* sens_rowof = nullptr;
     void* sens_partial = nullptr;
     double* sens_report = nullptr;
@@ -541,11 +545,17 @@ static void sess_free(lpx_session* s) {
     delete s;
 }
 
-static int launch_pair(lpx_session* s, int probe_only) {
-    if (s->P.npartial > 0)
+static void launch_select(lpx_session* s, int probe_only) {
+    if (s->dual)
+        stream_dual_select_kernel<<<1, 1024, 0, s->stream>>>(s->P, probe_only);
+    else if (s->P.npartial > 0)
         stream_prep_kernel<<<s->P.npartial, LPX_PREP_THREADS, (size_t)s->P.m * 8, s->stream>>>(s->P, probe_only);
     else
         stream_select_kernel<<<1, 1024, 0, s->stream>>>(s->P, probe_only);
+}
+
+static int launch_pair(lpx_session* s, int probe_only) {
+    launch_select(s, probe_only);
     count_launch();
     if (!probe_only) {
         stream_update_kernel<4><<<s->grid_update, 256, 0, s->stream>>>(s->P);
@@ -664,7 +674,7 @@ static int launch_pipe_probe(lpx_session* s) {
 }
 
 // tableau buffer that holds the current tableau once every launched pass has finished
-static int pipe_current_buffer(lpx_session* s, const StreamCtl& h) {
+static int pipe_current_buffer(const lpx_session* s, const StreamCtl& h) {
     if (!s->pipe || s->blocks == 0) return 0;
     const int q = (int)((s->blocks - 1) & 1);
     return h.blk_in[q] ^ (h.blk_cnt[q] > 0 ? 1 : 0);
@@ -681,17 +691,18 @@ static int launch_block(lpx_session* s, int budget) {
     return LPX_OK;
 }
 
-// A, b, c: device pointers valid until this call returns (setup runs synchronously).
-static lpx_session* session_create(int m, int n, int sense, const double* dA, const int* rel, const double* db,
-                                   const double* dc, const lpx_options* opt) {
-    if (ensure_device() != LPX_OK) return nullptr;
-    std::lock_guard<std::recursive_mutex> lk(rt().mu);
+// A session of mm tableau rows (after EQ expansion) and n decision variables, shared by the sessions built from
+// (A, b, c) and the re-optimization queries built from a base: the stream, the sizing, every buffer, the protocol
+// and the launch grids.  dual: the Dual Simplex per-pivot protocol (stream_dual_select_kernel + the per-pivot pass,
+// limit 10000); otherwise opt's Primal Simplex protocol.  m_in / n: the model's constraints and variables (b, c).
+static lpx_session* session_new(int m_in, int n, int sense, int mm, const lpx_options* opt, bool dual) {
     lpx_session* s = new lpx_session();
     lpx_default_options(&s->opt);
     if (opt) s->opt = *opt;
-    s->m_in = m;
+    s->m_in = m_in;
     s->n = n;
     s->sense = sense;
+    s->dual = dual;
     s->device = rt().device;
     if (cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking) != cudaSuccess) {
         set_error("cudaStreamCreate failed");
@@ -700,21 +711,6 @@ static lpx_session* session_create(int m, int n, int sense, const double* dA, co
     }
     s->own_stream = true;
 
-    // row map of the EQ expansion, and the first '>=' row, both known from rel on the host
-    std::vector<int> rsrc, rsgn, rmap;
-    int first_ge = INT_MAX;
-    for (int r = 0; r < m; r++) {
-        const int rl = rel ? rel[r] : 0;
-        if (rl == 1 && first_ge == INT_MAX) first_ge = r;
-        rmap.push_back(rl == 2 ? -(int)rsrc.size() - 1 : (int)rsrc.size());
-        rsrc.push_back(r);
-        rsgn.push_back(0);
-        if (rl == 2) {
-            rsrc.push_back(r);
-            rsgn.push_back(1);
-        }
-    }
-    const int mm = (int)rsrc.size();
     StreamParams& P = s->P;
     P.m = mm;
     P.n = n;
@@ -722,14 +718,15 @@ static lpx_session* session_create(int m, int n, int sense, const double* dA, co
     P.width = n + mm + 1;
     P.ld = (P.width + 15) & ~15;
     P.colstride = (P.rows + 15) & ~15;
-    P.max_iter = s->opt.max_iterations;
+    P.max_iter = dual ? LPX_DUAL_MAX_ITER : s->opt.max_iterations;
     P.pivlog_cap = std::max(1, std::min(P.max_iter, 1 << 20));
     const size_t tbytes = (size_t)P.rows * P.ld * 8;
     P.T = (double*)sess_alloc(s, tbytes);
     P.colbuf = (double*)sess_alloc(s, (size_t)2 * P.colstride * 8);
     P.rhsbuf = (double*)sess_alloc(s, (size_t)P.colstride * 8);
     P.prow = (double*)sess_alloc(s, (size_t)P.ld * 8);
-    P.ratio = (double*)sess_alloc(s, (size_t)P.colstride * 8);
+    // the primal ratio test runs over rows, the dual one over columns
+    P.ratio = (double*)sess_alloc(s, (size_t)(dual ? std::max(P.colstride, P.ld) : P.colstride) * 8);
     P.basis = (int*)sess_alloc(s, (size_t)mm * 4);
     P.pivlog = (int*)sess_alloc(s, (size_t)P.pivlog_cap * 8);
     P.ctl = (StreamCtl*)sess_alloc(s, sizeof(StreamCtl));
@@ -742,7 +739,8 @@ static lpx_session* session_create(int m, int n, int sense, const double* dA, co
     // stream_protocol: 0 auto, 1 single-CTA select per pivot, 2 multi-CTA prep per pivot.  stream_block: pivots per pass.
     P.kblock = 0;
     // stream_protocol == 3 forces the single-CTA look-ahead (tests); otherwise the cluster version is preferred.
-    const bool blocked_wanted = s->opt.stream_protocol == 0 || s->opt.stream_protocol == 3 || s->opt.stream_protocol == 4;
+    const bool blocked_wanted =
+        !dual && (s->opt.stream_protocol == 0 || s->opt.stream_protocol == 3 || s->opt.stream_protocol == 4);
     if (blocked_wanted) {
         const int kb = s->opt.stream_block > 0 ? std::min(s->opt.stream_block, LPX_BLOCK_KMAX) : 8;
         if (s->opt.stream_protocol != 3 && lookahead_cluster_smem(P) + 24 * 1024 <= (size_t)max_smem_optin() &&
@@ -762,7 +760,7 @@ static lpx_session* session_create(int m, int n, int sense, const double* dA, co
         }
         cudaGetLastError();
     }
-    if (s->opt.stream_protocol == 1) P.npartial = 0;
+    if (dual || s->opt.stream_protocol == 1) P.npartial = 0;
     // stream_protocol 0: pipelined when the cluster look-ahead is available and the block size allows it
     // (<= 8 pivots per block); 4 forces the non-pipelined blocked protocol.
     const bool want_pipe = s->opt.stream_protocol == 0 && s->la_cluster && P.kblock > 0 && P.kblock <= LPX_PIPE_K;
@@ -812,35 +810,16 @@ static lpx_session* session_create(int m, int n, int sense, const double* dA, co
         cudaFuncSetAttribute(stream_prep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prep_smem) !=
             cudaSuccess)
         P.npartial = 0;
-    int* drsrc = (int*)sess_alloc(s, (size_t)mm * 4);
-    int* drsgn = (int*)sess_alloc(s, (size_t)mm * 4);
-    s->sens_b = (double*)sess_alloc(s, (size_t)m * 8);
+    s->sens_b = (double*)sess_alloc(s, (size_t)m_in * 8);
     s->sens_c = (double*)sess_alloc(s, (size_t)n * 8);
-    s->sens_rmap = (int*)sess_alloc(s, (size_t)m * 4);
+    s->sens_rmap = (int*)sess_alloc(s, (size_t)m_in * 4);
     if (!P.T || !P.colbuf || !P.rhsbuf || !P.prow || !P.ratio || !P.basis || !P.pivlog || !P.ctl || !P.partial || !P.Fbuf ||
-        !P.Pbuf || !P.Lbuf || !drsrc || !drsgn || !s->sens_b || !s->sens_c || !s->sens_rmap) {
+        !P.Pbuf || !P.Lbuf || !s->sens_b || !s->sens_c || !s->sens_rmap) {
         sess_free(s);
         return nullptr;
     }
-    cudaStream_t st = s->stream;
-    bool ok = true;
-    ok = ok && cudaMemcpyAsync(drsrc, rsrc.data(), (size_t)mm * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
-    ok = ok && cudaMemcpyAsync(drsgn, rsgn.data(), (size_t)mm * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
-    ok = ok && cudaMemcpyAsync(s->sens_b, db, (size_t)m * 8, cudaMemcpyDeviceToDevice, st) == cudaSuccess;
-    ok = ok && cudaMemcpyAsync(s->sens_c, dc, (size_t)n * 8, cudaMemcpyDeviceToDevice, st) == cudaSuccess;
-    ok = ok && cudaMemcpyAsync(s->sens_rmap, rmap.data(), (size_t)m * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
-    ok = ok && cudaMemsetAsync(P.colbuf, 0, (size_t)2 * P.colstride * 8, st) == cudaSuccess;
-    ok = ok && cudaMemsetAsync(P.rhsbuf, 0, (size_t)P.colstride * 8, st) == cudaSuccess;
-    if (ok) {
-        stream_validate_kernel<<<1, 1024, 0, st>>>(P.ctl, db, m, first_ge);
-        const int bgrid = std::min(P.rows, sm_count() * 8);
-        stream_build_kernel<<<bgrid, 256, 0, st>>>(P, dA, db, dc, drsrc, drsgn, sense);
-        stream_first_kernel<<<1, 1024, 0, st>>>(P);
-        stream_gather_kernel<<<(P.rows + 255) / 256, 256, 0, st>>>(P);
-        count_launch(4);
-        ok = cudaGetLastError() == cudaSuccess && cudaStreamSynchronize(st) == cudaSuccess;
-    }
-    if (!ok) {
+    if (cudaMemsetAsync(P.colbuf, 0, (size_t)2 * P.colstride * 8, s->stream) != cudaSuccess ||
+        cudaMemsetAsync(P.rhsbuf, 0, (size_t)P.colstride * 8, s->stream) != cudaSuccess) {
         cuda_fail(cudaGetLastError(), "session setup", __FILE__, __LINE__);
         sess_free(s);
         return nullptr;
@@ -909,6 +888,175 @@ static lpx_session* session_create(int m, int n, int sense, const double* dA, co
     return s;
 }
 
+// A, b, c: device pointers valid until this call returns (setup runs synchronously).
+static lpx_session* session_create(int m, int n, int sense, const double* dA, const int* rel, const double* db,
+                                   const double* dc, const lpx_options* opt) {
+    if (ensure_device() != LPX_OK) return nullptr;
+    std::lock_guard<std::recursive_mutex> lk(rt().mu);
+    // row map of the EQ expansion, and the first '>=' row, both known from rel on the host
+    std::vector<int> rsrc, rsgn, rmap;
+    int first_ge = INT_MAX;
+    for (int r = 0; r < m; r++) {
+        const int rl = rel ? rel[r] : 0;
+        if (rl == 1 && first_ge == INT_MAX) first_ge = r;
+        rmap.push_back(rl == 2 ? -(int)rsrc.size() - 1 : (int)rsrc.size());
+        rsrc.push_back(r);
+        rsgn.push_back(0);
+        if (rl == 2) {
+            rsrc.push_back(r);
+            rsgn.push_back(1);
+        }
+    }
+    const int mm = (int)rsrc.size();
+    lpx_session* s = session_new(m, n, sense, mm, opt, false);
+    if (!s) return nullptr;
+    s->rmap = rmap;
+    StreamParams& P = s->P;
+    int* drsrc = (int*)sess_alloc(s, (size_t)mm * 4);
+    int* drsgn = (int*)sess_alloc(s, (size_t)mm * 4);
+    if (!drsrc || !drsgn) {
+        sess_free(s);
+        return nullptr;
+    }
+    cudaStream_t st = s->stream;
+    bool ok = true;
+    ok = ok && cudaMemcpyAsync(drsrc, rsrc.data(), (size_t)mm * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(drsgn, rsgn.data(), (size_t)mm * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(s->sens_b, db, (size_t)m * 8, cudaMemcpyDeviceToDevice, st) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(s->sens_c, dc, (size_t)n * 8, cudaMemcpyDeviceToDevice, st) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(s->sens_rmap, rmap.data(), (size_t)m * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    if (ok) {
+        stream_validate_kernel<<<1, 1024, 0, st>>>(P.ctl, db, m, first_ge);
+        const int bgrid = std::min(P.rows, sm_count() * 8);
+        stream_build_kernel<<<bgrid, 256, 0, st>>>(P, dA, db, dc, drsrc, drsgn, sense);
+        stream_first_kernel<<<1, 1024, 0, st>>>(P);
+        stream_gather_kernel<<<(P.rows + 255) / 256, 256, 0, st>>>(P);
+        count_launch(4);
+        ok = cudaGetLastError() == cudaSuccess && cudaStreamSynchronize(st) == cudaSuccess;
+    }
+    if (!ok) {
+        cuda_fail(cudaGetLastError(), "session setup", __FILE__, __LINE__);
+        sess_free(s);
+        return nullptr;
+    }
+    return s;
+}
+
+// lpx_session_reoptimize: the query session of one what-if edit of an optimal base session (include/lpx.h,
+// "Re-optimization").  The terms of the edit are listed on the host in the definition's order; the build kernel
+// writes the query's tableau straight from the base's current buffer, then the query's protocol is armed as a new
+// session's is.  The base is only read, and is idle once this returns (setup runs synchronously).
+static lpx_session* session_reoptimize(const lpx_session* base, int kind, const double* pay, const lpx_options* opt) {
+    const StreamParams& B = base->P;
+    const int m_in = base->m_in, n = base->n, mb = B.m;
+    StreamCtl h;
+    std::vector<int> bb(mb);
+    std::vector<double> hb(m_in), hc(n);
+    if (cudaMemcpyAsync(&h, B.ctl, sizeof h, cudaMemcpyDeviceToHost, base->stream) != cudaSuccess ||
+        cudaMemcpyAsync(bb.data(), B.basis, (size_t)mb * 4, cudaMemcpyDeviceToHost, base->stream) != cudaSuccess ||
+        cudaMemcpyAsync(hb.data(), base->sens_b, (size_t)m_in * 8, cudaMemcpyDeviceToHost, base->stream) != cudaSuccess ||
+        cudaMemcpyAsync(hc.data(), base->sens_c, (size_t)n * 8, cudaMemcpyDeviceToHost, base->stream) != cudaSuccess ||
+        cudaStreamSynchronize(base->stream) != cudaSuccess) {
+        cuda_fail(cudaGetLastError(), "lpx_session_reoptimize: reading the base", __FILE__, __LINE__);
+        return nullptr;
+    }
+    if (h.status != LPX_OPTIMAL) {
+        set_error("lpx_session_reoptimize: the base session's status is " + std::to_string(h.status) +
+                  ", not LPX_OPTIMAL (step or sync it to OPTIMAL first)");
+        return nullptr;
+    }
+    const double* Tb = (base->pipe && pipe_current_buffer(base, h)) ? B.T1 : B.T;
+    const bool ge = kind == LPX_REOPT_ROW && pay[n] == 1.0;
+    // the terms, and the query's basis, model vectors (b, c: what the sensitivity report of an RHS / COST query
+    // reads) and constraint map
+    std::vector<ReoptTerm> terms;
+    std::vector<int> qb(bb), qmap(base->rmap);
+    std::vector<double> qbv(hb), qcv(hc);
+    double zstart = 0.0;
+    auto slack_terms = [&](const double* d) {
+        for (int i = 0; i < m_in; i++) {
+            if (d[i] == 0.0) continue;
+            const int r = base->rmap[i];
+            const int s1 = n + (r < 0 ? -r - 1 : r);
+            terms.push_back(ReoptTerm{d[i], s1, 0});
+            if (r < 0) terms.push_back(ReoptTerm{d[i], s1 + 1, 1});
+        }
+    };
+    if (kind == LPX_REOPT_RHS) {
+        slack_terms(pay);
+        for (int i = 0; i < m_in; i++) qbv[i] = hb[i] + pay[i];
+    } else if (kind == LPX_REOPT_COST) {
+        std::vector<int> rowof(n, -1);
+        for (int r = 0; r < mb; r++)
+            if (bb[r] < n) rowof[bb[r]] = r;
+        for (int j = 0; j < n; j++) {
+            if (pay[j] == 0.0) continue;
+            terms.push_back(ReoptTerm{base->sense == 1 ? -pay[j] : pay[j], rowof[j], j});
+        }
+        for (int j = 0; j < n; j++) qcv[j] = hc[j] + pay[j];
+    } else if (kind == LPX_REOPT_ROW) {
+        for (int r = 0; r < mb; r++) {
+            const int j = bb[r];
+            if (j >= n || pay[j] == 0.0) continue;
+            terms.push_back(ReoptTerm{ge ? -pay[j] : pay[j], r, 0});
+        }
+        qb.push_back(B.width - 1);  // the new slack is basic in the new row
+        qmap.push_back(mb);
+        qbv.push_back(ge ? -pay[n + 1] : pay[n + 1]);
+    } else {
+        slack_terms(pay);
+        const double cp = base->sense == 1 ? -pay[m_in] : pay[m_in];
+        zstart = -cp;
+        for (int& j : qb)
+            if (j >= n) j++;
+        qcv.push_back(pay[m_in]);
+    }
+    const bool dual = kind == LPX_REOPT_RHS || kind == LPX_REOPT_ROW;
+    const int qm_in = (int)qmap.size(), qn = kind == LPX_REOPT_COL ? n + 1 : n, qmm = (int)qb.size();
+    lpx_session* s = session_new(qm_in, qn, base->sense, qmm, opt ? opt : &base->opt, dual);
+    if (!s) return nullptr;
+    s->rmap = qmap;
+    s->sens_ok = base->sens_ok && (kind == LPX_REOPT_RHS || kind == LPX_REOPT_COST);
+    const size_t stride = lpx_reopt_payload_stride(kind, m_in, n);
+    ReoptTerm* dterms = (ReoptTerm*)sess_alloc(s, std::max<size_t>(terms.size(), 1) * sizeof(ReoptTerm));
+    double* dpay = (double*)sess_alloc(s, stride * 8);
+    if (!dterms || !dpay) {
+        sess_free(s);
+        return nullptr;
+    }
+    StreamParams& P = s->P;
+    cudaStream_t st = s->stream;
+    bool ok = true;
+    ok = ok && (terms.empty() || cudaMemcpyAsync(dterms, terms.data(), terms.size() * sizeof(ReoptTerm),
+                                                 cudaMemcpyHostToDevice, st) == cudaSuccess);
+    ok = ok && cudaMemcpyAsync(dpay, pay, stride * 8, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(P.basis, qb.data(), (size_t)qmm * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(s->sens_b, qbv.data(), (size_t)qm_in * 8, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(s->sens_c, qcv.data(), (size_t)qn * 8, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(s->sens_rmap, qmap.data(), (size_t)qm_in * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    if (ok) {
+        // validate with no constraints only resets StreamCtl to RUNNING, 0 pivots
+        stream_validate_kernel<<<1, 1024, 0, st>>>(P.ctl, nullptr, 0, INT_MAX);
+        const int strips = (P.ld + 255) / 256;
+        const int groups = std::max(1, std::min(P.rows, sm_count() * 8 / strips));
+        stream_reopt_build_kernel<<<dim3(strips, groups, 1), 256, 0, st>>>(P, Tb, B.ld, B.width, mb, n, kind, dterms,
+                                                                            (int)terms.size(), dpay, zstart, ge ? 1 : 0);
+        if (!dual) {
+            stream_first_kernel<<<1, 1024, 0, st>>>(P);
+            count_launch();
+        }
+        stream_gather_kernel<<<(P.rows + 255) / 256, 256, 0, st>>>(P);  // dual: no entering column, the RHS only
+        count_launch(3);
+        ok = cudaGetLastError() == cudaSuccess && cudaStreamSynchronize(st) == cudaSuccess;
+    }
+    if (!ok) {
+        cuda_fail(cudaGetLastError(), "lpx_session_reoptimize: setup", __FILE__, __LINE__);
+        sess_free(s);
+        return nullptr;
+    }
+    return s;
+}
+
 int stream_solve_host(int m, int n, int sense, const double* A, const int* rel, const double* b, const double* c,
                       const lpx_options* opt, int* status, int* n_pivots, int* pivots, int pivots_cap, int* basis,
                       double* x, double* z, double* tableau, double* history, int history_cap) {
@@ -970,6 +1118,20 @@ lpx_session* lpx_session_open(int m, int n, int sense, const double* A, const in
     return s;
 }
 
+lpx_session* lpx_session_reoptimize(const lpx_session* base, int kind, const double* payload, const lpx_options* opt) {
+    if (!base || !payload || kind < LPX_REOPT_RHS || kind > LPX_REOPT_COL) {
+        set_error("lpx_session_reoptimize: bad arguments (NULL base or payload, or an unknown kind)");
+        return nullptr;
+    }
+    if (kind == LPX_REOPT_ROW && payload[base->n] != 0.0 && payload[base->n] != 1.0) {
+        set_error("lpx_session_reoptimize: the added row's rel must be 0 (<=) or 1 (>=)");
+        return nullptr;
+    }
+    if (ensure_device() != LPX_OK) return nullptr;
+    std::lock_guard<std::recursive_mutex> lk(rt().mu);
+    return session_reoptimize(base, kind, payload, opt);
+}
+
 int lpx_session_step_async(lpx_session* s, int max_pivots) {
     if (!s || max_pivots < 0) {
         set_error("lpx_session_step_async: bad arguments");
@@ -1023,10 +1185,7 @@ int lpx_session_profile(lpx_session* s, int n, double* us) {
             LPX_CUDA(cudaEventRecord(ev[3 * k + 2], s->stream));
             continue;
         }
-        if (s->P.npartial > 0)
-            stream_prep_kernel<<<s->P.npartial, LPX_PREP_THREADS, (size_t)s->P.m * 8, s->stream>>>(s->P, 0);
-        else
-            stream_select_kernel<<<1, 1024, 0, s->stream>>>(s->P, 0);
+        launch_select(s, 0);
         LPX_CUDA(cudaEventRecord(ev[3 * k + 1], s->stream));
         stream_update_kernel<4><<<s->grid_update, 256, 0, s->stream>>>(s->P);
         LPX_CUDA(cudaEventRecord(ev[3 * k + 2], s->stream));
@@ -1105,6 +1264,10 @@ int lpx_session_read_tableau(lpx_session* s, double* tableau) {
 int lpx_session_sensitivity(lpx_session* s, double* report) {
     if (!s || !report) {
         set_error("lpx_session_sensitivity: bad arguments");
+        return LPX_E_BAD_ARGS;
+    }
+    if (!s->sens_ok) {
+        set_error("lpx_session_sensitivity: not defined for the query session of an added row or column");
         return LPX_E_BAD_ARGS;
     }
     std::lock_guard<std::recursive_mutex> lk(rt().mu);
