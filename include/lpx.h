@@ -65,7 +65,11 @@ typedef struct lpx_options {
     int knap_spec_depth;  /* knapsack B&B: look-ahead depth under the front runner (0 = default 2) */
     int stream_protocol;  /* streaming kernels: 0 auto (pipelined blocked look-ahead: the look-ahead of block
                              B+1 overlaps the HBM pass of block B), 1 single-CTA select per pivot, 2 multi-CTA
-                             prep per pivot, 3 blocked with a one-CTA look-ahead, 4 blocked, not pipelined */
+                             prep per pivot, 3 blocked with a one-CTA look-ahead, 4 blocked, not pipelined.
+                             Dual Simplex sessions (lpx_dual_session_open, RHS / ROW re-optimization queries):
+                             1 and 2 one pivot per HBM pass; 0, 3 and 4 the blocked dual look-ahead (one CTA
+                             decides stream_block pivots, one HBM pass applies them; not pipelined), or one
+                             pivot per pass when the look-ahead's shared-memory carve does not fit */
     int reg_variant;      /* register-resident kernel: 0 = default build (4 when n <= 128, else 2), 1 one CTA per SM
                              (all registers), 2 two CTAs per SM (two column slots in shared memory), 3 three CTAs per
                              SM (four slots), 4 condensed tableau (non-basic columns only), three CTAs per SM, 8 row
@@ -131,7 +135,9 @@ int lpx_primal_solve_batched_dev(int count, int m, int n, int sense, const doubl
 
 /* ---- Dual Simplex: DualSimplex.Solve, R/Models/DualSimplex.cs:15-114 ------------------------ */
 /* pivots lists the *silent ForceDualFeasibility pivots first (R/Models/DualSimplex.cs:195-228);
- * history[0] is the tableau after them ("Iteration 0"). */
+ * history[0] is the tableau after them ("Iteration 0").  opt.kernel AUTO routes as lpx_primal_solve does (per-CTA
+ * kernels while the tableau fits shared memory or has at most 96 K elements, else a Dual Simplex session on the whole
+ * GPU; with history the per-CTA global-memory kernel); LPX_KERNEL_STREAM forces the session (history: E_CAPACITY). */
 int lpx_dual_solve(int m, int n, int sense, const double* A, const int* rel, const double* b, const double* c,
                    const lpx_options* opt, int* status, int* n_pivots, int* silent_pivots, int* pivots,
                    int pivots_cap, int* basis, double* x, double* z, double* tableau, double* history,
@@ -157,6 +163,22 @@ int lpx_session_read_tableau(lpx_session* s, double* tableau);          /* rows 
 int lpx_session_read_solution(lpx_session* s, int* basis, double* x, double* z);
 int lpx_session_read_pivots(lpx_session* s, int* pivots, int pivots_cap);
 void lpx_session_close(lpx_session* s);
+/* Dual Simplex (DualSimplex.Solve, R/Models/DualSimplex.cs:15-114) on a large LP whose tableau lives in HBM: the rules
+ * of lpx_dual_solve, bit for bit.  Open prepares the rows (PrepareForTableau: Min costs negated; an EQ row as given,
+ * then negated; a GE row negated unless -b < -1e-9; an LE row negated when b < -1e-9; no GE / negative-RHS
+ * validation), builds the tableau and runs the silent ForceDualFeasibility phase (at most 100 Primal Simplex pivots,
+ * ratio margin 1e-12) synchronously.  Silent pivots come first in the pivot log and count in pivots_total; step / sync
+ * then run the Dual Simplex loop (OPTIMAL / INFEASIBLE, or LPX_S_ITER_LIMIT after 10000 Dual Simplex pivots,
+ * independent of opt.max_iterations).  opt.stream_protocol / stream_block / stream_pass_variant choose the protocol
+ * (see lpx_options).  Every other session call works on it; lpx_session_sensitivity returns LPX_E_BAD_ARGS and
+ * lpx_session_reoptimize returns NULL for it.  NULL (lpx_last_error() says why) for bad arguments. */
+lpx_session* lpx_dual_session_open(int m, int n, int sense, const double* A, const int* rel, const double* b,
+                                   const double* c, const lpx_options* opt);
+/* A, b, c are DEVICE pointers, rel a host pointer; b is read back once for the row signs. */
+lpx_session* lpx_dual_session_open_dev(int m, int n, int sense, const double* A, const int* rel, const double* b,
+                                       const double* c, const lpx_options* opt);
+/* Silent ForceDualFeasibility pivots of a Dual Simplex session; 0 for every other session. */
+int lpx_session_silent_pivots(const lpx_session* s, int* silent);
 
 /* ---- Branch & Bound (simplex): BranchAndBound.Solve, R/Models/Branch&Bound.cs:30-123 -------- */
 /* One record per LP relaxation the reference solves (root LP, then every SolveNode call), in the
@@ -385,8 +407,9 @@ int lpx_reoptimize(int kind, int m, int n, int sense, const double* A, const int
  * stepped, read or re-queried afterwards; several query sessions of one base may be open at once.  kind / payload
  * (host pointer, lpx_reopt_payload_stride(kind, m, n) doubles, m / n the base model's) are the definition above; the
  * edit is applied to the base's current tableau and basis, and the query's results equal oracle/orc_reopt.cpp on them
- * bit for bit.  RHS / ROW run the Dual Simplex rules (limit 10000) one pivot per HBM pass; COST / COL run the Primal
- * Simplex rules with opt's max_iterations and stream protocol, as lpx_session_open does.  opt NULL: the base's options.
+ * bit for bit.  RHS / ROW run the Dual Simplex rules (limit 10000) with opt's stream protocol (see lpx_options: the
+ * blocked dual look-ahead or one pivot per HBM pass); COST / COL run the Primal Simplex rules with opt's max_iterations
+ * and stream protocol, as lpx_session_open does.  opt NULL: the base's options.
  * NULL (lpx_last_error() says why) when the base's status, as of its last step / sync, is not LPX_OPTIMAL, for an
  * unknown kind, a ROW rel other than 0 / 1, or a NULL base / payload.  The query is read with the session calls:
  * step / sync run its loop, pivots count from 0, dims give its shape (ROW: rows + 1; ROW / COL: cols + 1),

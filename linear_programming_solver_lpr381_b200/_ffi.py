@@ -33,7 +33,8 @@ EXPORTS = [
     "lpx_reset_counters", "lpx_revised_solve", "lpx_revised_history_stride", "lpx_measure_fp64_rate", "lpx_measure_latencies", "lpx_session_profile", "lpx_session_debug_stamps",
     "lpx_bnb_last_stats", "lpx_bnb_pooled", "lpx_sensitivity_stride", "lpx_sensitivity_batched_dev",
     "lpx_primal_solve_sensitivity_batched", "lpx_session_sensitivity", "lpx_reopt_payload_stride", "lpx_reopt_dims",
-    "lpx_reoptimize_batched_dev", "lpx_reoptimize", "lpx_session_reoptimize",
+    "lpx_reoptimize_batched_dev", "lpx_reoptimize", "lpx_session_reoptimize", "lpx_dual_session_open",
+    "lpx_dual_session_open_dev", "lpx_session_silent_pivots",
 ]
 
 
@@ -107,6 +108,10 @@ def lib():
                                    C.c_void_p]
     L.lpx_session_open_dev.restype = C.c_void_p
     L.lpx_session_open_dev.argtypes = L.lpx_session_open.argtypes
+    for f in ("lpx_dual_session_open", "lpx_dual_session_open_dev"):
+        getattr(L, f).restype = C.c_void_p
+        getattr(L, f).argtypes = L.lpx_session_open.argtypes
+    L.lpx_session_silent_pivots.argtypes = [C.c_void_p, _ip]
     L.lpx_session_stream.restype = C.c_void_p
     L.lpx_session_stream.argtypes = [C.c_void_p]
     for f in ("lpx_session_step",):
@@ -178,6 +183,7 @@ def make_options(max_iterations=10000, kernel=KERNEL_AUTO, threads=0, spec_nodes
     o.knap_spec_nodes = spec_nodes
     o.knap_spec_depth = spec_depth
     o.stream_protocol = single_cta_select  # 0 blocked look-ahead (cluster), 3 blocked (one CTA), 1 / 2 per pivot
+    # (Dual Simplex sessions: 0 / 3 / 4 the blocked dual look-ahead, 1 / 2 per pivot)
     o.reg_variant = reg_variant
     o.stream_block = kblock
     o.stream_pass_variant = pass_variant

@@ -245,27 +245,34 @@ def reoptimize_batched_dev(kind, count, m, n, sense, drel, dbase_status, dbase_b
 
 
 class Session:
-    """Large single LP whose tableau lives in HBM (lpx_session_*)."""
+    """Large single LP whose tableau lives in HBM (lpx_session_*).  dual=True: DualSimplex.Solve on the model
+    (lpx_dual_session_open); the silent ForceDualFeasibility pivots run inside the constructor and `.silent` counts
+    them.  A Dual Simplex session has no sensitivity report and cannot be a re-optimization base."""
 
     def __init__(self, A, b, c, rel=None, sense=0, max_iterations=10000, device_ptrs=False, m=None, n=None,
-                 single_cta_select=0, kblock=0, pass_variant=0):
+                 single_cta_select=0, kblock=0, pass_variant=0, dual=False):
         opt = F.make_options(max_iterations, single_cta_select=single_cta_select, kblock=kblock,
                              pass_variant=pass_variant)
+        L = F.lib()
         if device_ptrs:
             self.m, self.n = m, n
             relp = None if rel is None else np.ascontiguousarray(rel, dtype=np.int32)
-            self._h = F.lib().lpx_session_open_dev(m, n, sense, F.ptr(A), F.ptr(relp), F.ptr(b), F.ptr(c),
-                                                   C.cast(C.byref(opt), C.c_void_p))
+            open_dev = L.lpx_dual_session_open_dev if dual else L.lpx_session_open_dev
+            self._h = open_dev(m, n, sense, F.ptr(A), F.ptr(relp), F.ptr(b), F.ptr(c), C.cast(C.byref(opt), C.c_void_p))
         else:
             A, b, c, rel = _prep(A, b, c, rel)
             self.m, self.n = A.shape
-            self._h = F.lib().lpx_session_open(self.m, self.n, sense, F.ptr(A), F.ptr(rel), F.ptr(b), F.ptr(c),
-                                               C.cast(C.byref(opt), C.c_void_p))
+            open_host = L.lpx_dual_session_open if dual else L.lpx_session_open
+            self._h = open_host(self.m, self.n, sense, F.ptr(A), F.ptr(rel), F.ptr(b), F.ptr(c),
+                                C.cast(C.byref(opt), C.c_void_p))
         if not self._h:
             raise F.LpxError(F.E_CUDA, F.last_error())
         r, cc = C.c_int(), C.c_int()
-        F.check(F.lib().lpx_session_dims(self._h, C.byref(r), C.byref(cc)))
+        F.check(L.lpx_session_dims(self._h, C.byref(r), C.byref(cc)))
         self.rows, self.cols = r.value, cc.value
+        silent = C.c_int()
+        F.check(L.lpx_session_silent_pivots(self._h, C.byref(silent)))
+        self.dual, self.silent = dual, silent.value
 
     def step(self, max_pivots):
         st, tot = C.c_int(), C.c_int()
@@ -313,6 +320,7 @@ class Session:
             raise F.LpxError(F.E_BAD_ARGS, F.last_error())
         q = Session.__new__(Session)
         q._h = h
+        q.dual, q.silent = False, 0
         q.m = self.m + (kind == F.REOPT_ROW)
         q.n = self.n + (kind == F.REOPT_COL)
         r, cc = C.c_int(), C.c_int()

@@ -117,6 +117,15 @@ namespace Linear_Programming_Solver.Models
         [DllImport(Lib)]
         public static extern IntPtr lpx_session_reoptimize(IntPtr base_session, int kind, double[] payload, IntPtr opt);
 
+        // Dual Simplex on a large LP in HBM (DualSimplex.Solve as lpx_dual_solve computes it); IntPtr.Zero on refusal.
+        [DllImport(Lib)]
+        public static extern IntPtr lpx_dual_session_open(int m, int n, int sense, double[] A, int[] rel, double[] b,
+            double[] c, ref LpxOptions opt);
+        [DllImport(Lib)]
+        public static extern IntPtr lpx_dual_session_open_dev(int m, int n, int sense, IntPtr A, int[] rel, IntPtr b,
+            IntPtr c, ref LpxOptions opt);
+        [DllImport(Lib)] public static extern int lpx_session_silent_pivots(IntPtr session, out int silent);
+
         [DllImport(Lib)]
         public static extern int lpx_primal_solve_batched(int count, int m, int n, int sense, double[] A, int[] rel,
             double[] b, double[] c, ref LpxOptions opt, int[] status, int[] n_pivots, int[] basis, double[] x,

@@ -20,6 +20,7 @@
 #define LPX_MARGIN_PRIMAL 1e-9  // PrimalSimplex.cs:235
 #define LPX_MARGIN_DUAL 1e-12   // DualSimplex.cs:85,220
 #define LPX_DUAL_MAX_ITER 10000  // DualSimplex.cs:39: a literal, independent of PrimalSimplex.MaxIterations
+#define LPX_DUAL_SILENT_MAX 100  // DualSimplex.cs:195-228: ForceDualFeasibility's guard
 
 namespace lpx {
 

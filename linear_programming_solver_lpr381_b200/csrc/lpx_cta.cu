@@ -428,6 +428,18 @@ static int primal_batched_pipeline(int count, int m, int n, int sense, const dou
     return result;
 }
 
+// opt.kernel AUTO for one LP (lpx_primal_solve, lpx_dual_solve): the per-CTA kernels win while the tableau is small;
+// past that a single SM cannot stream it fast enough and the whole-GPU streaming kernels take over.
+static int single_auto_kernel(int mm, int n, bool want_history) {
+    const size_t elems = (size_t)(mm + 1) * (n + mm + 1);
+    int kernel = (cta_fits_smem(mm + 1, n + mm + 1) || elems <= (size_t)96 * 1024) ? LPX_KERNEL_CTA_SMEM
+                                                                                    : LPX_KERNEL_STREAM;
+    if (kernel == LPX_KERNEL_CTA_SMEM && !cta_fits_smem(mm + 1, n + mm + 1))
+        kernel = cta_cluster_size_for(mm + 1, n + mm + 1) ? LPX_KERNEL_CTA_CLUSTER : LPX_KERNEL_CTA_GLOBAL;
+    if (want_history && kernel == LPX_KERNEL_STREAM) kernel = LPX_KERNEL_CTA_GLOBAL;
+    return kernel;
+}
+
 }  // namespace lpx
 
 using namespace lpx;
@@ -443,16 +455,7 @@ int lpx_primal_solve(int m, int n, int sense, const double* A, const int* rel, c
     std::lock_guard<std::recursive_mutex> lk(rt().mu);
     const int mm = expanded_rows(m, rel);
     int kernel = opt ? opt->kernel : LPX_KERNEL_AUTO;
-    if (kernel == LPX_KERNEL_AUTO) {
-        // one tableau: the per-CTA kernels win while the tableau is small; past that a single SM
-        // cannot stream it fast enough and the whole-GPU streaming kernels take over.
-        const size_t elems = (size_t)(mm + 1) * (n + mm + 1);
-        kernel = (cta_fits_smem(mm + 1, n + mm + 1) || elems <= (size_t)96 * 1024) ? LPX_KERNEL_CTA_SMEM
-                                                                                    : LPX_KERNEL_STREAM;
-        if (kernel == LPX_KERNEL_CTA_SMEM && !cta_fits_smem(mm + 1, n + mm + 1))
-            kernel = cta_cluster_size_for(mm + 1, n + mm + 1) ? LPX_KERNEL_CTA_CLUSTER : LPX_KERNEL_CTA_GLOBAL;
-        if (history && history_cap > 0 && kernel == LPX_KERNEL_STREAM) kernel = LPX_KERNEL_CTA_GLOBAL;
-    }
+    if (kernel == LPX_KERNEL_AUTO) kernel = single_auto_kernel(mm, n, history && history_cap > 0);
     if (kernel == LPX_KERNEL_STREAM)
         return stream_solve_host(m, n, sense, A, rel, b, c, opt, status, n_pivots, pivots, pivots_cap, basis, x, z,
                                  tableau, history, history_cap);
@@ -475,10 +478,10 @@ int lpx_dual_solve(int m, int n, int sense, const double* A, const int* rel, con
     lpx_options o;
     lpx_default_options(&o);
     if (opt) o = *opt;
-    if (o.kernel == LPX_KERNEL_STREAM) {
-        set_error("lpx_dual_solve runs on the per-CTA kernels only");
-        return LPX_E_BAD_ARGS;
-    }
+    if (o.kernel == LPX_KERNEL_AUTO) o.kernel = single_auto_kernel(expanded_rows(m, rel), n, history && history_cap > 0);
+    if (o.kernel == LPX_KERNEL_STREAM)
+        return stream_dual_solve_host(m, n, sense, A, rel, b, c, &o, status, n_pivots, silent_pivots, pivots,
+                                      pivots_cap, basis, x, z, tableau, history, history_cap);
     return solve_single_cta(1, m, n, sense, A, rel, b, c, &o, status, n_pivots, silent_pivots, pivots, pivots_cap,
                             basis, x, z, tableau, history, history_cap);
 }

@@ -171,7 +171,11 @@ __global__ void __launch_bounds__(256) stream_gather_kernel(StreamParams P) {
 
 // ---- per-pivot kernels ------------------------------------------------------------------------
 
+// FORCE: the ratio margin of DualSimplex.ForceDualFeasibility (1e-12) instead of PrimalSimplex's (1e-9), for the silent
+// Primal Simplex pivots that open a Dual Simplex session (session_dual_silent_phase).
+template <bool FORCE>
 __global__ void __launch_bounds__(1024) stream_select_kernel(StreamParams P, int probe_only) {
+    constexpr double margin = FORCE ? LPX_MARGIN_DUAL : LPX_MARGIN_PRIMAL;
     __shared__ ArgMin red[34];
     __shared__ int ired[34];
     StreamCtl* ctl = P.ctl;
@@ -199,7 +203,7 @@ __global__ void __launch_bounds__(1024) stream_select_kernel(StreamParams P, int
         P.ratio[i] = r;
     }
     __syncthreads();
-    // ... then the reference's sequential rule "take i if ratio < best - 1e-9", reproduced exactly:
+    // ... then the reference's sequential rule "take i if ratio < best - margin", reproduced exactly:
     // repeatedly find the FIRST row after the last accepted one that beats the running best.
     // The number of rounds is the number of accepted updates (about ln m on random data).
     const int R = (m + 1023) / 1024;
@@ -207,7 +211,7 @@ __global__ void __launch_bounds__(1024) stream_select_kernel(StreamParams P, int
     double best = __longlong_as_double(0x7ff0000000000000LL);
     int row = -1, start = 0;
     while (true) {
-        const double thr = __dsub_rn(best, LPX_MARGIN_PRIMAL);
+        const double thr = __dsub_rn(best, margin);
         int cand = INT_MAX;
         for (int i = max(lo, start); i < hi; i++)
             if (P.ratio[i] < thr) {
@@ -477,6 +481,7 @@ __global__ void __launch_bounds__(256, 4) stream_update_kernel(StreamParams P) {
 #include "lpx_stream_block.cuh"
 #include "lpx_stream_pipe.cuh"
 #include "lpx_stream_reopt.cuh"
+#include "lpx_stream_dual.cuh"
 
 
 // ---- session object -----------------------------------------------------------------------------
@@ -497,7 +502,9 @@ struct lpx_session {
     int* sens_rmap = nullptr;
     std::vector<int> rmap;  // host copy of sens_rmap: constraint i -> expanded row i1 (EQ: -i1 - 1)
     bool sens_ok = true;    // false for ROW / COL re-optimization queries and their descendants
-    bool dual = false;      // Dual Simplex per-pivot protocol (RHS / ROW re-optimization queries)
+    bool dual = false;      // Dual Simplex rules (RHS / ROW re-optimization queries, Dual Simplex sessions)
+    bool dual_model = false;  // opened by lpx_dual_session_open(_dev): DualSimplex.Solve on the model
+    int silent = 0;           // ForceDualFeasibility pivots performed inside lpx_dual_session_open
     int* sens_rowof = nullptr;
     void* sens_partial = nullptr;
     double* sens_report = nullptr;
@@ -551,7 +558,7 @@ static void launch_select(lpx_session* s, int probe_only) {
     else if (s->P.npartial > 0)
         stream_prep_kernel<<<s->P.npartial, LPX_PREP_THREADS, (size_t)s->P.m * 8, s->stream>>>(s->P, probe_only);
     else
-        stream_select_kernel<<<1, 1024, 0, s->stream>>>(s->P, probe_only);
+        stream_select_kernel<false><<<1, 1024, 0, s->stream>>>(s->P, probe_only);
 }
 
 static int launch_pair(lpx_session* s, int probe_only) {
@@ -575,7 +582,9 @@ static size_t lookahead_cluster_smem(const StreamParams& P) {
 }
 
 static void launch_lookahead(lpx_session* s, int budget) {
-    if (s->la_cluster)
+    if (s->dual)
+        stream_dual_lookahead_kernel<<<1, 1024, dual_lookahead_smem(s->P), s->stream>>>(s->P, budget);
+    else if (s->la_cluster)
         stream_lookahead_cluster_kernel<<<LPX_LA_CLUSTER, LPX_LA_THREADS, lookahead_cluster_smem(s->P), s->stream>>>(
             s->P, budget);
     else
@@ -693,8 +702,11 @@ static int launch_block(lpx_session* s, int budget) {
 
 // A session of mm tableau rows (after EQ expansion) and n decision variables, shared by the sessions built from
 // (A, b, c) and the re-optimization queries built from a base: the stream, the sizing, every buffer, the protocol
-// and the launch grids.  dual: the Dual Simplex per-pivot protocol (stream_dual_select_kernel + the per-pivot pass,
-// limit 10000); otherwise opt's Primal Simplex protocol.  m_in / n: the model's constraints and variables (b, c).
+// and the launch grids.  dual: the Dual Simplex rules (limit 10000 dual pivots; the pivot log also holds the up to
+// 100 silent pivots of a Dual Simplex session) with the blocked dual look-ahead (stream_dual_lookahead_kernel + the
+// blocked pass) or, for stream_protocol 1 / 2 or when its carve does not fit, the per-pivot protocol
+// (stream_dual_select_kernel + stream_update_kernel<4>); otherwise opt's Primal Simplex protocol.  m_in / n: the
+// model's constraints and variables (b, c).
 static lpx_session* session_new(int m_in, int n, int sense, int mm, const lpx_options* opt, bool dual) {
     lpx_session* s = new lpx_session();
     lpx_default_options(&s->opt);
@@ -719,7 +731,7 @@ static lpx_session* session_new(int m_in, int n, int sense, int mm, const lpx_op
     P.ld = (P.width + 15) & ~15;
     P.colstride = (P.rows + 15) & ~15;
     P.max_iter = dual ? LPX_DUAL_MAX_ITER : s->opt.max_iterations;
-    P.pivlog_cap = std::max(1, std::min(P.max_iter, 1 << 20));
+    P.pivlog_cap = std::max(1, std::min(P.max_iter, 1 << 20)) + (dual ? LPX_DUAL_SILENT_MAX : 0);
     const size_t tbytes = (size_t)P.rows * P.ld * 8;
     P.T = (double*)sess_alloc(s, tbytes);
     P.colbuf = (double*)sess_alloc(s, (size_t)2 * P.colstride * 8);
@@ -758,6 +770,15 @@ static lpx_session* session_new(int m_in, int n, int sense, int mm, const lpx_op
                                         (int)lookahead_smem(P)) == cudaSuccess) {
             P.kblock = kb;
         }
+        cudaGetLastError();
+    }
+    if (dual && (s->opt.stream_protocol == 0 || s->opt.stream_protocol == 3 || s->opt.stream_protocol == 4)) {
+        // blocked dual look-ahead: one CTA, not pipelined; z-row + compact RHS + one column in shared memory
+        const int kb = s->opt.stream_block > 0 ? std::min(s->opt.stream_block, LPX_BLOCK_KMAX) : 8;
+        if (dual_lookahead_smem(P) + 4096 <= (size_t)max_smem_optin() &&
+            cudaFuncSetAttribute(stream_dual_lookahead_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)dual_lookahead_smem(P)) == cudaSuccess)
+            P.kblock = kb;
         cudaGetLastError();
     }
     if (dual || s->opt.stream_protocol == 1) P.npartial = 0;
@@ -888,12 +909,51 @@ static lpx_session* session_new(int m_in, int n, int sense, int mm, const lpx_op
     return s;
 }
 
-// A, b, c: device pointers valid until this call returns (setup runs synchronously).
+// The silent phase of a Dual Simplex session (DualSimplex.ForceDualFeasibility): at most 100 Primal Simplex pivots with
+// the ratio margin 1e-12, on the per-pivot single-CTA primal protocol.  It ends, with no status, on no entering column,
+// no leaving row or the guard; the select kernel marks those OPTIMAL / UNBOUNDED / ITER_LIMIT (with max_iter = 100
+// during the phase) and makes every later launch of the phase a no-op, so the 100 pairs are enqueued at once and the
+// control block is re-armed for the Dual Simplex loop afterwards.  Runs synchronously, inside open.
+static int session_dual_silent_phase(lpx_session* s) {
+    StreamParams F = s->P;
+    F.max_iter = LPX_DUAL_SILENT_MAX;
+    F.npartial = 0;
+    cudaStream_t st = s->stream;
+    stream_first_kernel<<<1, 1024, 0, st>>>(F);
+    stream_gather_kernel<<<(F.rows + 255) / 256, 256, 0, st>>>(F);
+    count_launch(2);
+    for (int k = 0; k < LPX_DUAL_SILENT_MAX; k++) {
+        stream_select_kernel<true><<<1, 1024, 0, st>>>(F, 0);
+        stream_update_kernel<4><<<s->grid_update, 256, 0, st>>>(F);
+        count_launch(2);
+    }
+    LPX_CUDA(cudaGetLastError());
+    StreamCtl h;
+    LPX_CUDA(cudaMemcpyAsync(&h, F.ctl, sizeof h, cudaMemcpyDeviceToHost, st));
+    LPX_CUDA(cudaStreamSynchronize(st));
+    s->silent = h.pivots;
+    h.status = LPX_RUNNING;
+    h.enter = -1;
+    h.leave = -1;
+    h.active = 0;
+    h.capture = -1;
+    h.block_cnt = 0;
+    LPX_CUDA(cudaMemcpyAsync(F.ctl, &h, sizeof h, cudaMemcpyHostToDevice, st));
+    LPX_CUDA(cudaStreamSynchronize(st));
+    s->P.max_iter = s->silent + LPX_DUAL_MAX_ITER;  // the limit counts Dual Simplex pivots only
+    return LPX_OK;
+}
+
+// A, b, c: device pointers valid until this call returns (setup runs synchronously).  dual: a Dual Simplex session
+// (DualSimplex.Solve); hb is then b on the host, for the row signs of DualSimplex.PrepareForTableau.
 static lpx_session* session_create(int m, int n, int sense, const double* dA, const int* rel, const double* db,
-                                   const double* dc, const lpx_options* opt) {
+                                   const double* dc, const lpx_options* opt, bool dual = false,
+                                   const double* hb = nullptr) {
     if (ensure_device() != LPX_OK) return nullptr;
     std::lock_guard<std::recursive_mutex> lk(rt().mu);
-    // row map of the EQ expansion, and the first '>=' row, both known from rel on the host
+    // row map of the EQ expansion, and the first '>=' row, both known from rel on the host.  Dual Simplex row signs
+    // (PrepareForTableau): an EQ row as given, then negated; a GE row negated, then negated back when the negated b is
+    // below -1e-9 (so flipped unless -b < -1e-9); an LE row negated when b < -1e-9.  No GE / negative-RHS validation.
     std::vector<int> rsrc, rsgn, rmap;
     int first_ge = INT_MAX;
     for (int r = 0; r < m; r++) {
@@ -901,16 +961,21 @@ static lpx_session* session_create(int m, int n, int sense, const double* dA, co
         if (rl == 1 && first_ge == INT_MAX) first_ge = r;
         rmap.push_back(rl == 2 ? -(int)rsrc.size() - 1 : (int)rsrc.size());
         rsrc.push_back(r);
-        rsgn.push_back(0);
+        int flip = 0;
+        if (dual && rl == 1) flip = !(-hb[r] < -LPX_EPS);
+        if (dual && rl == 0) flip = hb[r] < -LPX_EPS;
+        rsgn.push_back(flip);
         if (rl == 2) {
             rsrc.push_back(r);
             rsgn.push_back(1);
         }
     }
     const int mm = (int)rsrc.size();
-    lpx_session* s = session_new(m, n, sense, mm, opt, false);
+    lpx_session* s = session_new(m, n, sense, mm, opt, dual);
     if (!s) return nullptr;
     s->rmap = rmap;
+    s->dual_model = dual;
+    s->sens_ok = !dual;
     StreamParams& P = s->P;
     int* drsrc = (int*)sess_alloc(s, (size_t)mm * 4);
     int* drsgn = (int*)sess_alloc(s, (size_t)mm * 4);
@@ -925,7 +990,14 @@ static lpx_session* session_create(int m, int n, int sense, const double* dA, co
     ok = ok && cudaMemcpyAsync(s->sens_b, db, (size_t)m * 8, cudaMemcpyDeviceToDevice, st) == cudaSuccess;
     ok = ok && cudaMemcpyAsync(s->sens_c, dc, (size_t)n * 8, cudaMemcpyDeviceToDevice, st) == cudaSuccess;
     ok = ok && cudaMemcpyAsync(s->sens_rmap, rmap.data(), (size_t)m * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
-    if (ok) {
+    if (ok && dual) {
+        // validate with no constraints only resets StreamCtl to RUNNING, 0 pivots
+        stream_validate_kernel<<<1, 1024, 0, st>>>(P.ctl, nullptr, 0, INT_MAX);
+        const int bgrid = std::min(P.rows, sm_count() * 8);
+        stream_build_kernel<<<bgrid, 256, 0, st>>>(P, dA, db, dc, drsrc, drsgn, sense);
+        count_launch(2);
+        ok = cudaGetLastError() == cudaSuccess && session_dual_silent_phase(s) == LPX_OK;
+    } else if (ok) {
         stream_validate_kernel<<<1, 1024, 0, st>>>(P.ctl, db, m, first_ge);
         const int bgrid = std::min(P.rows, sm_count() * 8);
         stream_build_kernel<<<bgrid, 256, 0, st>>>(P, dA, db, dc, drsrc, drsgn, sense);
@@ -947,6 +1019,11 @@ static lpx_session* session_create(int m, int n, int sense, const double* dA, co
 // writes the query's tableau straight from the base's current buffer, then the query's protocol is armed as a new
 // session's is.  The base is only read, and is idle once this returns (setup runs synchronously).
 static lpx_session* session_reoptimize(const lpx_session* base, int kind, const double* pay, const lpx_options* opt) {
+    if (base->dual_model) {
+        set_error("lpx_session_reoptimize: the base is a Dual Simplex session; re-optimization is defined for Primal "
+                  "Simplex results");
+        return nullptr;
+    }
     const StreamParams& B = base->P;
     const int m_in = base->m_in, n = base->n, mb = B.m;
     StreamCtl h;
@@ -1080,9 +1157,91 @@ int stream_solve_host(int m, int n, int sense, const double* A, const int* rel, 
     return rc;
 }
 
+// lpx_dual_solve with kernel = LPX_KERNEL_STREAM: one Dual Simplex session stepped to its terminal status.
+int stream_dual_solve_host(int m, int n, int sense, const double* A, const int* rel, const double* b, const double* c,
+                           const lpx_options* opt, int* status, int* n_pivots, int* silent_pivots, int* pivots,
+                           int pivots_cap, int* basis, double* x, double* z, double* tableau, double* history,
+                           int history_cap) {
+    if (history && history_cap > 0) {
+        set_error("per-iteration history is not available on the streaming kernel; use LPX_KERNEL_CTA_GLOBAL");
+        return LPX_E_CAPACITY;
+    }
+    lpx_session* s = lpx_dual_session_open(m, n, sense, A, rel, b, c, opt);
+    if (!s) return LPX_E_CUDA;
+    int st = LPX_RUNNING, np = 0, rc = LPX_OK;
+    while (st == LPX_RUNNING && rc == LPX_OK) rc = lpx_session_step(s, 512, &st, &np);
+    if (rc == LPX_OK) {
+        if (status) *status = st;
+        if (n_pivots) *n_pivots = np;
+        if (silent_pivots) *silent_pivots = s->silent;
+        if (pivots && pivots_cap > 0) rc = lpx_session_read_pivots(s, pivots, pivots_cap);
+        const bool solved = st >= 0 || st == LPX_S_ITER_LIMIT;
+        if (rc == LPX_OK && solved && (basis || x || z)) rc = lpx_session_read_solution(s, basis, x, z);
+        if (rc == LPX_OK && solved && tableau) rc = lpx_session_read_tableau(s, tableau);
+    }
+    lpx_session_close(s);
+    return rc;
+}
+
 }  // namespace lpx
 
 extern "C" {
+
+static bool dual_open_args_ok(const char* who, int m, int n, int sense, const double* A, const int* rel,
+                              const double* b, const double* c) {
+    bool ok = m >= 1 && n >= 1 && A && b && c && (sense == 0 || sense == 1);
+    for (int i = 0; ok && rel && i < m; i++) ok = rel[i] >= 0 && rel[i] <= 2;
+    if (!ok) set_error(std::string(who) + ": bad arguments (need m >= 1, n >= 1, sense 0 / 1, non-null A, b, c, rel[i] "
+                                          "in 0..2)");
+    return ok;
+}
+
+lpx_session* lpx_dual_session_open_dev(int m, int n, int sense, const double* A, const int* rel, const double* b,
+                                       const double* c, const lpx_options* opt) {
+    if (!dual_open_args_ok("lpx_dual_session_open_dev", m, n, sense, A, rel, b, c)) return nullptr;
+    if (ensure_device() != LPX_OK) return nullptr;
+    std::lock_guard<std::recursive_mutex> lk(rt().mu);
+    // the row signs need b on the host
+    std::vector<double> hb(m);
+    cudaStream_t st = rt().stream;
+    if (cudaMemcpyAsync(hb.data(), b, (size_t)m * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess) {
+        cuda_fail(cudaGetLastError(), "lpx_dual_session_open_dev: reading b", __FILE__, __LINE__);
+        return nullptr;
+    }
+    return session_create(m, n, sense, A, rel, b, c, opt, true, hb.data());
+}
+
+lpx_session* lpx_dual_session_open(int m, int n, int sense, const double* A, const int* rel, const double* b,
+                                   const double* c, const lpx_options* opt) {
+    if (!dual_open_args_ok("lpx_dual_session_open", m, n, sense, A, rel, b, c)) return nullptr;
+    if (ensure_device() != LPX_OK) return nullptr;
+    std::lock_guard<std::recursive_mutex> lk(rt().mu);
+    double *dA = nullptr, *db = nullptr, *dc = nullptr;
+    lpx_session* s = nullptr;
+    if (cudaMalloc(&dA, (size_t)m * n * 8) == cudaSuccess && cudaMalloc(&db, (size_t)m * 8) == cudaSuccess &&
+        cudaMalloc(&dc, (size_t)n * 8) == cudaSuccess &&
+        cudaMemcpy(dA, A, (size_t)m * n * 8, cudaMemcpyHostToDevice) == cudaSuccess &&
+        cudaMemcpy(db, b, (size_t)m * 8, cudaMemcpyHostToDevice) == cudaSuccess &&
+        cudaMemcpy(dc, c, (size_t)n * 8, cudaMemcpyHostToDevice) == cudaSuccess) {
+        s = session_create(m, n, sense, dA, rel, db, dc, opt, true, b);
+    } else {
+        cuda_fail(cudaGetLastError(), "lpx_dual_session_open: staging inputs", __FILE__, __LINE__);
+    }
+    cudaFree(dA);
+    cudaFree(db);
+    cudaFree(dc);
+    return s;
+}
+
+int lpx_session_silent_pivots(const lpx_session* s, int* silent) {
+    if (!s || !silent) {
+        set_error("lpx_session_silent_pivots: bad arguments");
+        return LPX_E_BAD_ARGS;
+    }
+    *silent = s->silent;
+    return LPX_OK;
+}
 
 lpx_session* lpx_session_open_dev(int m, int n, int sense, const double* A, const int* rel, const double* b,
                                   const double* c, const lpx_options* opt) {
@@ -1264,6 +1423,11 @@ int lpx_session_read_tableau(lpx_session* s, double* tableau) {
 int lpx_session_sensitivity(lpx_session* s, double* report) {
     if (!s || !report) {
         set_error("lpx_session_sensitivity: bad arguments");
+        return LPX_E_BAD_ARGS;
+    }
+    if (s->dual_model) {
+        set_error("lpx_session_sensitivity: not defined for a Dual Simplex session (its tableau treats '>=' rows as "
+                  "'<='); the report is defined for Primal Simplex results");
         return LPX_E_BAD_ARGS;
     }
     if (!s->sens_ok) {

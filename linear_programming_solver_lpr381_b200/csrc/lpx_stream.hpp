@@ -10,6 +10,11 @@ namespace lpx {
 int stream_solve_host(int m, int n, int sense, const double* A, const int* rel, const double* b, const double* c,
                       const lpx_options* opt, int* status, int* n_pivots, int* pivots, int pivots_cap, int* basis,
                       double* x, double* z, double* tableau, double* history, int history_cap);
+// the same for the Dual Simplex (lpx_dual_session_open)
+int stream_dual_solve_host(int m, int n, int sense, const double* A, const int* rel, const double* b, const double* c,
+                           const lpx_options* opt, int* status, int* n_pivots, int* silent_pivots, int* pivots,
+                           int pivots_cap, int* basis, double* x, double* z, double* tableau, double* history,
+                           int history_cap);
 
 // register-resident batched kernel (lpx_reg.cu)
 bool reg_kernel_supports(int m, int n, int m_expanded, bool has_rel);

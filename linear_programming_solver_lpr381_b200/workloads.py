@@ -48,6 +48,21 @@ def large_c3(m=4096, n=8192, seed=7):
     return lp_integer(m, n, seed)
 
 
+def large_dual(m_eq=2048, n=8192, seed=17):
+    """Dual Simplex workload of C3's tableau shape: Min c.x subject to A x = b, x >= 0, every row an equality.
+    A U{1..9}, c U{1..9}; b = A x0 for a random sparse integer x0 >= 0 (about n/64 entries U{1..4}), so the LP is
+    feasible by construction and bounded (c > 0).  2 m_eq + 1 rows after the EQ expansion: 4097 x 12289 by default.
+    Returns (A, b, c, rel, sense) with sense = 1 (Min); smaller m_eq, n for tests."""
+    r = _rng(seed)
+    A = r.integers(1, 10, size=(m_eq, n)).astype(np.float64)
+    c = r.integers(1, 10, size=n).astype(np.float64)
+    x0 = np.zeros(n)
+    k = max(1, n // 64)
+    x0[r.choice(n, size=k, replace=False)] = r.integers(1, 5, size=k)
+    b = A @ x0
+    return A, b, c, np.full(m_eq, 2, dtype=np.int32), 1
+
+
 def ip_c4(m=60, n=120, seed=11):
     """C4: general IP, A U{1..19}, b U{5n..15n-1}, c U{1..29}."""
     r = _rng(seed)
