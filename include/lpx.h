@@ -301,7 +301,13 @@ int lpx_comm_rank(void);
  * xB (m), Binv (m x m, row-major), x (n) = basic decision variables mapped back.
  * history (nullable): history_cap records of lpx_revised_history_stride(m, n) doubles, one per
  * BuildIterationBlock call (:62, :134): [Binv m*m][x_B m][z][r_N n][d m][theta][Bidx m][Nidx n][entering],
- * integers stored as doubles; record 0 is the initial basis (r_N, d, theta unused, entering -1). */
+ * integers stored as doubles; record 0 is the initial basis (r_N, d, theta unused, entering -1).  On
+ * LPX_S_SINGULAR only status, n_iters and the records of the completed iterations are written.
+ * opt.kernel: LPX_KERNEL_CTA_GLOBAL one CTA (the work vectors of 20n + 68m + 16 bytes in shared memory, else
+ * LPX_E_CAPACITY); LPX_KERNEL_STREAM the whole GPU (blocked Gauss-Jordan inversion with opt.stream_block steps per
+ * pass, 0 = 8, and the pass kernel of opt.stream_pass_variant; grid-wide pricing); any other value AUTO: one CTA
+ * while the vectors fit and m <= 64, else the whole GPU.  Both give the same bits.  A history the device cannot
+ * hold fails the whole-GPU call with LPX_E_CAPACITY and the reason in lpx_last_error(); nothing is written. */
 int lpx_revised_solve(int m, int n, int sense, const double* A, const int* rel, const double* b, const double* c,
                       const lpx_options* opt, int* status, int* n_iters, int* pivots, double* theta, int pivots_cap,
                       int* basis, int* nonbasic, double* xB, double* Binv, double* x, double* history,

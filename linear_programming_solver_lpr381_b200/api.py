@@ -75,11 +75,14 @@ def dual_solve(A, b, c, rel=None, sense=0, max_iterations=10000, kernel=F.KERNEL
     return out
 
 
-def revised_solve(A, b, c, rel=None, sense=0, max_iterations=10000, cap=16384, history=0):
-    """lpx_revised_solve: RevisedPrimalSimplex numerics (pivots, theta, final basis state)."""
+def revised_solve(A, b, c, rel=None, sense=0, max_iterations=10000, cap=16384, history=0, kernel=F.KERNEL_AUTO,
+                  kblock=0, pass_variant=0):
+    """lpx_revised_solve: RevisedPrimalSimplex numerics (pivots, theta, final basis state).  kernel: AUTO, STREAM
+    (the whole GPU) or CTA_GLOBAL (one CTA); kblock / pass_variant: Gauss-Jordan steps per pass and the pass kernel
+    of the whole-GPU inversion."""
     A, b, c, rel = _prep(A, b, c, rel)
     m, n = A.shape
-    opt = F.make_options(max_iterations)
+    opt = F.make_options(max_iterations, kernel, kblock=kblock, pass_variant=pass_variant)
     status, n_iters = C.c_int(), C.c_int()
     pivots = np.full((cap, 2), -1, dtype=np.int32)
     theta = np.zeros(cap)

@@ -3,6 +3,8 @@
 // It reuses the reference's own printing code, which must be made `internal static`
 // (BuildIterationBlock, BuildFinalSummary); LPSolver.cs then maps "revised primal simplex" /
 // "revised primal" to this class, and CuttingPlaneRevised.cs:16 constructs it instead of the CPU solver.
+// Default options: a small model runs on one CTA, a large one (m past the crossover, or work vectors past shared
+// memory) on the whole GPU, with the same results (include/lpx.h).
 // Source only (no .NET toolchain in this image); host/revised_host.cpp is the compiled twin.
 using System;
 using System.Collections.Generic;

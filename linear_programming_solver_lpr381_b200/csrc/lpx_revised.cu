@@ -17,8 +17,14 @@
 
 #include "lpx_cta.cuh"
 #include "lpx_runtime.hpp"
+#include "lpx_stream.hpp"
 
 namespace lpx {
+
+// AUTO's crossover: the largest m that stays on the one-CTA kernel.  Measured on one B200 (1000 W,
+// profiles/r08_revised_stream.json, DESIGN.md §4.11): at m = 64 the two paths are within 4 % per iteration (square
+// 0.304 vs 0.316 ms, wide 0.322 vs 0.315 ms); at m = 96 the whole GPU is 2.0-3.2x faster.
+#define LPX_REV_CTA_MAX_M 64
 
 struct RevBatch {
     const double* A;  // m x n
@@ -317,7 +323,14 @@ int lpx_revised_solve(int m, int n, int sense, const double* A, const int* rel, 
     if (pivots_cap < 0 || !pivots) pivots_cap = 0;
     if (!history) history_cap = 0;
     const size_t smem = ((size_t)(n + m) + 7 * (size_t)m + n) * 8 + ((size_t)m + n) * 4 + 16;
-    if (smem > (size_t)max_smem_optin()) {
+    const bool fits = smem <= (size_t)max_smem_optin();
+    // STREAM forces the whole-GPU path, CTA_GLOBAL this kernel; anything else is AUTO: this kernel while its
+    // work vectors fit and m is at most LPX_REV_CTA_MAX_M (measured crossover, above)
+    const bool stream = o.kernel == LPX_KERNEL_STREAM || (o.kernel != LPX_KERNEL_CTA_GLOBAL && (!fits || m > LPX_REV_CTA_MAX_M));
+    if (stream)
+        return revised_stream_solve(m, n, sense, A, b, c, o, status, n_iters, pivots, theta, pivots_cap, basis, nonbasic,
+                                    xB, Binv, x, history, history_cap);
+    if (!fits) {
         set_error("lpx_revised_solve: m + n too large for the shared-memory work vectors");
         return LPX_E_CAPACITY;
     }

@@ -594,28 +594,69 @@ static void launch_lookahead(lpx_session* s, int budget) {
 // pass variants: LDG/STG kernels <KMAX, doubles per thread, rows in flight> or the TMA-staged kernel
 typedef void (*BlockPassFn)(StreamParams, int);
 // the TMA-staged kernel is the default (measured 143 us vs 182 us per 8-pivot pass at 4097 x 12289)
-static bool block_pass_is_tma(const lpx_session* s) {
-    return s->opt.stream_pass_variant == 3 || s->opt.stream_pass_variant == 0;
-}
-static BlockPassFn block_pass_fn(const lpx_session* s) {
-    const int variant = s->opt.stream_pass_variant;  // 0 auto; 1: two doubles/thread; 2: one; 3: TMA-staged
-    if (variant == 3 || variant == 0)
-        return s->P.kblock <= 8 ? stream_update_block_tma_kernel<8> : stream_update_block_tma_kernel<16>;
-    if (s->P.kblock <= 8) return variant == 2 ? stream_update_block_kernel<8, 1, 4> : stream_update_block_kernel<8, 2, 4>;
+static bool block_pass_is_tma(int variant) { return variant == 3 || variant == 0; }
+static BlockPassFn block_pass_fn(int variant, int kblock) {
+    // variant: 0 auto; 1: two doubles/thread; 2: one; 3: TMA-staged
+    if (block_pass_is_tma(variant))
+        return kblock <= 8 ? stream_update_block_tma_kernel<8> : stream_update_block_tma_kernel<16>;
+    if (kblock <= 8) return variant == 2 ? stream_update_block_kernel<8, 1, 4> : stream_update_block_kernel<8, 2, 4>;
     return variant == 2 ? stream_update_block_kernel<16, 1, 4> : stream_update_block_kernel<16, 2, 2>;
 }
-static int block_pass_vec(const lpx_session* s) {
-    const int variant = s->opt.stream_pass_variant;
-    return variant == 2 ? 1 : 2;
+static size_t block_pass_smem(int variant, int kblock, int rpc) {
+    const int kmax = kblock <= 8 ? 8 : 16;
+    if (block_pass_is_tma(variant))
+        return (size_t)LPX_TMA_STAGES * (kblock <= 8 ? sizeof(TmaTile<8>) : sizeof(TmaTile<16>)) + 128;
+    return (size_t)kmax * rpc * 8 + (size_t)((rpc + 15) & ~15);
 }
+static BlockPassFn block_pass_fn(const lpx_session* s) { return block_pass_fn(s->opt.stream_pass_variant, s->P.kblock); }
 static size_t block_pass_smem(const lpx_session* s) {
-    const int kmax = s->P.kblock <= 8 ? 8 : 16;
-    if (block_pass_is_tma(s))
-        return (size_t)LPX_TMA_STAGES * (s->P.kblock <= 8 ? sizeof(TmaTile<8>) : sizeof(TmaTile<16>)) + 128;
-    return (size_t)kmax * s->rpc_block * 8 + (size_t)((s->rpc_block + 15) & ~15);
+    return block_pass_smem(s->opt.stream_pass_variant, s->P.kblock, s->rpc_block);
 }
 static void launch_block_pass(lpx_session* s) {
     block_pass_fn(s)<<<s->grid_block, 256, block_pass_smem(s), s->stream>>>(s->P, s->rpc_block);
+}
+
+// Rows per CTA and grid of the blocked pass over P (P.kblock > 0), sized to one resident wave; sets the pass
+// kernel's shared-memory attribute.
+static void size_block_pass(const StreamParams& P, int variant, int* rpc_out, dim3* grid_out) {
+    if (block_pass_is_tma(variant)) {
+        // TMA-staged pass: strips of 256 columns, row chunks (multiples of 8 rows) sized to one wave
+        const size_t smem = block_pass_smem(variant, P.kblock, 0);
+        cudaFuncSetAttribute(block_pass_fn(variant, P.kblock), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        int got = 0;
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&got, block_pass_fn(variant, P.kblock), 256, smem);
+        if (got < 1) got = 1;
+        const int bstrips = (P.ld + LPX_TMA_COLS - 1) / LPX_TMA_COLS;
+        int ch = std::max(1, (sm_count() * got) / bstrips);
+        int rpc = (P.rows + ch - 1) / ch;
+        rpc = (rpc + 7) & ~7;
+        *rpc_out = rpc;
+        *grid_out = dim3(bstrips, (P.rows + rpc - 1) / rpc, 1);
+        cudaGetLastError();
+        return;
+    }
+    // blocked pass: column strips x row chunks sized to one resident wave; the factor slices of a
+    // chunk must fit in shared memory next to the other resident CTAs
+    const int vec = variant == 2 ? 1 : 2;
+    const int bstrips = (P.ld / vec + 255) / 256;
+    int best_rpc = 0;
+    for (int want_occ = 4; want_occ >= 1 && !best_rpc; want_occ--) {
+        int ch = std::max(1, (sm_count() * want_occ) / bstrips);
+        ch = std::min(ch, P.rows);
+        const int rpc = (P.rows + ch - 1) / ch;
+        const size_t smem = block_pass_smem(variant, P.kblock, rpc);
+        if (smem > (size_t)max_smem_optin()) continue;
+        cudaFuncSetAttribute(block_pass_fn(variant, P.kblock), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        int got = 0;
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&got, block_pass_fn(variant, P.kblock), 256, smem);
+        if (got >= want_occ || want_occ == 1) best_rpc = rpc;
+    }
+    if (!best_rpc) best_rpc = 64;
+    *rpc_out = best_rpc;
+    cudaFuncSetAttribute(block_pass_fn(variant, P.kblock), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         (int)block_pass_smem(variant, P.kblock, best_rpc));
+    cudaGetLastError();
+    *grid_out = dim3(bstrips, (P.rows + best_rpc - 1) / best_rpc, 1);
 }
 
 static bool create_priority_stream(cudaStream_t* st) {
@@ -867,45 +908,7 @@ static lpx_session* session_new(int m_in, int n, int sense, int mm, const lpx_op
         s->grid_pipe = dim3(bstrips, (P.rows + rpc - 1) / rpc, 1);
         cudaGetLastError();
     }
-    if (P.kblock > 0 && block_pass_is_tma(s)) {
-        // TMA-staged pass: strips of 256 columns, row chunks (multiples of 8 rows) sized to one wave
-        const size_t smem = block_pass_smem(s);
-        cudaFuncSetAttribute(block_pass_fn(s), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        int got = 0;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&got, block_pass_fn(s), 256, smem);
-        if (got < 1) got = 1;
-        const int bstrips = (P.ld + LPX_TMA_COLS - 1) / LPX_TMA_COLS;
-        int ch = std::max(1, (sm_count() * got) / bstrips);
-        int rpc = (P.rows + ch - 1) / ch;
-        rpc = (rpc + 7) & ~7;
-        s->rpc_block = rpc;
-        s->grid_block = dim3(bstrips, (P.rows + rpc - 1) / rpc, 1);
-        cudaGetLastError();
-    } else if (P.kblock > 0) {
-        // blocked pass: column strips x row chunks sized to one resident wave; the factor slices of a
-        // chunk must fit in shared memory next to the other resident CTAs
-        const int vec = block_pass_vec(s);
-        const int kmax = P.kblock <= 8 ? 8 : 16;
-        const int bstrips = (P.ld / vec + 255) / 256;
-        int best_rpc = 0;
-        for (int want_occ = 4; want_occ >= 1 && !best_rpc; want_occ--) {
-            int ch = std::max(1, (sm_count() * want_occ) / bstrips);
-            ch = std::min(ch, P.rows);
-            const int rpc = (P.rows + ch - 1) / ch;
-            const size_t smem = (size_t)kmax * rpc * 8 + (size_t)((rpc + 15) & ~15);
-            if (smem > (size_t)max_smem_optin()) continue;
-            cudaFuncSetAttribute(block_pass_fn(s), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            int got = 0;
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&got, block_pass_fn(s), 256, smem);
-            if (got >= want_occ || want_occ == 1) best_rpc = rpc;
-        }
-        if (!best_rpc) best_rpc = 64;
-        s->rpc_block = best_rpc;
-        const size_t smem = (size_t)kmax * best_rpc * 8 + (size_t)((best_rpc + 15) & ~15);
-        cudaFuncSetAttribute(block_pass_fn(s), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        cudaGetLastError();
-        s->grid_block = dim3(bstrips, (P.rows + best_rpc - 1) / best_rpc, 1);
-    }
+    if (P.kblock > 0) size_block_pass(P, s->opt.stream_pass_variant, &s->rpc_block, &s->grid_block);
     return s;
 }
 
@@ -1184,6 +1187,8 @@ int stream_dual_solve_host(int m, int n, int sense, const double* A, const int* 
 }
 
 }  // namespace lpx
+
+#include "lpx_revised_stream.cuh"
 
 extern "C" {
 

@@ -16,6 +16,13 @@ int stream_dual_solve_host(int m, int n, int sense, const double* A, const int* 
                            int pivots_cap, int* basis, double* x, double* z, double* tableau, double* history,
                            int history_cap);
 
+// Revised Primal Simplex on the whole GPU (lpx_revised_stream.cuh), host buffers in / host buffers out; the caller
+// holds the runtime lock and has checked the arguments and the reference's precondition
+int revised_stream_solve(int m, int n, int sense, const double* A, const double* b, const double* c,
+                         const lpx_options& o, int* status, int* n_iters, int* pivots, double* theta, int pivots_cap,
+                         int* basis, int* nonbasic, double* xB, double* Binv, double* x, double* history,
+                         int history_cap);
+
 // register-resident batched kernel (lpx_reg.cu)
 bool reg_kernel_supports(int m, int n, int m_expanded, bool has_rel);
 int reg_launch_batched(int count, int m, int n, int sense, const double* A, const double* b, const double* c,
