@@ -423,6 +423,53 @@ int lpx_reoptimize(int kind, int m, int n, int sense, const double* A, const int
  * c + dc) for RHS / COST queries and returns LPX_E_BAD_ARGS for ROW / COL queries.  Free with lpx_session_close. */
 lpx_session* lpx_session_reoptimize(const lpx_session* base, int kind, const double* payload, const lpx_options* opt);
 
+/* ---- Gomory cutting plane: CuttingPlane.Solve, R/Models/CuttingPlane.cs:13-164 ------------------------------ */
+/* `count` IPs, one CTA each, all rounds on the device.  A round solves the model plus the cuts so far with Primal
+ * Simplex (the rules and bits of lpx_primal_solve, opt.max_iterations), reads x (an UNBOUNDED round's too), finds the
+ * first j with 1e-9 < x_j - floor(x_j) < 1 - 1e-9 and, if there is one, appends the cut read from tableau row
+ * (x_j's basis position + 1) — the reference's quirk: the row below x_j's, the z-row when x_j is basic in the last
+ * constraint row: a_k = f_k when f_k = T[row][k] - floor(T[row][k]) > 1e-9, else +0.0, over the n decision columns;
+ * b = rhs - floor(rhs); relation '<='.  The loop ends at an integral x (INTEGER), when Primal Simplex throws
+ * (GE row or negative RHS in round 1, the iteration limit in any round: LP_ERROR), or after 50 rounds (INCOMPLETE).
+ * A round's tableau is built cold as PrimalSimplex.Solve builds it for the grown model: the base rows (EQ expanded),
+ * then the cuts in order, each with +1 in its own slack column, then the z-row.
+ *   Shape      one per call: m, n, sense and rel are shared; A[count][m][n], b[count][m], c[count][n] strided per IP.
+ *   end        LPX_CUT_*; n_rounds = rounds run (PrimalSimplex calls), n_cuts = n_rounds for INCOMPLETE, else
+ *              n_rounds - 1.
+ *   Per round  [count][50]: lp_status = LPX_OPTIMAL, LPX_UNBOUNDED or the LPX_S_* of the round that threw; lp_pivots =
+ *              pivots of that round (0 for GE / negative RHS, max_iterations for LPX_S_ITER_LIMIT); rounds not run:
+ *              LPX_RUNNING and 0.
+ *   Per cut    [count][50]: frac_var, cut_row (the tableau row read), cut_a [count][50][n], cut_b; cuts not made: -1,
+ *              -1, +0.0, +0.0.
+ *   Final LP   only for INTEGER: basis [count][m'+49], x [count][n], z [count], tableau [count][max_rows*max_cols]
+ *              hold the last round's LP, the tableau compact (rows = m' + n_cuts + 1, cols = n + m' + n_cuts + 1) at
+ *              the start of the slot; every other entry, and all of them for any other end, is zero.
+ * Every output except `end` may be NULL.  opt.kernel: AUTO (the tableau in shared memory when the 50-round shape fits,
+ * else in global memory), LPX_KERNEL_CTA_SMEM (LPX_E_CAPACITY when it does not fit) or LPX_KERNEL_CTA_GLOBAL; any other
+ * value is LPX_E_BAD_ARGS, as are count < 1, m < 1, n < 1, a rel value outside 0..2 or a sense outside 0..1 (checked
+ * before any device work).  opt.threads is honoured.  Bit-exact with oracle/orc_cut.cpp (numbers) and oracle/orc_cutting.cpp (text). */
+#define LPX_CUT_INTEGER    0   /* all x_j integral: the final LP's outputs are written */
+#define LPX_CUT_INCOMPLETE 1   /* 50 rounds, 50 cuts */
+#define LPX_CUT_LP_ERROR   2   /* a round's PrimalSimplex threw: its lp_status says which */
+#define LPX_CUT_NONBASIC   3   /* kept for the oracle's enum; unreachable for a basic fractional value */
+#define LPX_CUT_MAX_ROUNDS 50
+/* max_rows = m' + 50, max_cols = n + m' + 50: the output strides (rel: host pointer, nullable = all LE) */
+int lpx_cutting_plane_dims(int m, int n, const int* rel, int* max_rows, int* max_cols);
+/* Host buffers. */
+int lpx_cutting_plane_batched(int count, int m, int n, int sense, const double* A, const int* rel, const double* b,
+                              const double* c, const lpx_options* opt, int* end, int* n_rounds, int* n_cuts,
+                              int* lp_status, int* lp_pivots, int* frac_var, int* cut_row, double* cut_a, double* cut_b,
+                              int* basis, double* x, double* z, double* tableau, long long* total_pivots);
+/* Same, all pointers are DEVICE pointers (rel too; it is read back once for the tableau shape and checked then),
+ * asynchronous on `stream`.  total_pivots: as in lpx_primal_solve_batched_dev (zero it first).  cut_a / cut_b, when
+ * given, are the cut store the rounds read back; without them, and for the global-memory build without a tableau,
+ * the library uses scratch of its own. */
+int lpx_cutting_plane_batched_dev(int count, int m, int n, int sense, const double* A, const int* rel, const double* b,
+                                  const double* c, const lpx_options* opt, int* end, int* n_rounds, int* n_cuts,
+                                  int* lp_status, int* lp_pivots, int* frac_var, int* cut_row, double* cut_a,
+                                  double* cut_b, int* basis, double* x, double* z, double* tableau,
+                                  unsigned long long* total_pivots, void* stream);
+
 /* ---- measurement helpers (bench.py) --------------------------------------------------------- */
 /* Unfused FP64 rate (separate DMUL and DADD, the only arithmetic the bit-exactness contract
  * allows) in TFLOP/s: the roofline denominator of the on-chip batched kernels. */

@@ -19,6 +19,7 @@ E_BAD_ARGS, E_CUDA, E_CAPACITY, E_NCCL = -4, -5, -8, -9
 KERNEL_AUTO, KERNEL_CTA_SMEM, KERNEL_CTA_GLOBAL, KERNEL_STREAM, KERNEL_CTA_REG, KERNEL_CTA_CLUSTER = 0, 1, 2, 3, 4, 5
 BNB_WANT_HISTORY = 1
 REOPT_RHS, REOPT_COST, REOPT_ROW, REOPT_COL = 1, 2, 3, 4
+CUT_INTEGER, CUT_INCOMPLETE, CUT_LP_ERROR, CUT_NONBASIC, CUT_MAX_ROUNDS = 0, 1, 2, 3, 50
 
 # every symbol include/lpx.h declares; tests check that the library exports all of them
 EXPORTS = [
@@ -34,7 +35,8 @@ EXPORTS = [
     "lpx_bnb_last_stats", "lpx_bnb_pooled", "lpx_sensitivity_stride", "lpx_sensitivity_batched_dev",
     "lpx_primal_solve_sensitivity_batched", "lpx_session_sensitivity", "lpx_reopt_payload_stride", "lpx_reopt_dims",
     "lpx_reoptimize_batched_dev", "lpx_reoptimize", "lpx_session_reoptimize", "lpx_dual_session_open",
-    "lpx_dual_session_open_dev", "lpx_session_silent_pivots",
+    "lpx_dual_session_open_dev", "lpx_session_silent_pivots", "lpx_cutting_plane_dims", "lpx_cutting_plane_batched",
+    "lpx_cutting_plane_batched_dev",
 ]
 
 
@@ -150,6 +152,9 @@ def lib():
                                  + [C.c_void_p] * 4)
     L.lpx_session_reoptimize.restype = C.c_void_p
     L.lpx_session_reoptimize.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
+    L.lpx_cutting_plane_dims.argtypes = [C.c_int, C.c_int, C.c_void_p, _ip, _ip]
+    L.lpx_cutting_plane_batched.argtypes = [C.c_int] * 4 + [C.c_void_p] * 18 + [_llp]
+    L.lpx_cutting_plane_batched_dev.argtypes = [C.c_int] * 4 + [C.c_void_p] * 20
     L.lpx_bnb_simplex_batched.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]

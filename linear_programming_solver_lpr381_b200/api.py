@@ -247,6 +247,73 @@ def reoptimize_batched_dev(kind, count, m, n, sense, drel, dbase_status, dbase_b
         F.ptr(stream or 0)))
 
 
+def cutting_plane_dims(m, n, rel=None):
+    """(max_rows, max_cols) = (m' + 50, n + m' + 50): the per-IP stride of the cutting-plane tableau output."""
+    rows, cols = C.c_int(), C.c_int()
+    rel = None if rel is None else np.ascontiguousarray(rel, dtype=np.int32)
+    F.check(F.lib().lpx_cutting_plane_dims(m, n, F.ptr(rel), C.byref(rows), C.byref(cols)))
+    return rows.value, cols.value
+
+
+def cutting_plane_batched(A, b, c, rel=None, sense=0, max_iterations=10000, kernel=F.KERNEL_AUTO, threads=0,
+                          want_tableau=True):
+    """lpx_cutting_plane_batched: CuttingPlane.Solve for `count` IPs of one shape (A (count, m, n), b (count, m),
+    c (count, n)), every round on the GPU.  Returns end, n_rounds, n_cuts (count), lp_status / lp_pivots (count, 50),
+    frac_var / cut_row (count, 50), cut_a (count, 50, n), cut_b (count, 50), and the final LP of the integral ends:
+    basis (count, m' + 49), x, z and tableau (count, m' + 50, n + m' + 50; the final tableau compact at the start of
+    each slot: tableau_of() reshapes it), plus total_pivots."""
+    A, b, c, rel = _prep(A, b, c, rel)
+    count, m, n = A.shape
+    R = F.CUT_MAX_ROUNDS
+    max_rows, max_cols = cutting_plane_dims(m, n, rel)
+    opt = F.make_options(max_iterations, kernel, threads)
+    out = dict(end=np.zeros(count, np.int32), n_rounds=np.zeros(count, np.int32), n_cuts=np.zeros(count, np.int32),
+               lp_status=np.zeros((count, R), np.int32), lp_pivots=np.zeros((count, R), np.int32),
+               frac_var=np.zeros((count, R), np.int32), cut_row=np.zeros((count, R), np.int32),
+               cut_a=np.zeros((count, R, n)), cut_b=np.zeros((count, R)),
+               basis=np.zeros((count, max_rows - 1), np.int32), x=np.zeros((count, n)), z=np.zeros(count),
+               tableau=np.zeros((count, max_rows, max_cols)) if want_tableau else None)
+    total = C.c_longlong()
+    F.check(F.lib().lpx_cutting_plane_batched(
+        count, m, n, sense, F.ptr(A), F.ptr(rel), F.ptr(b), F.ptr(c), C.byref(opt),
+        *[F.ptr(out[k]) for k in ("end", "n_rounds", "n_cuts", "lp_status", "lp_pivots", "frac_var", "cut_row",
+                                  "cut_a", "cut_b", "basis", "x", "z", "tableau")], C.byref(total)))
+    out["total_pivots"] = total.value
+    return out
+
+
+def cutting_plane(A, b, c, rel=None, sense=0, **kw):
+    """One IP through cutting_plane_batched: the same fields without the leading count axis; `tableau` is the final
+    LP's tableau (m' + n_cuts + 1, n + m' + n_cuts + 1) for an integral end, else None."""
+    A = np.asarray(A, dtype=np.float64)
+    r = cutting_plane_batched(A[None], np.asarray(b, np.float64)[None], np.asarray(c, np.float64)[None], rel, sense,
+                              **kw)
+    out = {k: (v[0] if isinstance(v, np.ndarray) else v) for k, v in r.items()}
+    out["tableau"] = tableau_of(out, A.shape[1]) if out["end"] == F.CUT_INTEGER and r["tableau"] is not None else None
+    return out
+
+
+def tableau_of(one, n):
+    """The compact final tableau at the start of one IP's tableau slot (an integral end only)."""
+    slot = np.asarray(one["tableau"]).reshape(-1)
+    mm = one["basis"].shape[-1] - 49
+    rows, cols = mm + one["n_cuts"] + 1, n + mm + one["n_cuts"] + 1
+    return slot[: rows * cols].reshape(rows, cols)
+
+
+def cutting_plane_batched_dev(count, m, n, sense, dA, drel, db, dc, dend, dn_rounds, dn_cuts, dlp_status, dlp_pivots,
+                              dfrac_var, dcut_row, dcut_a, dcut_b, dbasis, dx, dz, dtableau, dtotal, stream,
+                              max_iterations=10000, kernel=F.KERNEL_AUTO, threads=0):
+    """lpx_cutting_plane_batched_dev: raw device pointers (ints, 0 / None for the nullable ones), asynchronous on
+    `stream` (a cudaStream_t)."""
+    opt = F.make_options(max_iterations, kernel, threads)
+    F.check(F.lib().lpx_cutting_plane_batched_dev(
+        count, m, n, sense, F.ptr(dA), F.ptr(drel), F.ptr(db), F.ptr(dc), C.byref(opt), F.ptr(dend),
+        F.ptr(dn_rounds), F.ptr(dn_cuts), F.ptr(dlp_status), F.ptr(dlp_pivots), F.ptr(dfrac_var), F.ptr(dcut_row),
+        F.ptr(dcut_a), F.ptr(dcut_b), F.ptr(dbasis), F.ptr(dx), F.ptr(dz), F.ptr(dtableau), F.ptr(dtotal),
+        F.ptr(stream or 0)))
+
+
 class Session:
     """Large single LP whose tableau lives in HBM (lpx_session_*).  dual=True: DualSimplex.Solve on the model
     (lpx_dual_session_open); the silent ForceDualFeasibility pivots run inside the constructor and `.silent` counts

@@ -126,6 +126,22 @@ namespace Linear_Programming_Solver.Models
             IntPtr c, ref LpxOptions opt);
         [DllImport(Lib)] public static extern int lpx_session_silent_pivots(IntPtr session, out int silent);
 
+        // Gomory cutting plane (CuttingPlane.Solve, all rounds on the GPU, one CTA per IP; include/lpx.h).  No
+        // ILPAlgorithm shim: the reference's CuttingPlane text prints every round's iteration tableaux, which stay on
+        // the host path.  end: 0 integer, 1 incomplete (50 rounds), 2 LP error; any other output may be null.
+        public const int LPX_CUT_MAX_ROUNDS = 50;
+        [DllImport(Lib)] public static extern int lpx_cutting_plane_dims(int m, int n, int[] rel, out int max_rows, out int max_cols);
+        [DllImport(Lib)]
+        public static extern int lpx_cutting_plane_batched(int count, int m, int n, int sense, double[] A, int[] rel,
+            double[] b, double[] c, ref LpxOptions opt, int[] end, int[] n_rounds, int[] n_cuts, int[] lp_status,
+            int[] lp_pivots, int[] frac_var, int[] cut_row, double[] cut_a, double[] cut_b, int[] basis, double[] x,
+            double[] z, double[] tableau, out long total_pivots);
+        [DllImport(Lib)]
+        public static extern int lpx_cutting_plane_batched_dev(int count, int m, int n, int sense, IntPtr A, IntPtr rel,
+            IntPtr b, IntPtr c, ref LpxOptions opt, IntPtr end, IntPtr n_rounds, IntPtr n_cuts, IntPtr lp_status,
+            IntPtr lp_pivots, IntPtr frac_var, IntPtr cut_row, IntPtr cut_a, IntPtr cut_b, IntPtr basis, IntPtr x,
+            IntPtr z, IntPtr tableau, IntPtr total_pivots, IntPtr stream);
+
         [DllImport(Lib)]
         public static extern int lpx_primal_solve_batched(int count, int m, int n, int sense, double[] A, int[] rel,
             double[] b, double[] c, ref LpxOptions opt, int[] status, int[] n_pivots, int[] basis, double[] x,

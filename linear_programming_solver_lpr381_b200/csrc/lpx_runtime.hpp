@@ -19,6 +19,7 @@ enum Slot {
     WS_PL_IN, WS_PL_OUT, WS_PL_ALL,  // pooled-tree B&B: node descriptors, own results, everybody's results
     WS_SENS,  // sensitivity reports of lpx_primal_solve_sensitivity_batched
     WS_RO_REC, WS_RO_PAY, WS_RO_SRC, WS_RO_BASE_T, WS_RO_BASE_I,  // re-optimization: records, payloads, base
+    WS_CUT_INT, WS_CUT_DBL, WS_CUT_STORE,  // cutting plane: integer / double outputs, the cut store without one
     WS_BB_SET0,  // pipelined B&B: descriptors, results, scratch of each of LPX_BB_SETS evaluation sets
     WS_COUNT = WS_BB_SET0 + 3 * 4
 };
