@@ -470,6 +470,86 @@ int lpx_cutting_plane_batched_dev(int count, int m, int n, int sense, const doub
                                   double* cut_b, int* basis, double* x, double* z, double* tableau,
                                   unsigned long long* total_pivots, void* stream);
 
+/* ---- Parametric analysis of an optimal Primal Simplex result — NOT the reference's ------------------------ */
+/* The optimal value z*(theta) along a line, b + theta d (RHS) or c + theta d (COST) for theta in [0, theta_max]:
+ * piecewise linear, one segment per basis, each with its intercept, slope and x*(theta), and the reason the analysis
+ * stopped.  Checked against oracle/orc_param.cpp bit for bit and against an independent LP solver.  Notation as in
+ * the sensitivity and re-optimization sections: m' rows after EQ expansion, W = n + m' + 1, the slack of constraint i
+ * is s1 = n + i1 (an EQ row also has s2 = n + i2), T[m'] is the z-row in max form, EPS = 1e-9, FP64 with separate
+ * multiply / add / subtract and true division.  The base is a final Primal Simplex tableau with status LPX_OPTIMAL and
+ * its basis.  One kind per call; each query has lpx_param_payload_stride(kind, m, n) doubles: d, then theta_max
+ * (>= 0 or +inf; NaN or a negative value is LPX_E_BAD_ARGS).
+ *   LPX_PARAM_RHS   payload d[m], theta_max.  Working tableau: the base's plus a direction column g at index W.  On
+ *                   every row r (z-row included) g_r starts at +0.0; for i ascending with d_i != 0:
+ *                   g_r += d_i * T[r][s1], an EQ row also g_r -= d_i * T[r][s2] (the RHS query's terms).
+ *                   x_B(theta) = beta + theta g.  theta_cand = min{-(beta_r / g_r) : constraint row r, g_r < -EPS},
+ *                   +inf if none.  That row leaves; the entering column is the Dual Simplex rule's (min z_j / -a over
+ *                   a < -EPS, margin 1e-12, columns < W - 1); none: INFEASIBLE.  The pivot updates all W + 1 columns.
+ *                   Segment: z0 = T[m'][W-1], dz = T[m'][W]; basic decision x_j in row r: x0_j = beta_r, dx_j = g_r;
+ *                   other j: +0.0, +0.0.
+ *   LPX_PARAM_COST  payload d[n] in the model's sense, theta_max.  Working tableau: the base's plus a direction row h at
+ *                   index m' + 1: h starts at +0.0; for j ascending with d_j != 0, delta = d_j (Max) or -d_j (Min):
+ *                   if j is basic in row r, h[k] += delta * T[r][k] for all k < W; then h[j] -= delta (the COST
+ *                   query's terms applied to a zero row).  Reduced costs at theta: T[m'][k] + theta h[k].
+ *                   theta_cand = min{-(T[m'][k] / h[k]) : non-basic k < W - 1, h[k] < -EPS}.  That column enters; the
+ *                   leaving row is the Primal Simplex rule's (ratio margin 1e-9); none: UNBOUNDED.  The pivot updates
+ *                   every row, h included.  Segment: z0 = T[m'][W-1], dz = h[W-1]; x0 from the RHS column, dx = +0.0.
+ * In both minima -0.0 equals +0.0, the lowest index wins ties (the sensitivity report's rule) and a NaN ratio is never
+ * chosen.  The loop starts at theta_lo = 0, k = 0:
+ *   1. theta_end = theta_cand < theta_lo ? theta_lo : theta_cand (a slightly negative beta or reduced cost gives a
+ *      zero-length segment, not a step back);
+ *   2. theta_end >= theta_max: segment [theta_lo, theta_max], end REACHED (theta_max = +inf with no limit: the last
+ *      segment is [theta_lo, +inf]);
+ *   3. else k + 1 == seg_cap: segment [theta_lo, theta_end], end SEG_LIMIT;
+ *   4. else the pivot search; none: segment [theta_lo, theta_end], end INFEASIBLE (RHS) or UNBOUNDED (COST);
+ *   5. else segment [theta_lo, theta_end] with its (leaving row, entering column), the pivot, theta_lo = theta_end,
+ *      k + 1, repeat.
+ * Segment values are read before the pivot.  z and x are in max form, as every other entry point returns them.  Only
+ * theta >= 0 is covered: the other side is the query with -d.  A query whose base is not LPX_OPTIMAL gets end
+ * NO_BASE, 0 segments and zeroed outputs.  Per query:
+ *   end; n_segments; n_pivots = n_segments - 1 (0 for NO_BASE);
+ *   segments    [seg_cap] records of lpx_param_segment_stride(n) = 4 + 2n doubles:
+ *               theta_lo | theta_hi | z0 | dz | x0[n] | dx[n]; records past the last are zero;
+ *   seg_pivots  [seg_cap][2] ints (leaving row, entering column), (-1, -1) for the last segment and past it;
+ *   basis       [m'], the final basis;
+ *   tableau     the final working tableau, compact, rows x cols of lpx_parametric_dims: (m' + 1) x (W + 1) for RHS,
+ *               (m' + 2) x W for COST.
+ * Every output except end may be NULL.  opt.kernel: AUTO (the working tableau in shared memory when it fits, else in
+ * global memory), LPX_KERNEL_CTA_SMEM (LPX_E_CAPACITY when it does not fit) or LPX_KERNEL_CTA_GLOBAL; any other value
+ * is LPX_E_BAD_ARGS, as are an unknown kind, count < 0, m < 1, n < 1, seg_cap < 1, a sense outside 0..1, a rel value
+ * outside 0..2 and a bad theta_max (checked before any device work).  opt.threads is honoured.
+ * Scope: results of the Primal Simplex entry points (Dual Simplex results are excluded, as for the sensitivity
+ * report); one direction in b or in c per query. */
+#define LPX_PARAM_RHS  1
+#define LPX_PARAM_COST 2
+#define LPX_PARAM_REACHED    0  /* theta_max reached */
+#define LPX_PARAM_UNBOUNDED  1  /* COST: unbounded beyond the last breakpoint */
+#define LPX_PARAM_INFEASIBLE 2  /* RHS: infeasible beyond the last breakpoint */
+#define LPX_PARAM_SEG_LIMIT  3  /* seg_cap segments recorded */
+#define LPX_PARAM_NO_BASE    4  /* the base is not LPX_OPTIMAL */
+/* doubles per query payload: m + 1 (RHS), n + 1 (COST); 0 for an unknown kind */
+size_t lpx_param_payload_stride(int kind, int m, int n);
+/* doubles per segment record: 4 + 2n */
+size_t lpx_param_segment_stride(int n);
+/* rows / cols of a query's working tableau (rel: host pointer, nullable = all LE) */
+int lpx_parametric_dims(int kind, int m, int n, const int* rel, int* rows, int* cols);
+/* Device pointers throughout (rel included; the outputs of lpx_primal_solve_batched_dev serve as the bases),
+ * asynchronous on `stream`; rel and the theta_max entries are read back once and checked.  base_status /
+ * base_basis / base_tableau: the bases, indexed by src[q] (nullable: query q uses base q).  payload: count x stride.
+ * tableau must not overlap the bases.  total_pivots: as in lpx_primal_solve_batched_dev (zero it first). */
+int lpx_parametric_batched_dev(int kind, int count, int m, int n, int sense, const int* rel, const int* base_status,
+                               const int* base_basis, const double* base_tableau, const int* src,
+                               const double* payload, int seg_cap, const lpx_options* opt, int* end, int* n_segments,
+                               int* n_pivots, double* segments, int* seg_pivots, int* basis, double* tableau,
+                               unsigned long long* total_pivots, void* stream);
+/* Host buffers: one GPU Primal Simplex solve of the base (A, rel, b, c; opt.max_iterations and opt.threads apply to it,
+ * the kernel is chosen automatically) and `count` queries of one kind against its final tableau.  *base_status
+ * (nullable) is the base's status. */
+int lpx_parametric(int kind, int m, int n, int sense, const double* A, const int* rel, const double* b,
+                   const double* c, const lpx_options* opt, int count, const double* payload, int seg_cap,
+                   int* base_status, int* end, int* n_segments, int* n_pivots, double* segments, int* seg_pivots,
+                   int* basis, double* tableau);
+
 /* ---- measurement helpers (bench.py) --------------------------------------------------------- */
 /* Unfused FP64 rate (separate DMUL and DADD, the only arithmetic the bit-exactness contract
  * allows) in TFLOP/s: the roofline denominator of the on-chip batched kernels. */

@@ -20,6 +20,8 @@ KERNEL_AUTO, KERNEL_CTA_SMEM, KERNEL_CTA_GLOBAL, KERNEL_STREAM, KERNEL_CTA_REG, 
 BNB_WANT_HISTORY = 1
 REOPT_RHS, REOPT_COST, REOPT_ROW, REOPT_COL = 1, 2, 3, 4
 CUT_INTEGER, CUT_INCOMPLETE, CUT_LP_ERROR, CUT_NONBASIC, CUT_MAX_ROUNDS = 0, 1, 2, 3, 50
+PARAM_RHS, PARAM_COST = 1, 2
+PARAM_REACHED, PARAM_UNBOUNDED, PARAM_INFEASIBLE, PARAM_SEG_LIMIT, PARAM_NO_BASE = 0, 1, 2, 3, 4
 
 # every symbol include/lpx.h declares; tests check that the library exports all of them
 EXPORTS = [
@@ -36,7 +38,8 @@ EXPORTS = [
     "lpx_primal_solve_sensitivity_batched", "lpx_session_sensitivity", "lpx_reopt_payload_stride", "lpx_reopt_dims",
     "lpx_reoptimize_batched_dev", "lpx_reoptimize", "lpx_session_reoptimize", "lpx_dual_session_open",
     "lpx_dual_session_open_dev", "lpx_session_silent_pivots", "lpx_cutting_plane_dims", "lpx_cutting_plane_batched",
-    "lpx_cutting_plane_batched_dev",
+    "lpx_cutting_plane_batched_dev", "lpx_param_payload_stride", "lpx_param_segment_stride", "lpx_parametric_dims",
+    "lpx_parametric_batched_dev", "lpx_parametric",
 ]
 
 
@@ -155,6 +158,13 @@ def lib():
     L.lpx_cutting_plane_dims.argtypes = [C.c_int, C.c_int, C.c_void_p, _ip, _ip]
     L.lpx_cutting_plane_batched.argtypes = [C.c_int] * 4 + [C.c_void_p] * 18 + [_llp]
     L.lpx_cutting_plane_batched_dev.argtypes = [C.c_int] * 4 + [C.c_void_p] * 20
+    L.lpx_param_payload_stride.restype = C.c_size_t
+    L.lpx_param_payload_stride.argtypes = [C.c_int, C.c_int, C.c_int]
+    L.lpx_param_segment_stride.restype = C.c_size_t
+    L.lpx_param_segment_stride.argtypes = [C.c_int]
+    L.lpx_parametric_dims.argtypes = [C.c_int, C.c_int, C.c_int, C.c_void_p, _ip, _ip]
+    L.lpx_parametric_batched_dev.argtypes = [C.c_int] * 5 + [C.c_void_p] * 6 + [C.c_int] + [C.c_void_p] * 10
+    L.lpx_parametric.argtypes = [C.c_int] * 4 + [C.c_void_p] * 5 + [C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 8
     L.lpx_bnb_simplex_batched.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]

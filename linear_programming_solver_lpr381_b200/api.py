@@ -247,6 +247,75 @@ def reoptimize_batched_dev(kind, count, m, n, sense, drel, dbase_status, dbase_b
         F.ptr(stream or 0)))
 
 
+PARAM_KINDS = {"rhs": F.PARAM_RHS, "cost": F.PARAM_COST}
+
+
+def param_payload_stride(kind, m, n):
+    return int(F.lib().lpx_param_payload_stride(PARAM_KINDS.get(kind, kind), m, n))
+
+
+def parametric_dims(kind, m, n, rel=None):
+    """(rows, cols) of a parametric query's working tableau: (m' + 1, W + 1) for RHS, (m' + 2, W) for COST."""
+    rows, cols = C.c_int(), C.c_int()
+    rel = None if rel is None else np.ascontiguousarray(rel, dtype=np.int32)
+    F.check(F.lib().lpx_parametric_dims(PARAM_KINDS.get(kind, kind), m, n, F.ptr(rel), C.byref(rows),
+                                        C.byref(cols)))
+    return rows.value, cols.value
+
+
+def split_segments(segments, n):
+    """Named views of parametric segment records (include/lpx.h): theta_lo, theta_hi, z0, dz (one each), x0, dx
+    (n each); `segments` has records of 4 + 2n doubles on its last axis."""
+    return dict(theta_lo=segments[..., 0], theta_hi=segments[..., 1], z0=segments[..., 2], dz=segments[..., 3],
+                x0=segments[..., 4:4 + n], dx=segments[..., 4 + n:4 + 2 * n])
+
+
+def parametric(kind, A, b, c, directions, theta_max=np.inf, rel=None, sense=0, seg_cap=64, kernel=F.KERNEL_AUTO,
+               threads=0, max_iterations=10000, want_tableau=True):
+    """lpx_parametric: one GPU Primal Simplex solve of the base, then one parametric analysis per direction ("rhs":
+    b + theta d, "cost": c + theta d, or LPX_PARAM_*) on theta in [0, theta_max] (a scalar or one per direction).
+    Returns base_status and per query end, n_segments, n_pivots, segments (count, seg_cap, 4 + 2n) with its
+    split_segments views, seg_pivots (count, seg_cap, 2), basis and tableau."""
+    kind = PARAM_KINDS.get(kind, kind)
+    A, b, c, rel = _prep(A, b, c, rel)
+    m, n = A.shape
+    dirs = np.atleast_2d(np.asarray(directions, dtype=np.float64))
+    count = dirs.shape[0]
+    tmax = np.broadcast_to(np.asarray(theta_max, dtype=np.float64), (count,))
+    pay = np.ascontiguousarray(np.hstack([dirs, tmax[:, None]]))
+    if pay.shape[1] != param_payload_stride(kind, m, n):
+        raise F.LpxError(F.E_BAD_ARGS, "a direction has %d entries, kind %d needs %d" % (
+            dirs.shape[1], kind, param_payload_stride(kind, m, n) - 1))
+    rows, cols = parametric_dims(kind, m, n, rel)
+    mm = m if rel is None else m + int(np.sum(rel == 2))
+    opt = F.make_options(max_iterations, kernel, threads)
+    base_status = C.c_int()
+    out = dict(end=np.zeros(count, np.int32), n_segments=np.zeros(count, np.int32),
+               n_pivots=np.zeros(count, np.int32), segments=np.zeros((count, seg_cap, 4 + 2 * n)),
+               seg_pivots=np.zeros((count, seg_cap, 2), np.int32), basis=np.zeros((count, mm), np.int32),
+               tableau=np.zeros((count, rows, cols)) if want_tableau else None)
+    F.check(F.lib().lpx_parametric(kind, m, n, sense, F.ptr(A), F.ptr(rel), F.ptr(b), F.ptr(c), C.byref(opt), count,
+                                   F.ptr(pay), seg_cap, C.byref(base_status),
+                                   *[F.ptr(out[k]) for k in ("end", "n_segments", "n_pivots", "segments", "seg_pivots",
+                                                             "basis", "tableau")]))
+    out["base_status"] = base_status.value
+    out.update(split_segments(out["segments"], n))
+    return out
+
+
+def parametric_batched_dev(kind, count, m, n, sense, drel, dbase_status, dbase_basis, dbase_tableau, dsrc, dpayload,
+                           seg_cap, dend, dn_segments, dn_pivots, dsegments, dseg_pivots, dbasis, dtableau, dtotal,
+                           stream, kernel=F.KERNEL_AUTO, threads=0):
+    """lpx_parametric_batched_dev: raw device pointers (ints, 0 / None for the nullable ones), asynchronous on
+    `stream`; the bases are outputs of primal_solve_batched_dev, dpayload holds count x (d, theta_max)."""
+    opt = F.make_options(kernel=kernel, threads=threads)
+    F.check(F.lib().lpx_parametric_batched_dev(
+        PARAM_KINDS.get(kind, kind), count, m, n, sense, F.ptr(drel), F.ptr(dbase_status), F.ptr(dbase_basis),
+        F.ptr(dbase_tableau), F.ptr(dsrc), F.ptr(dpayload), seg_cap, C.byref(opt), F.ptr(dend), F.ptr(dn_segments),
+        F.ptr(dn_pivots), F.ptr(dsegments), F.ptr(dseg_pivots), F.ptr(dbasis), F.ptr(dtableau), F.ptr(dtotal),
+        F.ptr(stream or 0)))
+
+
 def cutting_plane_dims(m, n, rel=None):
     """(max_rows, max_cols) = (m' + 50, n + m' + 50): the per-IP stride of the cutting-plane tableau output."""
     rows, cols = C.c_int(), C.c_int()

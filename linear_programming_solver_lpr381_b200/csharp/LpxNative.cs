@@ -142,6 +142,25 @@ namespace Linear_Programming_Solver.Models
             IntPtr lp_pivots, IntPtr frac_var, IntPtr cut_row, IntPtr cut_a, IntPtr cut_b, IntPtr basis, IntPtr x,
             IntPtr z, IntPtr tableau, IntPtr total_pivots, IntPtr stream);
 
+        // Parametric analysis (include/lpx.h): z*(theta) along b + theta d or c + theta d from an optimal Primal
+        // Simplex result, one CTA per query.  payload per query: d, then theta_max; segment records of
+        // lpx_param_segment_stride(n) = 4 + 2n doubles.  Every output except end may be null.
+        public const int LPX_PARAM_RHS = 1, LPX_PARAM_COST = 2;
+        public const int LPX_PARAM_REACHED = 0, LPX_PARAM_UNBOUNDED = 1, LPX_PARAM_INFEASIBLE = 2,
+            LPX_PARAM_SEG_LIMIT = 3, LPX_PARAM_NO_BASE = 4;
+        [DllImport(Lib)] public static extern UIntPtr lpx_param_payload_stride(int kind, int m, int n);
+        [DllImport(Lib)] public static extern UIntPtr lpx_param_segment_stride(int n);
+        [DllImport(Lib)] public static extern int lpx_parametric_dims(int kind, int m, int n, int[] rel, out int rows, out int cols);
+        [DllImport(Lib)]
+        public static extern int lpx_parametric(int kind, int m, int n, int sense, double[] A, int[] rel, double[] b,
+            double[] c, ref LpxOptions opt, int count, double[] payload, int seg_cap, out int base_status, int[] end,
+            int[] n_segments, int[] n_pivots, double[] segments, int[] seg_pivots, int[] basis, double[] tableau);
+        [DllImport(Lib)]
+        public static extern int lpx_parametric_batched_dev(int kind, int count, int m, int n, int sense, IntPtr rel,
+            IntPtr base_status, IntPtr base_basis, IntPtr base_tableau, IntPtr src, IntPtr payload, int seg_cap,
+            ref LpxOptions opt, IntPtr end, IntPtr n_segments, IntPtr n_pivots, IntPtr segments, IntPtr seg_pivots,
+            IntPtr basis, IntPtr tableau, IntPtr total_pivots, IntPtr stream);
+
         [DllImport(Lib)]
         public static extern int lpx_primal_solve_batched(int count, int m, int n, int sense, double[] A, int[] rel,
             double[] b, double[] c, ref LpxOptions opt, int[] status, int[] n_pivots, int[] basis, double[] x,

@@ -9,6 +9,8 @@
 //                                           prices, slacks, RHS / cost ranges; not the reference's text)
 //   lpr381 --what-if "<spec>" "Primal Simplex" [input]   repeatable: appends a "What-if" block, the optimum after
 //                                           each change, re-solved warm (whatif_host.cpp; not the reference's)
+//   lpr381 --parametric "<spec>" "Primal Simplex" [input]   repeatable: appends a "Parametric" block, the optimal
+//                                           value along a RHS or cost direction (parametric_host.cpp; not the reference's)
 #include <cstdio>
 #include <fstream>
 #include <iostream>
@@ -22,7 +24,7 @@ using namespace lpr381;
 int main(int argc, char** argv) {
     int arg = 1;
     bool as_export = false, sensitivity = false, bad_what_if = false;
-    std::vector<std::string> what_if;
+    std::vector<std::string> what_if, parametric;
     for (; arg < argc; arg++) {
         const std::string a = argv[arg];
         if (a == "--export") as_export = true;
@@ -30,6 +32,9 @@ int main(int argc, char** argv) {
         else if (a == "--sensitivity") sensitivity = true;
         else if (a == "--what-if") {
             if (++arg < argc) what_if.push_back(argv[arg]);
+            else bad_what_if = true;
+        } else if (a == "--parametric") {
+            if (++arg < argc) parametric.push_back(argv[arg]);
             else bad_what_if = true;
         } else break;
     }
@@ -39,12 +44,18 @@ int main(int argc, char** argv) {
                              "  --sensitivity (\"Primal Simplex\" only): this project's sensitivity report, not the "
                              "reference's\n"
                              "  --what-if (\"Primal Simplex\" only): rhs <i> <b_i> | cost <j> <c_j> | row <constraint> | "
-                             "col <c> <a_1> .. <a_m>\n");
+                             "col <c> <a_1> .. <a_m>\n"
+                             "  --parametric (\"Primal Simplex\" only): rhs <d_1> .. <d_m> [to <theta_max>] | "
+                             "cost <d_1> .. <d_n> [to <theta_max>]\n");
         return 2;
     }
     const std::string algorithm = argv[arg++];
     if ((sensitivity || !what_if.empty()) && algorithm != "Primal Simplex") {
         std::fprintf(stderr, "--sensitivity / --what-if: only \"Primal Simplex\" results are analysed\n");
+        return 2;
+    }
+    if (!parametric.empty() && algorithm != "Primal Simplex") {
+        std::fprintf(stderr, "--parametric: only \"Primal Simplex\" results are analysed\n");
         return 2;
     }
     std::stringstream in;
@@ -66,6 +77,7 @@ int main(int argc, char** argv) {
         LPProblem problem = LPParser::ParseFromText(input);
         if (sensitivity) sens_block = "\n\n" + SensitivityText(problem);
         if (!what_if.empty()) sens_block += "\n\n" + WhatIfText(problem, what_if);
+        if (!parametric.empty()) sens_block += "\n\n" + ParametricText(problem, parametric);
         SimplexResult result;
         // the dropdown routes "Branch and Bound Knapsack" to plain BranchAndBound upstream
         // (Form1.cs:263-270); the knapsack solver itself is reachable here under its class name

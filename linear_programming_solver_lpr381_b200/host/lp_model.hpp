@@ -125,6 +125,9 @@ struct LPController {
 std::string SensitivityText(const LPProblem& problem);
 // `lpr381 --what-if`: re-optimization queries against the optimal Primal Simplex result (whatif_host.cpp)
 std::string WhatIfText(const LPProblem& problem, const std::vector<std::string>& specs);
+// `lpr381 --parametric`: the optimal value along a RHS or cost direction from the optimal Primal Simplex result
+// (parametric_host.cpp)
+std::string ParametricText(const LPProblem& problem, const std::vector<std::string>& specs);
 
 // Environment.NewLine of the host ("\n"; the reference's Windows build uses "\r\n")
 std::string& NewLine();
