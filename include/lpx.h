@@ -549,6 +549,22 @@ int lpx_parametric(int kind, int m, int n, int sense, const double* A, const int
                    const double* c, const lpx_options* opt, int count, const double* payload, int seg_cap,
                    int* base_status, int* end, int* n_segments, int* n_pivots, double* segments, int* seg_pivots,
                    int* basis, double* tableau);
+/* The parametric analysis defined above, for one query against an optimal base session, on the whole GPU. */
+/* kind / payload (host pointer, lpx_param_payload_stride(kind, m, n) doubles, m / n the base model's) are the
+ * definition above, applied to the base's current tableau and basis; the results equal oracle/orc_param.cpp on them
+ * (and lpx_parametric_batched_dev on the same base) bit for bit.  Host buffers, synchronous, ordered after the base's
+ * enqueued work; the base is only read and may be stepped, read or queried afterwards.  Outputs as one query of
+ * lpx_parametric: end, n_segments, n_pivots, segments [seg_cap][4 + 2n], seg_pivots [seg_cap][2], basis [m'] and the
+ * compact working tableau ((m' + 1) x (W + 1) for RHS, (m' + 2) x W for COST); every output except end may be NULL.
+ * opt NULL: the base's options.  opt.stream_block is K, the breakpoints decided per HBM pass (0: 8, at most 16; 1: one
+ * pass per breakpoint); opt.stream_pass_variant picks the blocked pass.  A base whose status, as of its last step /
+ * sync, is not LPX_OPTIMAL gets end LPX_PARAM_NO_BASE, 0 segments and zeroed outputs (seg_pivots -1).
+ * LPX_E_BAD_ARGS (before any device work, lpx_last_error() says why): a NULL base / payload / end, an unknown kind,
+ * seg_cap < 1, a NaN or negative theta_max, a Dual Simplex session as base, or the query session of an added row or
+ * column as base.  The query session of an RHS / COST edit is a valid base, analysed on its modified model. */
+int lpx_session_parametric(const lpx_session* base, int kind, const double* payload, int seg_cap,
+                           const lpx_options* opt, int* end, int* n_segments, int* n_pivots, double* segments,
+                           int* seg_pivots, int* basis, double* tableau);
 
 /* ---- measurement helpers (bench.py) --------------------------------------------------------- */
 /* Unfused FP64 rate (separate DMUL and DADD, the only arithmetic the bit-exactness contract

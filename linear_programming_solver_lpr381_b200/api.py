@@ -467,6 +467,32 @@ class Session:
         q.rows, q.cols = r.value, cc.value
         return q
 
+    def parametric(self, kind, direction, theta_max=np.inf, seg_cap=64, want_tableau=True, **opts):
+        """lpx_session_parametric: z*(theta) along b + theta d ("rhs") or c + theta d ("cost", or LPX_PARAM_*) on
+        theta in [0, theta_max] against this session, which is only read, on the whole GPU.  opts (kblock: breakpoints
+        per HBM pass, pass_variant) select the protocol; none given: this session's options.  Returns the per-query
+        fields of parametric(): end, n_segments, n_pivots, segments (seg_cap, 4 + 2n) with its split_segments views,
+        seg_pivots (seg_cap, 2), basis and tableau."""
+        kind = PARAM_KINDS.get(kind, kind)
+        d = np.ascontiguousarray(direction, dtype=np.float64).ravel()
+        if kind in PARAM_KINDS.values() and d.size + 1 != param_payload_stride(kind, self.m, self.n):
+            raise F.LpxError(F.E_BAD_ARGS, "a direction has %d entries, kind %d needs %d" % (
+                d.size, kind, param_payload_stride(kind, self.m, self.n) - 1))
+        pay = np.ascontiguousarray(np.append(d, float(theta_max)))
+        opt = F.make_options(**opts) if opts else None
+        mm = self.rows - 1
+        rows, cols = (mm + 2, self.cols) if kind == F.PARAM_COST else (mm + 1, self.cols + 1)
+        end, ns, npv = C.c_int(), C.c_int(), C.c_int()
+        out = dict(segments=np.zeros((seg_cap, 4 + 2 * self.n)), seg_pivots=np.zeros((seg_cap, 2), np.int32),
+                   basis=np.zeros(mm, np.int32), tableau=np.zeros((rows, cols)) if want_tableau else None)
+        F.check(F.lib().lpx_session_parametric(
+            self._h, kind, F.ptr(pay), seg_cap, None if opt is None else C.cast(C.byref(opt), C.c_void_p),
+            C.byref(end), C.byref(ns), C.byref(npv),
+            *[F.ptr(out[k]) for k in ("segments", "seg_pivots", "basis", "tableau")]))
+        out.update(end=end.value, n_segments=ns.value, n_pivots=npv.value)
+        out.update(split_segments(out["segments"], self.n))
+        return out
+
     def sensitivity(self):
         """Sensitivity report of the session's tableau (NaNs unless its status is OPTIMAL): `report` and its
         named views."""

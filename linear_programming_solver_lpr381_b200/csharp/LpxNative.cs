@@ -160,6 +160,12 @@ namespace Linear_Programming_Solver.Models
             IntPtr base_status, IntPtr base_basis, IntPtr base_tableau, IntPtr src, IntPtr payload, int seg_cap,
             ref LpxOptions opt, IntPtr end, IntPtr n_segments, IntPtr n_pivots, IntPtr segments, IntPtr seg_pivots,
             IntPtr basis, IntPtr tableau, IntPtr total_pivots, IntPtr stream);
+        // One query against an OPTIMAL session, on the whole GPU (host buffers, synchronous; the base is only read);
+        // opt IntPtr.Zero = the base's options (stream_block: breakpoints per HBM pass).  Any output but end may be null.
+        [DllImport(Lib)]
+        public static extern int lpx_session_parametric(IntPtr base_session, int kind, double[] payload, int seg_cap,
+            IntPtr opt, out int end, out int n_segments, out int n_pivots, double[] segments, int[] seg_pivots,
+            int[] basis, double[] tableau);
 
         [DllImport(Lib)]
         public static extern int lpx_primal_solve_batched(int count, int m, int n, int sense, double[] A, int[] rel,

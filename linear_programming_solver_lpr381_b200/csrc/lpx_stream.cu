@@ -482,6 +482,7 @@ __global__ void __launch_bounds__(256, 4) stream_update_kernel(StreamParams P) {
 #include "lpx_stream_pipe.cuh"
 #include "lpx_stream_reopt.cuh"
 #include "lpx_stream_dual.cuh"
+#include "lpx_stream_param.cuh"
 
 
 // ---- session object -----------------------------------------------------------------------------
@@ -747,8 +748,10 @@ static int launch_block(lpx_session* s, int budget) {
 // 100 silent pivots of a Dual Simplex session) with the blocked dual look-ahead (stream_dual_lookahead_kernel + the
 // blocked pass) or, for stream_protocol 1 / 2 or when its carve does not fit, the per-pivot protocol
 // (stream_dual_select_kernel + stream_update_kernel<4>); otherwise opt's Primal Simplex protocol.  m_in / n: the
-// model's constraints and variables (b, c).
-static lpx_session* session_new(int m_in, int n, int sense, int mm, const lpx_options* opt, bool dual) {
+// model's constraints and variables (b, c).  xcol / xrow: room for one more column past the width (ld) or one more
+// row below the z-row (rows, colstride): the direction column g / row h of a parametric working session.
+static lpx_session* session_new(int m_in, int n, int sense, int mm, const lpx_options* opt, bool dual, int xcol = 0,
+                                int xrow = 0) {
     lpx_session* s = new lpx_session();
     lpx_default_options(&s->opt);
     if (opt) s->opt = *opt;
@@ -767,9 +770,9 @@ static lpx_session* session_new(int m_in, int n, int sense, int mm, const lpx_op
     StreamParams& P = s->P;
     P.m = mm;
     P.n = n;
-    P.rows = mm + 1;
+    P.rows = mm + 1 + xrow;
     P.width = n + mm + 1;
-    P.ld = (P.width + 15) & ~15;
+    P.ld = (P.width + xcol + 15) & ~15;
     P.colstride = (P.rows + 15) & ~15;
     P.max_iter = dual ? LPX_DUAL_MAX_ITER : s->opt.max_iterations;
     P.pivlog_cap = std::max(1, std::min(P.max_iter, 1 << 20)) + (dual ? LPX_DUAL_SILENT_MAX : 0);
@@ -1017,6 +1020,32 @@ static lpx_session* session_create(int m, int n, int sense, const double* dA, co
     return s;
 }
 
+// The terms of a change d[m_in] of b (RHS and COL edits, the parametric RHS direction), in the definition's order:
+// d_i * T[r][s1], and for an EQ row - d_i * T[r][s2].
+static void slack_terms(const lpx_session* base, const double* d, std::vector<ReoptTerm>& terms) {
+    for (int i = 0; i < base->m_in; i++) {
+        if (d[i] == 0.0) continue;
+        const int r = base->rmap[i];
+        const int s1 = base->n + (r < 0 ? -r - 1 : r);
+        terms.push_back(ReoptTerm{d[i], s1, 0});
+        if (r < 0) terms.push_back(ReoptTerm{d[i], s1 + 1, 1});
+    }
+}
+
+// The terms of a change d[n] of c in the model's sense (COST edits, the parametric COST direction): delta_j with the
+// basic row of column j (-1: non-basic).  bb: the base's basis.
+static void cost_terms(const lpx_session* base, const std::vector<int>& bb, const double* d,
+                       std::vector<ReoptTerm>& terms) {
+    const int n = base->n;
+    std::vector<int> rowof(n, -1);
+    for (int r = 0; r < (int)bb.size(); r++)
+        if (bb[r] < n) rowof[bb[r]] = r;
+    for (int j = 0; j < n; j++) {
+        if (d[j] == 0.0) continue;
+        terms.push_back(ReoptTerm{base->sense == 1 ? -d[j] : d[j], rowof[j], j});
+    }
+}
+
 // lpx_session_reoptimize: the query session of one what-if edit of an optimal base session (include/lpx.h,
 // "Re-optimization").  The terms of the edit are listed on the host in the definition's order; the build kernel
 // writes the query's tableau straight from the base's current buffer, then the query's protocol is armed as a new
@@ -1053,26 +1082,11 @@ static lpx_session* session_reoptimize(const lpx_session* base, int kind, const 
     std::vector<int> qb(bb), qmap(base->rmap);
     std::vector<double> qbv(hb), qcv(hc);
     double zstart = 0.0;
-    auto slack_terms = [&](const double* d) {
-        for (int i = 0; i < m_in; i++) {
-            if (d[i] == 0.0) continue;
-            const int r = base->rmap[i];
-            const int s1 = n + (r < 0 ? -r - 1 : r);
-            terms.push_back(ReoptTerm{d[i], s1, 0});
-            if (r < 0) terms.push_back(ReoptTerm{d[i], s1 + 1, 1});
-        }
-    };
     if (kind == LPX_REOPT_RHS) {
-        slack_terms(pay);
+        slack_terms(base, pay, terms);
         for (int i = 0; i < m_in; i++) qbv[i] = hb[i] + pay[i];
     } else if (kind == LPX_REOPT_COST) {
-        std::vector<int> rowof(n, -1);
-        for (int r = 0; r < mb; r++)
-            if (bb[r] < n) rowof[bb[r]] = r;
-        for (int j = 0; j < n; j++) {
-            if (pay[j] == 0.0) continue;
-            terms.push_back(ReoptTerm{base->sense == 1 ? -pay[j] : pay[j], rowof[j], j});
-        }
+        cost_terms(base, bb, pay, terms);
         for (int j = 0; j < n; j++) qcv[j] = hc[j] + pay[j];
     } else if (kind == LPX_REOPT_ROW) {
         for (int r = 0; r < mb; r++) {
@@ -1084,7 +1098,7 @@ static lpx_session* session_reoptimize(const lpx_session* base, int kind, const 
         qmap.push_back(mb);
         qbv.push_back(ge ? -pay[n + 1] : pay[n + 1]);
     } else {
-        slack_terms(pay);
+        slack_terms(base, pay, terms);
         const double cp = base->sense == 1 ? -pay[m_in] : pay[m_in];
         zstart = -cp;
         for (int& j : qb)
@@ -1135,6 +1149,167 @@ static lpx_session* session_reoptimize(const lpx_session* base, int kind, const 
         return nullptr;
     }
     return s;
+}
+
+// Where the parametric look-ahead keeps its vectors: in dynamic shared memory, in the order below, each one that fits
+// next to those placed before it; the others in global memory (`scratch`, 2 ld + 3 colstride doubles, which L2
+// holds).  Every shape runs: at worst every vector is in global memory.  Returns the dynamic shared-memory bytes.
+static size_t param_place(const StreamParams& P, bool cost, double* scratch, ParamLa& A) {
+    size_t len[PV_N];
+    len[PV_Z] = P.ld;
+    len[PV_HG] = cost ? P.ld : P.colstride;
+    len[PV_RHS] = P.colstride;
+    len[PV_COL] = P.colstride;
+    len[PV_RATIO] = cost ? P.colstride : P.ld;
+    const int order[PV_N] = {PV_RHS, PV_COL, PV_HG, PV_RATIO, PV_Z};
+    const size_t cap = ((size_t)max_smem_optin() - 4096) / 8;  // 4 KB for the kernel's static shared memory
+    size_t used = 0, g = 0;
+    for (int v : order) {
+        A.gvec[v] = scratch + g;
+        g += len[v];
+        A.soff[v] = -1;
+        if (used + len[v] <= cap) {
+            A.soff[v] = (int)used;
+            used += len[v];
+        }
+    }
+    return used * 8;
+}
+
+// lpx_session_parametric with its arguments checked.  A working session of the working shape (RHS: ld with room for
+// g at column W, P.width = W so every rule still finds the RHS at W - 1; COST: h as row m' + 1, P.rows = m' + 2 with
+// the z-row still at P.m = m') is built from the base's current buffer; then blocks of stream_param_lookahead_kernel
+// + the blocked pass are enqueued in chunks behind the device status word (ParamState::end), one synchronise per
+// chunk, and the outputs are copied out.  The base is only read.
+static int session_parametric(const lpx_session* base, int kind, const double* pay, int seg_cap, const lpx_options* opt,
+                              int* end, int* n_segments, int* n_pivots, double* segments, int* seg_pivots, int* basis,
+                              double* tableau) {
+    const StreamParams& B = base->P;
+    const int n = base->n, mb = B.m, W = B.width;
+    const bool cost = kind == LPX_PARAM_COST;
+    const int rows = mb + 1 + (cost ? 1 : 0), cols = W + (cost ? 0 : 1);
+    const size_t sstride = lpx_param_segment_stride(n), cap = (size_t)seg_cap;
+    StreamCtl h;
+    std::vector<int> bb(mb);
+    LPX_CUDA(cudaMemcpyAsync(&h, B.ctl, sizeof h, cudaMemcpyDeviceToHost, base->stream));
+    LPX_CUDA(cudaMemcpyAsync(bb.data(), B.basis, (size_t)mb * 4, cudaMemcpyDeviceToHost, base->stream));
+    LPX_CUDA(cudaStreamSynchronize(base->stream));
+    if (h.status != LPX_OPTIMAL) {
+        *end = LPX_PARAM_NO_BASE;
+        if (n_segments) *n_segments = 0;
+        if (n_pivots) *n_pivots = 0;
+        if (segments) std::fill(segments, segments + cap * sstride, 0.0);
+        if (seg_pivots) std::fill(seg_pivots, seg_pivots + 2 * cap, -1);
+        if (basis) std::fill(basis, basis + mb, 0);
+        if (tableau) std::fill(tableau, tableau + (size_t)rows * cols, 0.0);
+        return LPX_OK;
+    }
+    const double* Tb = (base->pipe && pipe_current_buffer(base, h)) ? B.T1 : B.T;
+    std::vector<ReoptTerm> terms;
+    if (cost)
+        cost_terms(base, bb, pay, terms);
+    else
+        slack_terms(base, pay, terms);
+    // the working session always runs the parametric look-ahead and the blocked pass; protocol 4 (blocked, not
+    // pipelined) keeps session_new from allocating the pipelined protocol's second tableau
+    lpx_options o = opt ? *opt : base->opt;
+    o.stream_protocol = 4;
+    lpx_session* s = session_new(base->m_in, n, base->sense, mb, &o, false, cost ? 0 : 1, cost ? 1 : 0);
+    if (!s) return LPX_E_CUDA;
+    StreamParams& P = s->P;
+    P.kblock = o.stream_block > 0 ? std::min(o.stream_block, LPX_BLOCK_KMAX) : 8;
+    size_block_pass(P, o.stream_pass_variant, &s->rpc_block, &s->grid_block);
+    double* dvec = (double*)sess_alloc(s, (2 * (size_t)P.ld + 3 * (size_t)P.colstride) * 8);
+    ParamState* dstate = (ParamState*)sess_alloc(s, sizeof(ParamState));
+    int* disb = cost ? (int*)sess_alloc(s, (size_t)W * 4) : nullptr;
+    ReoptTerm* dterms = (ReoptTerm*)sess_alloc(s, std::max<size_t>(terms.size(), 1) * sizeof(ReoptTerm));
+    double* dseg = segments ? (double*)sess_alloc(s, cap * sstride * 8) : nullptr;
+    int* dspv = seg_pivots ? (int*)sess_alloc(s, cap * 2 * 4) : nullptr;
+    if (!dvec || !dstate || (cost && !disb) || !dterms || (segments && !dseg) || (seg_pivots && !dspv)) {
+        sess_free(s);
+        return LPX_E_CUDA;
+    }
+    ParamLa A{};
+    const size_t smem = param_place(P, cost, dvec, A);
+    A.isb = disb;
+    A.st = dstate;
+    A.seg = dseg;
+    A.spv = dspv;
+    A.seg_cap = seg_cap;
+    A.n = n;
+    A.theta_max = pay[lpx_param_payload_stride(kind, base->m_in, n) - 1];
+    void (*la)(StreamParams, ParamLa) = cost ? stream_param_lookahead_kernel<true> : stream_param_lookahead_kernel<false>;
+    const ParamState h0{0.0, 0, -1};
+    std::vector<int> isb(cost ? W : 0, 0);
+    for (int r = 0; r < mb && cost; r++) isb[bb[r]] = 1;
+    cudaStream_t st = s->stream;
+    bool ok = cudaFuncSetAttribute(la, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) == cudaSuccess;
+    ok = ok && (terms.empty() || cudaMemcpyAsync(dterms, terms.data(), terms.size() * sizeof(ReoptTerm),
+                                                 cudaMemcpyHostToDevice, st) == cudaSuccess);
+    ok = ok && cudaMemcpyAsync(dstate, &h0, sizeof h0, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    ok = ok && (!cost || cudaMemcpyAsync(disb, isb.data(), (size_t)W * 4, cudaMemcpyHostToDevice, st) == cudaSuccess);
+    ok = ok && cudaMemcpyAsync(P.basis, bb.data(), (size_t)mb * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    ok = ok && (!dseg || cudaMemsetAsync(dseg, 0, cap * sstride * 8, st) == cudaSuccess);
+    ok = ok && (!dspv || cudaMemsetAsync(dspv, 0xff, cap * 2 * 4, st) == cudaSuccess);  // (-1, -1)
+    if (ok) {
+        // validate with no constraints only resets StreamCtl (0 pivots, block_cnt 0)
+        stream_validate_kernel<<<1, 1024, 0, st>>>(P.ctl, nullptr, 0, INT_MAX);
+        const int strips = (P.ld + 255) / 256;
+        const int groups = std::max(1, std::min(P.rows, sm_count() * 8 / strips));
+        stream_param_build_kernel<<<dim3(strips, groups, 1), 256, 0, st>>>(P, Tb, B.ld, mb, cost ? 1 : 0, dterms,
+                                                                           (int)terms.size());
+        count_launch(2);
+        if (!cost) {
+            stream_param_g_kernel<<<(P.rows + LPX_PARAM_G_THREADS - 1) / LPX_PARAM_G_THREADS, LPX_PARAM_G_THREADS, 0,
+                                    st>>>(P, Tb, B.ld, dterms, (int)terms.size());
+            count_launch();
+        }
+        ok = cudaGetLastError() == cudaSuccess;
+    }
+    // every block but the last decides K pivots, and there are at most seg_cap - 1 of them
+    const long long max_blocks = (cap - 1 + P.kblock - 1) / P.kblock + 1;
+    long long launched = 0;
+    int chunk = 1;
+    ParamState hs = h0;
+    while (ok) {
+        const int todo = (int)std::min<long long>(chunk, max_blocks - launched);
+        for (int b = 0; b < todo; b++) {
+            la<<<1, 1024, smem, st>>>(P, A);
+            launch_block_pass(s);
+            count_launch(2);
+        }
+        launched += todo;
+        ok = cudaGetLastError() == cudaSuccess &&
+             cudaMemcpyAsync(&hs, dstate, sizeof hs, cudaMemcpyDeviceToHost, st) == cudaSuccess &&
+             cudaStreamSynchronize(st) == cudaSuccess;
+        if (!ok || hs.end >= 0) break;
+        if (launched >= max_blocks) {
+            set_error("lpx_session_parametric: the analysis did not end within seg_cap segments");
+            sess_free(s);
+            return LPX_E_CUDA;
+        }
+        chunk = std::min(2 * chunk, 64);
+    }
+    if (ok) {
+        *end = hs.end;
+        if (n_segments) *n_segments = hs.k;
+        if (n_pivots) *n_pivots = hs.k - 1;
+        auto down = [&](void* dst, const void* from, size_t bytes) {
+            return !dst || cudaMemcpyAsync(dst, from, bytes, cudaMemcpyDeviceToHost, st) == cudaSuccess;
+        };
+        ok = down(segments, dseg, cap * sstride * 8) && down(seg_pivots, dspv, cap * 2 * 4) &&
+             down(basis, P.basis, (size_t)mb * 4) &&
+             (!tableau || cudaMemcpy2DAsync(tableau, (size_t)cols * 8, P.T, (size_t)P.ld * 8, (size_t)cols * 8, rows,
+                                            cudaMemcpyDeviceToHost, st) == cudaSuccess) &&
+             cudaStreamSynchronize(st) == cudaSuccess;
+    }
+    if (!ok) {
+        cuda_fail(cudaGetLastError(), "lpx_session_parametric", __FILE__, __LINE__);
+        sess_free(s);
+        return LPX_E_CUDA;
+    }
+    sess_free(s);
+    return LPX_OK;
 }
 
 int stream_solve_host(int m, int n, int sense, const double* A, const int* rel, const double* b, const double* c,
@@ -1294,6 +1469,33 @@ lpx_session* lpx_session_reoptimize(const lpx_session* base, int kind, const dou
     if (ensure_device() != LPX_OK) return nullptr;
     std::lock_guard<std::recursive_mutex> lk(rt().mu);
     return session_reoptimize(base, kind, payload, opt);
+}
+
+int lpx_session_parametric(const lpx_session* base, int kind, const double* payload, int seg_cap,
+                           const lpx_options* opt, int* end, int* n_segments, int* n_pivots, double* segments,
+                           int* seg_pivots, int* basis, double* tableau) {
+    if (!base || !payload || !end || (kind != LPX_PARAM_RHS && kind != LPX_PARAM_COST) || seg_cap < 1) {
+        set_error("lpx_session_parametric: bad arguments (NULL base, payload or end, an unknown kind, or seg_cap < 1)");
+        return LPX_E_BAD_ARGS;
+    }
+    if (!(payload[lpx_param_payload_stride(kind, base->m_in, base->n) - 1] >= 0.0)) {
+        set_error("lpx_session_parametric: theta_max must be >= 0 or +inf (not NaN)");
+        return LPX_E_BAD_ARGS;
+    }
+    if (base->dual_model) {
+        set_error("lpx_session_parametric: the base is a Dual Simplex session (its tableau treats '>=' rows as '<='); "
+                  "parametric analysis is defined for Primal Simplex results");
+        return LPX_E_BAD_ARGS;
+    }
+    if (!base->sens_ok) {
+        set_error("lpx_session_parametric: not defined for the query session of an added row or column");
+        return LPX_E_BAD_ARGS;
+    }
+    int rc = ensure_device();
+    if (rc != LPX_OK) return rc;
+    std::lock_guard<std::recursive_mutex> lk(rt().mu);
+    return session_parametric(base, kind, payload, seg_cap, opt, end, n_segments, n_pivots, segments, seg_pivots, basis,
+                              tableau);
 }
 
 int lpx_session_step_async(lpx_session* s, int max_pivots) {
