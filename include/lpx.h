@@ -566,6 +566,63 @@ int lpx_session_parametric(const lpx_session* base, int kind, const double* payl
                            const lpx_options* opt, int* end, int* n_segments, int* n_pivots, double* segments,
                            int* seg_pivots, int* basis, double* tableau);
 
+/* ---- Two-phase Simplex — NOT the reference's ---------------------------------------------------------------- */
+/* A textbook two-phase Primal Simplex that solves models with '>=' rows, '=' rows and negative right-hand sides, which
+ * every reference-exact solver rejects or solves as a different model.  Checked against oracle/orc_twophase.cpp bit
+ * for bit and against an independent LP solver.  FP64 with separate multiply / add / subtract and true division;
+ * EPS = 1e-9.  One LP:
+ *   Normalisation  a row with b_i < 0 (strictly: -0.0 is not flipped) has every a_ij and b_i negated exactly; LE
+ *                  becomes GE and GE becomes LE.  EQ rows are not expanded.
+ *   Columns        the n structural columns; one slack per LE / GE row in row order (+1 for LE, -1 for GE); one
+ *                  artificial (+1) per GE / EQ row after normalisation, in row order; the RHS.  With s the number of
+ *                  non-EQ rows (it depends on rel only) and a the number of artificials (it depends on b too),
+ *                  W = n + s + a + 1 and the artificial of the k-th such row is column n + s + k.
+ *   Rows           0..m-1 the constraints; m the objective row as BuildTableau writes it (-c_j for Max, c_j for Min,
+ *                  +0 elsewhere); m+1 the Phase I row: for every non-artificial column j and the RHS,
+ *                  w_j = ((+0 - T[i1][j]) - T[i2][j]) - ... over the artificial rows in row order; +0 on the artificial
+ *                  columns.  An LE row starts with its slack basic, a GE / EQ row with its artificial.
+ *   Phase I        ChooseEntering on row m+1 over columns 0..W-2 (most negative below -EPS, lowest index on ties, NaN
+ *                  never chosen); ChooseLeaving over rows 0..m-1 (ratio over entries > EPS, the sequential rule with
+ *                  margin 1e-9); PrimalSimplex.Pivot on rows 0..m+1, every column.  It stops when no column enters or
+ *                  no row leaves.
+ *   Feasibility    w = T[m+1][W-1], S = the normalised b summed over the artificial rows in row order from +0,
+ *                  tol = 1e-9 * (1 + S).  INFEASIBLE iff !(w >= -tol) (a NaN is infeasible).
+ *   Drive-out      for each row r ascending whose basic variable is an artificial: pivot (rows 0..m+1) on the
+ *                  lowest-index non-artificial column j with |T[r][j]| > EPS; none: the row is redundant and its
+ *                  artificial stays basic.  These are Phase I pivots: logged and counted.
+ *   Phase II       ChooseEntering on row m over columns 0..n+s-1; leaving rule as in Phase I; the pivot updates
+ *                  rows 0..m.  Row m+1 and the artificial columns are not read again.
+ *   Limit          "iter > max_iterations" before choosing a column, in both phases, counting every pivot
+ *                  (drive-out pivots are counted, not checked): LPX_S_ITER_LIMIT.
+ * For all-'<=' models with b >= 0 there is no artificial, Phase I is empty, and every output equals
+ * lpx_primal_solve_batched's bit for bit.  Per LP, describing the tableau where the solve stopped whatever the status:
+ *   status         LPX_OPTIMAL / LPX_UNBOUNDED / LPX_INFEASIBLE / LPX_S_ITER_LIMIT;
+ *   phase1_pivots  Phase I pivots, drive-out included; n_pivots: all pivots;
+ *   pivots         [pivots_cap][2] (entering column, leaving row), the first pivots_cap pivots, (-1, -1) past the last;
+ *   basis          [m], internal column numbers;  x [n]: x_j = T[r][W-1] when j is basic in row r, else +0;
+ *   z              T[m][W-1], the engine's convention: for Min the maximum of -c.x, as every other entry point;
+ *   tableau        rows 0..m and the columns 0..n+s-1 plus the RHS, compact: lpx_two_phase_dims = (m+1) x (n+s+1).
+ * Every output except status may be NULL.  opt.kernel: AUTO (the tableau in shared memory when the widest shape,
+ * (m + 2) x (n + s + m + 1), fits, else in global memory), LPX_KERNEL_CTA_SMEM (LPX_E_CAPACITY when it does not fit)
+ * or LPX_KERNEL_CTA_GLOBAL; any other value is LPX_E_BAD_ARGS, as are count < 0, m < 1, n < 1, a sense outside 0..1,
+ * a rel value outside 0..2, a NULL A / b / c / status and pivots_cap < 0 (checked before any device work).
+ * opt.threads (128 / 256 / 512) is honoured.  Scope: no sensitivity, re-optimization or parametric analysis on these
+ * results (their slack layout is not the one those definitions read). */
+/* rows / cols of the output tableau: m + 1, n + s + 1 (rel: host pointer, nullable = all LE) */
+int lpx_two_phase_dims(int m, int n, const int* rel, int* rows, int* cols);
+/* Host buffers, strided per LP: A[count][m][n], b[count][m], c[count][n]; rel[m] shared. */
+int lpx_two_phase_solve_batched(int count, int m, int n, int sense, const double* A, const int* rel, const double* b,
+                                const double* c, const lpx_options* opt, int* status, int* phase1_pivots,
+                                int* n_pivots, int* pivots, int pivots_cap, int* basis, double* x, double* z,
+                                double* tableau, long long* total_pivots);
+/* Same, all pointers are DEVICE pointers (rel too; it is read back once for the shape and checked then), asynchronous
+ * on `stream`.  total_pivots: as in lpx_primal_solve_batched_dev (zero it first). */
+int lpx_two_phase_solve_batched_dev(int count, int m, int n, int sense, const double* A, const int* rel,
+                                    const double* b, const double* c, const lpx_options* opt, int* status,
+                                    int* phase1_pivots, int* n_pivots, int* pivots, int pivots_cap, int* basis,
+                                    double* x, double* z, double* tableau, unsigned long long* total_pivots,
+                                    void* stream);
+
 /* ---- measurement helpers (bench.py) --------------------------------------------------------- */
 /* Unfused FP64 rate (separate DMUL and DADD, the only arithmetic the bit-exactness contract
  * allows) in TFLOP/s: the roofline denominator of the on-chip batched kernels. */

@@ -39,7 +39,8 @@ EXPORTS = [
     "lpx_reoptimize_batched_dev", "lpx_reoptimize", "lpx_session_reoptimize", "lpx_dual_session_open",
     "lpx_dual_session_open_dev", "lpx_session_silent_pivots", "lpx_cutting_plane_dims", "lpx_cutting_plane_batched",
     "lpx_cutting_plane_batched_dev", "lpx_param_payload_stride", "lpx_param_segment_stride", "lpx_parametric_dims",
-    "lpx_parametric_batched_dev", "lpx_parametric", "lpx_session_parametric",
+    "lpx_parametric_batched_dev", "lpx_parametric", "lpx_session_parametric", "lpx_two_phase_dims",
+    "lpx_two_phase_solve_batched", "lpx_two_phase_solve_batched_dev",
 ]
 
 
@@ -165,6 +166,9 @@ def lib():
     L.lpx_parametric_dims.argtypes = [C.c_int, C.c_int, C.c_int, C.c_void_p, _ip, _ip]
     L.lpx_parametric_batched_dev.argtypes = [C.c_int] * 5 + [C.c_void_p] * 6 + [C.c_int] + [C.c_void_p] * 10
     L.lpx_parametric.argtypes = [C.c_int] * 4 + [C.c_void_p] * 5 + [C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 8
+    L.lpx_two_phase_dims.argtypes = [C.c_int, C.c_int, C.c_void_p, _ip, _ip]
+    L.lpx_two_phase_solve_batched.argtypes = [C.c_int] * 4 + [C.c_void_p] * 9 + [C.c_int] + [C.c_void_p] * 4 + [_llp]
+    L.lpx_two_phase_solve_batched_dev.argtypes = [C.c_int] * 4 + [C.c_void_p] * 9 + [C.c_int] + [C.c_void_p] * 6
     L.lpx_session_parametric.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 8
     L.lpx_bnb_simplex_batched.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,

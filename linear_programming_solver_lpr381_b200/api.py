@@ -383,6 +383,63 @@ def cutting_plane_batched_dev(count, m, n, sense, dA, drel, db, dc, dend, dn_rou
         F.ptr(stream or 0)))
 
 
+def two_phase_dims(m, n, rel=None):
+    """(rows, cols) of the two-phase output tableau: m + 1, n + s + 1 with s the non-EQ rows."""
+    rows, cols = C.c_int(), C.c_int()
+    rel = None if rel is None else np.ascontiguousarray(rel, dtype=np.int32)
+    F.check(F.lib().lpx_two_phase_dims(m, n, F.ptr(rel), C.byref(rows), C.byref(cols)))
+    return rows.value, cols.value
+
+
+def two_phase_solve_batched(A, b, c, rel=None, sense=0, max_iterations=10000, kernel=F.KERNEL_AUTO, threads=0,
+                            pivots_cap=None, want_tableau=True):
+    """lpx_two_phase_solve_batched: the two-phase Simplex (include/lpx.h; not the reference's) for `count` LPs of one
+    shape (A (count, m, n), b (count, m), c (count, n), rel shared).  Returns status, phase1_pivots, n_pivots (count),
+    pivots (count, pivots_cap, 2; (-1, -1) past the last; default cap 4 (m + n)), basis (count, m), x (count, n),
+    z (count; for Min the maximum of -c.x), tableau (count, m + 1, n + s + 1) and total_pivots."""
+    A, b, c, rel = _prep(A, b, c, rel)
+    count, m, n = A.shape
+    rows, cols = two_phase_dims(m, n, rel)
+    cap = 4 * (m + n) if pivots_cap is None else pivots_cap
+    opt = F.make_options(max_iterations, kernel, threads)
+    out = dict(status=np.zeros(count, np.int32), phase1_pivots=np.zeros(count, np.int32),
+               n_pivots=np.zeros(count, np.int32), pivots=np.zeros((count, cap, 2), np.int32),
+               basis=np.zeros((count, m), np.int32), x=np.zeros((count, n)), z=np.zeros(count),
+               tableau=np.zeros((count, rows, cols)) if want_tableau else None)
+    total = C.c_longlong()
+    F.check(F.lib().lpx_two_phase_solve_batched(
+        count, m, n, sense, F.ptr(A), F.ptr(rel), F.ptr(b), F.ptr(c), C.byref(opt),
+        *[F.ptr(out[k]) for k in ("status", "phase1_pivots", "n_pivots", "pivots")], cap,
+        *[F.ptr(out[k]) for k in ("basis", "x", "z", "tableau")], C.byref(total)))
+    out["total_pivots"] = total.value
+    return out
+
+
+def two_phase_solve(A, b, c, rel=None, sense=0, max_iterations=10000, **kw):
+    """One LP through two_phase_solve_batched: the same fields without the leading count axis, `pivots` cut to the
+    pivots made (the first max_iterations + m by default)."""
+    A = np.asarray(A, dtype=np.float64)
+    m, n = A.shape
+    kw.setdefault("pivots_cap", max_iterations + m)
+    r = two_phase_solve_batched(A[None], np.asarray(b, np.float64)[None], np.asarray(c, np.float64)[None], rel, sense,
+                                max_iterations, **kw)
+    out = {k: (v[0] if isinstance(v, np.ndarray) else v) for k, v in r.items()}
+    out["pivots"] = out["pivots"][: min(int(out["n_pivots"]), out["pivots"].shape[0])]
+    return out
+
+
+def two_phase_solve_batched_dev(count, m, n, sense, dA, drel, db, dc, dstatus, dphase1, dnpiv, dpivots, pivots_cap,
+                                dbasis, dx, dz, dtableau, dtotal, stream, max_iterations=10000, kernel=F.KERNEL_AUTO,
+                                threads=0):
+    """lpx_two_phase_solve_batched_dev: raw device pointers (ints, 0 / None for the nullable ones), asynchronous on
+    `stream` (a cudaStream_t)."""
+    opt = F.make_options(max_iterations, kernel, threads)
+    F.check(F.lib().lpx_two_phase_solve_batched_dev(
+        count, m, n, sense, F.ptr(dA), F.ptr(drel), F.ptr(db), F.ptr(dc), C.byref(opt), F.ptr(dstatus),
+        F.ptr(dphase1), F.ptr(dnpiv), F.ptr(dpivots), pivots_cap, F.ptr(dbasis), F.ptr(dx), F.ptr(dz),
+        F.ptr(dtableau), F.ptr(dtotal), F.ptr(stream or 0)))
+
+
 class Session:
     """Large single LP whose tableau lives in HBM (lpx_session_*).  dual=True: DualSimplex.Solve on the model
     (lpx_dual_session_open); the silent ForceDualFeasibility pivots run inside the constructor and `.silent` counts

@@ -160,6 +160,20 @@ namespace Linear_Programming_Solver.Models
             IntPtr base_status, IntPtr base_basis, IntPtr base_tableau, IntPtr src, IntPtr payload, int seg_cap,
             ref LpxOptions opt, IntPtr end, IntPtr n_segments, IntPtr n_pivots, IntPtr segments, IntPtr seg_pivots,
             IntPtr basis, IntPtr tableau, IntPtr total_pivots, IntPtr stream);
+
+        // Two-phase Simplex (include/lpx.h; not the reference's): '>=' rows, '=' rows and negative right-hand sides,
+        // one CTA per LP.  Output tableau (m + 1) x (n + s + 1), s = non-'=' rows; pivots past the last are (-1, -1).
+        // Every output except status may be null.
+        [DllImport(Lib)] public static extern int lpx_two_phase_dims(int m, int n, int[] rel, out int rows, out int cols);
+        [DllImport(Lib)]
+        public static extern int lpx_two_phase_solve_batched(int count, int m, int n, int sense, double[] A, int[] rel,
+            double[] b, double[] c, ref LpxOptions opt, int[] status, int[] phase1_pivots, int[] n_pivots, int[] pivots,
+            int pivots_cap, int[] basis, double[] x, double[] z, double[] tableau, out long total_pivots);
+        [DllImport(Lib)]
+        public static extern int lpx_two_phase_solve_batched_dev(int count, int m, int n, int sense, IntPtr A,
+            IntPtr rel, IntPtr b, IntPtr c, ref LpxOptions opt, IntPtr status, IntPtr phase1_pivots, IntPtr n_pivots,
+            IntPtr pivots, int pivots_cap, IntPtr basis, IntPtr x, IntPtr z, IntPtr tableau, IntPtr total_pivots,
+            IntPtr stream);
         // One query against an OPTIMAL session, on the whole GPU (host buffers, synchronous; the base is only read);
         // opt IntPtr.Zero = the base's options (stream_block: breakpoints per HBM pass).  Any output but end may be null.
         [DllImport(Lib)]

@@ -21,6 +21,7 @@ enum Slot {
     WS_RO_REC, WS_RO_PAY, WS_RO_SRC, WS_RO_BASE_T, WS_RO_BASE_I,  // re-optimization: records, payloads, base
     WS_CUT_INT, WS_CUT_DBL, WS_CUT_STORE,  // cutting plane: integer / double outputs, the cut store without one
     WS_PM_INT, WS_PM_DBL,  // parametric analysis: integer / double inputs and outputs of lpx_parametric
+    WS_TP_INT, WS_TP_DBL,  // two-phase Simplex: integer / double outputs of lpx_two_phase_solve_batched
     WS_BB_SET0,  // pipelined B&B: descriptors, results, scratch of each of LPX_BB_SETS evaluation sets
     WS_COUNT = WS_BB_SET0 + 3 * 4
 };

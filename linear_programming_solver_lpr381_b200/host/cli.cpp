@@ -11,6 +11,8 @@
 //                                           each change, re-solved warm (whatif_host.cpp; not the reference's)
 //   lpr381 --parametric "<spec>" "Primal Simplex" [input]   repeatable: appends a "Parametric" block, the optimal
 //                                           value along a RHS or cost direction (parametric_host.cpp; not the reference's)
+//   lpr381 --two-phase [input]               this project's "Two-Phase Simplex" block: models with '>=' rows, '=' rows
+//                                           and negative right-hand sides (two_phase_host.cpp; not the reference's)
 #include <cstdio>
 #include <fstream>
 #include <iostream>
@@ -23,13 +25,14 @@ using namespace lpr381;
 
 int main(int argc, char** argv) {
     int arg = 1;
-    bool as_export = false, sensitivity = false, bad_what_if = false;
+    bool as_export = false, sensitivity = false, bad_what_if = false, two_phase = false;
     std::vector<std::string> what_if, parametric;
     for (; arg < argc; arg++) {
         const std::string a = argv[arg];
         if (a == "--export") as_export = true;
         else if (a == "--crlf") NewLine() = "\r\n";
         else if (a == "--sensitivity") sensitivity = true;
+        else if (a == "--two-phase") two_phase = true;
         else if (a == "--what-if") {
             if (++arg < argc) what_if.push_back(argv[arg]);
             else bad_what_if = true;
@@ -38,9 +41,34 @@ int main(int argc, char** argv) {
             else bad_what_if = true;
         } else break;
     }
+    if (two_phase) {
+        if (sensitivity || !what_if.empty() || !parametric.empty() || bad_what_if || as_export || argc - arg > 1) {
+            std::fprintf(stderr, "usage: lpr381 [--crlf] --two-phase [input.txt]  (no algorithm, no other analysis)\n");
+            return 2;
+        }
+        std::stringstream in;
+        if (arg < argc) {
+            std::ifstream f(argv[arg]);
+            if (!f) {
+                std::fprintf(stderr, "Error reading file: %s\n", argv[arg]);
+                return 2;
+            }
+            in << f.rdbuf();
+        } else {
+            in << std::cin.rdbuf();
+        }
+        try {
+            std::cout << TwoPhaseText(LPParser::ParseFromText(in.str()));
+        } catch (const LpException& e) {
+            std::fprintf(stderr, "Error: %s\n", e.what());
+            return 1;
+        }
+        return 0;
+    }
     if (arg >= argc || bad_what_if) {
         std::fprintf(stderr, "usage: lpr381 [--export] [--crlf] [--sensitivity] [--what-if \"<spec>\"]... \"<algorithm>\" "
                              "[input.txt]\n"
+                             "       lpr381 [--crlf] --two-phase [input.txt]\n"
                              "  --sensitivity (\"Primal Simplex\" only): this project's sensitivity report, not the "
                              "reference's\n"
                              "  --what-if (\"Primal Simplex\" only): rhs <i> <b_i> | cost <j> <c_j> | row <constraint> | "

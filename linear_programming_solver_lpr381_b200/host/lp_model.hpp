@@ -128,6 +128,8 @@ std::string WhatIfText(const LPProblem& problem, const std::vector<std::string>&
 // `lpr381 --parametric`: the optimal value along a RHS or cost direction from the optimal Primal Simplex result
 // (parametric_host.cpp)
 std::string ParametricText(const LPProblem& problem, const std::vector<std::string>& specs);
+// `lpr381 --two-phase`: the model solved by the two-phase Simplex (two_phase_host.cpp)
+std::string TwoPhaseText(const LPProblem& problem);
 
 // Environment.NewLine of the host ("\n"; the reference's Windows build uses "\r\n")
 std::string& NewLine();

@@ -43,6 +43,43 @@ def batch_c2(count=4096, m=64, n=128, seed=1, kind="integer"):
     return A, b, c
 
 
+def batch_mixed(count=4096, m=64, n=128, seed=1, sense=1, infeasible=0.0):
+    """Two-phase Simplex workload of C2's shape: `count` LPs with '<=', '>=' and '=' rows and integer data.
+    rel (shared by the batch, about a third of each) comes from `seed`; instance k from seed * 4096 + k:
+      A U{-2..9}, except about one row in eight per LP with A U{-9..2}, so that some right-hand sides are negative;
+      x0 integer >= 0 (each entry U{1..4} with probability 1/4); b = A x0 + U{0..5} ('<='), A x0 - U{0..5} ('>='),
+      A x0 ('='): every LP is feasible at x0.
+      Bounded: Min (sense 1) with c U{1..9}, or Max (sense 0) with c U{1..9} and row 0 a '<=' row with A U{1..9}.
+      A fraction `infeasible` of the LPs gets one '>=' row equal to a '<=' row with its right-hand side 1 higher.
+    Returns (A, b, c, rel, sense)."""
+    rr = _rng(seed * 7919 + 1)
+    rel = rr.integers(0, 3, size=m).astype(np.int32)
+    rel[0] = 0
+    if m >= 3:
+        rel[1], rel[2] = 0, 1  # the pair made contradictory in infeasible instances
+    A = np.empty((count, m, n))
+    b = np.empty((count, m))
+    c = np.empty((count, n))
+    for k in range(count):
+        r = _rng(seed * 4096 + k)
+        a = r.integers(-2, 10, size=(m, n)).astype(np.float64)
+        neg = r.random(m) < 0.125
+        neg[0] = False
+        a[neg] = r.integers(-9, 3, size=(int(neg.sum()), n))
+        if sense == 0:
+            a[0] = r.integers(1, 10, size=n)
+        x0 = np.where(r.random(n) < 0.25, r.integers(1, 5, size=n), 0).astype(np.float64)
+        ax = a @ x0
+        slack = r.integers(0, 6, size=m).astype(np.float64)
+        bk = np.where(rel == 0, ax + slack, np.where(rel == 1, ax - slack, ax))
+        if m >= 3 and r.random() < infeasible:
+            a[2] = a[1]
+            bk[2] = bk[1] + 1.0
+        A[k], b[k] = a, bk
+        c[k] = r.integers(1, 10, size=n)
+    return A, b, c, rel, sense
+
+
 def large_c3(m=4096, n=8192, seed=7):
     """C3: one large dense LP, same integer generator."""
     return lp_integer(m, n, seed)
