@@ -607,7 +607,8 @@ int lpx_session_parametric(const lpx_session* base, int kind, const double* payl
  * or LPX_KERNEL_CTA_GLOBAL; any other value is LPX_E_BAD_ARGS, as are count < 0, m < 1, n < 1, a sense outside 0..1,
  * a rel value outside 0..2, a NULL A / b / c / status and pivots_cap < 0 (checked before any device work).
  * opt.threads (128 / 256 / 512) is honoured.  Scope: no sensitivity, re-optimization or parametric analysis on these
- * results (their slack layout is not the one those definitions read). */
+ * results (their slack layout is not the one those definitions read), whether they come from the batched call or from
+ * a two-phase session (below). */
 /* rows / cols of the output tableau: m + 1, n + s + 1 (rel: host pointer, nullable = all LE) */
 int lpx_two_phase_dims(int m, int n, const int* rel, int* rows, int* cols);
 /* Host buffers, strided per LP: A[count][m][n], b[count][m], c[count][n]; rel[m] shared. */
@@ -622,6 +623,33 @@ int lpx_two_phase_solve_batched_dev(int count, int m, int n, int sense, const do
                                     int* phase1_pivots, int* n_pivots, int* pivots, int pivots_cap, int* basis,
                                     double* x, double* z, double* tableau, unsigned long long* total_pivots,
                                     void* stream);
+/* Two-phase session: one LP whose two-phase tableau ((m + 2) x W doubles) lives in HBM, for models too large for one
+ * CTA, stepped with the session calls.  The same definition, bit for bit with the batched call and the oracle at every
+ * K, pass variant and split of the work into steps.  One CTA decides up to K pivots per launch (Phase I, drive-out and
+ * Phase II rules), then one HBM pass applies them.  Open is synchronous.  NULL (lpx_last_error() says why), before any
+ * device work, for m < 1, n < 1, a sense outside 0..1, a NULL A / b / c or a rel value outside 0..2 (rel NULL: all LE).
+ * opt.max_iterations counts the pivots of both phases; opt.stream_block is K, the pivots decided per HBM pass (0 means
+ * 8, at most 16); opt.stream_pass_variant picks the blocked pass.  The session has one protocol: opt.stream_protocol,
+ * opt.kernel and opt.threads are not read.  On a two-phase session:
+ *   step / step_async / sync   LPX_RUNNING until the end, then LPX_OPTIMAL, LPX_UNBOUNDED, LPX_INFEASIBLE or
+ *                              LPX_S_ITER_LIMIT; pivots_total counts every pivot, drive-out included.  sync reports a
+ *                              terminal status as soon as no further pivot is needed.
+ *   lpx_session_dims           lpx_two_phase_dims: (m + 1, n + s + 1).
+ *   read_tableau               rows 0..m: the columns 0..n+s-1, then the RHS, compact (the batched call's tableau).
+ *   read_solution              basis[m] in internal column numbers (an artificial can stay basic in a redundant row),
+ *                              x[n], z = T[m][W-1].
+ *   read_pivots                holds up to max_iterations + m pairs (drive-out pivots can go past the limit).
+ *   silent_pivots              0.  lpx_session_profile and close work as on any session.
+ *   sensitivity / parametric   LPX_E_BAD_ARGS; lpx_session_reoptimize returns NULL. */
+lpx_session* lpx_two_phase_session_open(int m, int n, int sense, const double* A, const int* rel, const double* b,
+                                        const double* c, const lpx_options* opt);
+/* A, b, c are DEVICE pointers, rel a host pointer; b is read back once (normalisation and column numbering). */
+lpx_session* lpx_two_phase_session_open_dev(int m, int n, int sense, const double* A, const int* rel,
+                                            const double* b, const double* c, const lpx_options* opt);
+/* phase: 0 for a session that is not two-phase; 1 until the feasibility test has passed (INFEASIBLE and a Phase I
+ * iteration limit leave it at 1); 2 from then on.  phase1_pivots: Phase I pivots so far, drive-out pivots included.
+ * As of the session's enqueued work (synchronises its stream). */
+int lpx_session_two_phase_info(lpx_session* s, int* phase, int* phase1_pivots);
 
 /* ---- measurement helpers (bench.py) --------------------------------------------------------- */
 /* Unfused FP64 rate (separate DMUL and DADD, the only arithmetic the bit-exactness contract

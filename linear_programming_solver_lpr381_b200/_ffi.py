@@ -40,7 +40,8 @@ EXPORTS = [
     "lpx_dual_session_open_dev", "lpx_session_silent_pivots", "lpx_cutting_plane_dims", "lpx_cutting_plane_batched",
     "lpx_cutting_plane_batched_dev", "lpx_param_payload_stride", "lpx_param_segment_stride", "lpx_parametric_dims",
     "lpx_parametric_batched_dev", "lpx_parametric", "lpx_session_parametric", "lpx_two_phase_dims",
-    "lpx_two_phase_solve_batched", "lpx_two_phase_solve_batched_dev",
+    "lpx_two_phase_solve_batched", "lpx_two_phase_solve_batched_dev", "lpx_two_phase_session_open",
+    "lpx_two_phase_session_open_dev", "lpx_session_two_phase_info",
 ]
 
 
@@ -114,10 +115,12 @@ def lib():
                                    C.c_void_p]
     L.lpx_session_open_dev.restype = C.c_void_p
     L.lpx_session_open_dev.argtypes = L.lpx_session_open.argtypes
-    for f in ("lpx_dual_session_open", "lpx_dual_session_open_dev"):
+    for f in ("lpx_dual_session_open", "lpx_dual_session_open_dev", "lpx_two_phase_session_open",
+              "lpx_two_phase_session_open_dev"):
         getattr(L, f).restype = C.c_void_p
         getattr(L, f).argtypes = L.lpx_session_open.argtypes
     L.lpx_session_silent_pivots.argtypes = [C.c_void_p, _ip]
+    L.lpx_session_two_phase_info.argtypes = [C.c_void_p, _ip, _ip]
     L.lpx_session_stream.restype = C.c_void_p
     L.lpx_session_stream.argtypes = [C.c_void_p]
     for f in ("lpx_session_step",):

@@ -443,22 +443,29 @@ def two_phase_solve_batched_dev(count, m, n, sense, dA, drel, db, dc, dstatus, d
 class Session:
     """Large single LP whose tableau lives in HBM (lpx_session_*).  dual=True: DualSimplex.Solve on the model
     (lpx_dual_session_open); the silent ForceDualFeasibility pivots run inside the constructor and `.silent` counts
-    them.  A Dual Simplex session has no sensitivity report and cannot be a re-optimization base."""
+    them.  A Dual Simplex session has no sensitivity report and cannot be a re-optimization base.  two_phase=True: the
+    two-phase Simplex on a model with '>=' rows, '=' rows and negative right-hand sides (lpx_two_phase_session_open);
+    `.rows` x `.cols` is its output tableau, (m + 1) x (n + s + 1), and `two_phase_info()` its progress.  It has no
+    sensitivity report, parametric analysis or re-optimization."""
 
     def __init__(self, A, b, c, rel=None, sense=0, max_iterations=10000, device_ptrs=False, m=None, n=None,
-                 single_cta_select=0, kblock=0, pass_variant=0, dual=False):
+                 single_cta_select=0, kblock=0, pass_variant=0, dual=False, two_phase=False):
+        if dual and two_phase:
+            raise ValueError("a session is either dual=True or two_phase=True, not both")
         opt = F.make_options(max_iterations, single_cta_select=single_cta_select, kblock=kblock,
                              pass_variant=pass_variant)
         L = F.lib()
         if device_ptrs:
             self.m, self.n = m, n
             relp = None if rel is None else np.ascontiguousarray(rel, dtype=np.int32)
-            open_dev = L.lpx_dual_session_open_dev if dual else L.lpx_session_open_dev
+            open_dev = (L.lpx_two_phase_session_open_dev if two_phase else
+                        L.lpx_dual_session_open_dev if dual else L.lpx_session_open_dev)
             self._h = open_dev(m, n, sense, F.ptr(A), F.ptr(relp), F.ptr(b), F.ptr(c), C.cast(C.byref(opt), C.c_void_p))
         else:
             A, b, c, rel = _prep(A, b, c, rel)
             self.m, self.n = A.shape
-            open_host = L.lpx_dual_session_open if dual else L.lpx_session_open
+            open_host = (L.lpx_two_phase_session_open if two_phase else
+                         L.lpx_dual_session_open if dual else L.lpx_session_open)
             self._h = open_host(self.m, self.n, sense, F.ptr(A), F.ptr(rel), F.ptr(b), F.ptr(c),
                                 C.cast(C.byref(opt), C.c_void_p))
         if not self._h:
@@ -469,6 +476,14 @@ class Session:
         silent = C.c_int()
         F.check(L.lpx_session_silent_pivots(self._h, C.byref(silent)))
         self.dual, self.silent = dual, silent.value
+        self.two_phase = two_phase
+
+    def two_phase_info(self):
+        """(phase, phase1_pivots) as of the enqueued work: phase 0 for a session that is not two-phase, 1 until the
+        feasibility test has passed, 2 from then on; phase1_pivots counts the drive-out pivots too."""
+        ph, p1 = C.c_int(), C.c_int()
+        F.check(F.lib().lpx_session_two_phase_info(self._h, C.byref(ph), C.byref(p1)))
+        return ph.value, p1.value
 
     def step(self, max_pivots):
         st, tot = C.c_int(), C.c_int()
@@ -516,7 +531,7 @@ class Session:
             raise F.LpxError(F.E_BAD_ARGS, F.last_error())
         q = Session.__new__(Session)
         q._h = h
-        q.dual, q.silent = False, 0
+        q.dual, q.silent, q.two_phase = False, 0, False
         q.m = self.m + (kind == F.REOPT_ROW)
         q.n = self.n + (kind == F.REOPT_COL)
         r, cc = C.c_int(), C.c_int()

@@ -174,6 +174,15 @@ namespace Linear_Programming_Solver.Models
             IntPtr rel, IntPtr b, IntPtr c, ref LpxOptions opt, IntPtr status, IntPtr phase1_pivots, IntPtr n_pivots,
             IntPtr pivots, int pivots_cap, IntPtr basis, IntPtr x, IntPtr z, IntPtr tableau, IntPtr total_pivots,
             IntPtr stream);
+        // Two-phase session: one LP whose two-phase tableau lives in HBM, stepped with the lpx_session_* calls.
+        [DllImport(Lib)]
+        public static extern IntPtr lpx_two_phase_session_open(int m, int n, int sense, double[] A, int[] rel,
+            double[] b, double[] c, ref LpxOptions opt);
+        [DllImport(Lib)]
+        public static extern IntPtr lpx_two_phase_session_open_dev(int m, int n, int sense, IntPtr A, int[] rel,
+            IntPtr b, IntPtr c, ref LpxOptions opt);
+        [DllImport(Lib)]
+        public static extern int lpx_session_two_phase_info(IntPtr s, out int phase, out int phase1_pivots);
         // One query against an OPTIMAL session, on the whole GPU (host buffers, synchronous; the base is only read);
         // opt IntPtr.Zero = the base's options (stream_block: breakpoints per HBM pass).  Any output but end may be null.
         [DllImport(Lib)]

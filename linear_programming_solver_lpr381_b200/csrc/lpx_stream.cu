@@ -483,6 +483,7 @@ __global__ void __launch_bounds__(256, 4) stream_update_kernel(StreamParams P) {
 #include "lpx_stream_reopt.cuh"
 #include "lpx_stream_dual.cuh"
 #include "lpx_stream_param.cuh"
+#include "lpx_stream_twophase.cuh"
 
 
 // ---- session object -----------------------------------------------------------------------------
@@ -521,6 +522,11 @@ struct lpx_session {
     dim3 grid_pipe;
     int rpc_pipe = 0;
     int device = 0;
+    // two-phase session (lpx_two_phase_session_open): its look-ahead and the compact output width n + s
+    bool two_phase = false;
+    TwoPhaseLa tla{};
+    size_t tla_smem = 0;
+    int tp_ns = 0;
 };
 
 namespace lpx {
@@ -583,7 +589,9 @@ static size_t lookahead_cluster_smem(const StreamParams& P) {
 }
 
 static void launch_lookahead(lpx_session* s, int budget) {
-    if (s->dual)
+    if (s->two_phase)
+        stream_two_phase_lookahead_kernel<<<1, 1024, s->tla_smem, s->stream>>>(s->P, s->tla, budget);
+    else if (s->dual)
         stream_dual_lookahead_kernel<<<1, 1024, dual_lookahead_smem(s->P), s->stream>>>(s->P, budget);
     else if (s->la_cluster)
         stream_lookahead_cluster_kernel<<<LPX_LA_CLUSTER, LPX_LA_THREADS, lookahead_cluster_smem(s->P), s->stream>>>(
@@ -749,9 +757,10 @@ static int launch_block(lpx_session* s, int budget) {
 // blocked pass) or, for stream_protocol 1 / 2 or when its carve does not fit, the per-pivot protocol
 // (stream_dual_select_kernel + stream_update_kernel<4>); otherwise opt's Primal Simplex protocol.  m_in / n: the
 // model's constraints and variables (b, c).  xcol / xrow: room for one more column past the width (ld) or one more
-// row below the z-row (rows, colstride): the direction column g / row h of a parametric working session.
+// row below the z-row (rows, colstride): the direction column g / row h of a parametric working session.  xlog: room
+// for that many more pairs in the pivot log.
 static lpx_session* session_new(int m_in, int n, int sense, int mm, const lpx_options* opt, bool dual, int xcol = 0,
-                                int xrow = 0) {
+                                int xrow = 0, int xlog = 0) {
     lpx_session* s = new lpx_session();
     lpx_default_options(&s->opt);
     if (opt) s->opt = *opt;
@@ -775,7 +784,7 @@ static lpx_session* session_new(int m_in, int n, int sense, int mm, const lpx_op
     P.ld = (P.width + xcol + 15) & ~15;
     P.colstride = (P.rows + 15) & ~15;
     P.max_iter = dual ? LPX_DUAL_MAX_ITER : s->opt.max_iterations;
-    P.pivlog_cap = std::max(1, std::min(P.max_iter, 1 << 20)) + (dual ? LPX_DUAL_SILENT_MAX : 0);
+    P.pivlog_cap = std::max(1, std::min(P.max_iter, 1 << 20)) + (dual ? LPX_DUAL_SILENT_MAX : 0) + xlog;
     const size_t tbytes = (size_t)P.rows * P.ld * 8;
     P.T = (double*)sess_alloc(s, tbytes);
     P.colbuf = (double*)sess_alloc(s, (size_t)2 * P.colstride * 8);
@@ -1151,9 +1160,27 @@ static lpx_session* session_reoptimize(const lpx_session* base, int kind, const 
     return s;
 }
 
-// Where the parametric look-ahead keeps its vectors: in dynamic shared memory, in the order below, each one that fits
-// next to those placed before it; the others in global memory (`scratch`, 2 ld + 3 colstride doubles, which L2
-// holds).  Every shape runs: at worst every vector is in global memory.  Returns the dynamic shared-memory bytes.
+// Where a single-CTA look-ahead keeps its vectors: in dynamic shared memory, in the order given, each one that fits next
+// to those placed before it; the others in global memory (`scratch`, every vector's home back to back in that order,
+// which L2 holds).  Every shape runs: at worst every vector is in global memory.  Returns the dynamic shared-memory
+// bytes.
+static size_t vec_place(const size_t* len, const int* order, int nv, double* scratch, double** gvec, int* soff) {
+    const size_t cap = ((size_t)max_smem_optin() - 4096) / 8;  // 4 KB for the kernel's static shared memory
+    size_t used = 0, g = 0;
+    for (int k = 0; k < nv; k++) {
+        const int v = order[k];
+        gvec[v] = scratch + g;
+        g += len[v];
+        soff[v] = -1;
+        if (used + len[v] <= cap) {
+            soff[v] = (int)used;
+            used += len[v];
+        }
+    }
+    return used * 8;
+}
+
+// The parametric look-ahead's vectors (scratch: 2 ld + 3 colstride doubles).
 static size_t param_place(const StreamParams& P, bool cost, double* scratch, ParamLa& A) {
     size_t len[PV_N];
     len[PV_Z] = P.ld;
@@ -1162,18 +1189,7 @@ static size_t param_place(const StreamParams& P, bool cost, double* scratch, Par
     len[PV_COL] = P.colstride;
     len[PV_RATIO] = cost ? P.colstride : P.ld;
     const int order[PV_N] = {PV_RHS, PV_COL, PV_HG, PV_RATIO, PV_Z};
-    const size_t cap = ((size_t)max_smem_optin() - 4096) / 8;  // 4 KB for the kernel's static shared memory
-    size_t used = 0, g = 0;
-    for (int v : order) {
-        A.gvec[v] = scratch + g;
-        g += len[v];
-        A.soff[v] = -1;
-        if (used + len[v] <= cap) {
-            A.soff[v] = (int)used;
-            used += len[v];
-        }
-    }
-    return used * 8;
+    return vec_place(len, order, PV_N, scratch, A.gvec, A.soff);
 }
 
 // lpx_session_parametric with its arguments checked.  A working session of the working shape (RHS: ld with room for
@@ -1312,6 +1328,88 @@ static int session_parametric(const lpx_session* base, int kind, const double* p
     return LPX_OK;
 }
 
+// lpx_two_phase_session_open(_dev) with its arguments checked.  A, b, c: device pointers valid until this returns
+// (setup runs synchronously); rel, hb: host.  The normalisation, the column numbering, a, W and S come from rel and b on
+// the host; the session has m + 2 rows of width W and always runs the two-phase look-ahead with the blocked pass.
+static lpx_session* session_two_phase(int m, int n, int sense, const double* dA, const int* rel, const double* db,
+                                      const double* dc, const double* hb, const lpx_options* opt) {
+    std::vector<int> info((size_t)4 * m);  // flip | slk | art | the artificial rows in row order
+    int* flip = info.data();
+    int *slk = flip + m, *art = slk + m, *arows = art + m;
+    int ns = n;
+    for (int i = 0; i < m; i++) ns += (rel && rel[i] == 2) ? 0 : 1;
+    int sk = n, a = 0;
+    double S = 0.0;
+    for (int i = 0; i < m; i++) {
+        const int rl = rel ? rel[i] : 0;
+        flip[i] = hb[i] < 0.0;
+        const int rn = (flip[i] && rl != 2) ? 1 - rl : rl;
+        slk[i] = rl != 2 ? sk++ : -1;
+        art[i] = -1;
+        if (rn != 0) {
+            art[i] = ns + a;
+            arows[a++] = i;
+            S += flip[i] ? -hb[i] : hb[i];
+        }
+    }
+    const int W = ns + a + 1;
+    lpx_options o;
+    lpx_default_options(&o);
+    if (opt) o = *opt;
+    o.stream_protocol = 4;  // blocked, not pipelined: session_new allocates no second tableau and no L2 window
+    // W - (n + m + 1) >= 0 more columns: every EQ row has an artificial, so s + a >= m
+    lpx_session* s = session_new(m, n, sense, m, &o, false, W - (n + m + 1), 1, m);
+    if (!s) return nullptr;
+    s->two_phase = true;
+    s->sens_ok = false;
+    s->tp_ns = ns;
+    StreamParams& P = s->P;
+    P.width = W;
+    P.kblock = o.stream_block > 0 ? std::min(o.stream_block, LPX_BLOCK_KMAX) : 8;
+    size_block_pass(P, o.stream_pass_variant, &s->rpc_block, &s->grid_block);
+    double* dvec = (double*)sess_alloc(s, ((size_t)P.ld + 3 * (size_t)P.colstride) * 8);
+    TwoPhaseState* dstate = (TwoPhaseState*)sess_alloc(s, sizeof(TwoPhaseState));
+    int* dinfo = (int*)sess_alloc(s, info.size() * 4);
+    if (!dvec || !dstate || !dinfo) {
+        sess_free(s);
+        return nullptr;
+    }
+    size_t len[TV_N];
+    len[TV_Z] = P.ld;
+    len[TV_RHS] = P.colstride;
+    len[TV_COL] = P.colstride;
+    len[TV_RATIO] = P.colstride;
+    const int order[TV_N] = {TV_RHS, TV_COL, TV_RATIO, TV_Z};
+    s->tla_smem = vec_place(len, order, TV_N, dvec, s->tla.gvec, s->tla.soff);
+    s->tla.st = dstate;
+    s->tla.ns = ns;
+    const TwoPhaseRows R{dinfo, dinfo + m, dinfo + 2 * m, dinfo + 3 * m, a};
+    TwoPhaseState h0{};
+    h0.phase = 1;
+    h0.S = S;
+    cudaStream_t st = s->stream;
+    bool ok = cudaFuncSetAttribute(stream_two_phase_lookahead_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   (int)s->tla_smem) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(dinfo, info.data(), info.size() * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(dstate, &h0, sizeof h0, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    if (ok) {
+        // validate with no constraints only resets StreamCtl to RUNNING, 0 pivots, no entering column
+        stream_validate_kernel<<<1, 1024, 0, st>>>(P.ctl, nullptr, 0, INT_MAX);
+        const int strips = (P.ld + 255) / 256;
+        const int groups = std::max(1, std::min(P.rows, sm_count() * 8 / strips));
+        stream_two_phase_build_kernel<<<dim3(strips, groups, 1), 256, 0, st>>>(P, dA, db, dc, R, sense, ns);
+        stream_gather_kernel<<<(P.rows + 255) / 256, 256, 0, st>>>(P);  // the compact RHS
+        count_launch(3);
+        ok = cudaGetLastError() == cudaSuccess && cudaStreamSynchronize(st) == cudaSuccess;
+    }
+    if (!ok) {
+        cuda_fail(cudaGetLastError(), "lpx_two_phase_session_open: setup", __FILE__, __LINE__);
+        sess_free(s);
+        return nullptr;
+    }
+    return s;
+}
+
 int stream_solve_host(int m, int n, int sense, const double* A, const int* rel, const double* b, const double* c,
                       const lpx_options* opt, int* status, int* n_pivots, int* pivots, int pivots_cap, int* basis,
                       double* x, double* z, double* tableau, double* history, int history_cap) {
@@ -1414,6 +1512,61 @@ lpx_session* lpx_dual_session_open(int m, int n, int sense, const double* A, con
     return s;
 }
 
+lpx_session* lpx_two_phase_session_open_dev(int m, int n, int sense, const double* A, const int* rel, const double* b,
+                                            const double* c, const lpx_options* opt) {
+    if (!dual_open_args_ok("lpx_two_phase_session_open_dev", m, n, sense, A, rel, b, c)) return nullptr;
+    if (ensure_device() != LPX_OK) return nullptr;
+    std::lock_guard<std::recursive_mutex> lk(rt().mu);
+    // the normalisation and the column numbering need b on the host
+    std::vector<double> hb(m);
+    cudaStream_t st = rt().stream;
+    if (cudaMemcpyAsync(hb.data(), b, (size_t)m * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess) {
+        cuda_fail(cudaGetLastError(), "lpx_two_phase_session_open_dev: reading b", __FILE__, __LINE__);
+        return nullptr;
+    }
+    return session_two_phase(m, n, sense, A, rel, b, c, hb.data(), opt);
+}
+
+lpx_session* lpx_two_phase_session_open(int m, int n, int sense, const double* A, const int* rel, const double* b,
+                                        const double* c, const lpx_options* opt) {
+    if (!dual_open_args_ok("lpx_two_phase_session_open", m, n, sense, A, rel, b, c)) return nullptr;
+    if (ensure_device() != LPX_OK) return nullptr;
+    std::lock_guard<std::recursive_mutex> lk(rt().mu);
+    double *dA = nullptr, *db = nullptr, *dc = nullptr;
+    lpx_session* s = nullptr;
+    cudaStream_t st = rt().stream;
+    if (cudaMalloc(&dA, (size_t)m * n * 8) == cudaSuccess && cudaMalloc(&db, (size_t)m * 8) == cudaSuccess &&
+        cudaMalloc(&dc, (size_t)n * 8) == cudaSuccess &&
+        cudaMemcpyAsync(dA, A, (size_t)m * n * 8, cudaMemcpyHostToDevice, st) == cudaSuccess &&
+        cudaMemcpyAsync(db, b, (size_t)m * 8, cudaMemcpyHostToDevice, st) == cudaSuccess &&
+        cudaMemcpyAsync(dc, c, (size_t)n * 8, cudaMemcpyHostToDevice, st) == cudaSuccess &&
+        cudaStreamSynchronize(st) == cudaSuccess) {
+        s = session_two_phase(m, n, sense, dA, rel, db, dc, b, opt);
+    } else {
+        cuda_fail(cudaGetLastError(), "lpx_two_phase_session_open: staging inputs", __FILE__, __LINE__);
+    }
+    cudaFree(dA);
+    cudaFree(db);
+    cudaFree(dc);
+    return s;
+}
+
+int lpx_session_two_phase_info(lpx_session* s, int* phase, int* phase1_pivots) {
+    if (!s) {
+        set_error("lpx_session_two_phase_info: null session");
+        return LPX_E_BAD_ARGS;
+    }
+    TwoPhaseState h{};
+    if (s->two_phase) {
+        LPX_CUDA(cudaMemcpyAsync(&h, s->tla.st, sizeof h, cudaMemcpyDeviceToHost, s->stream));
+        LPX_CUDA(cudaStreamSynchronize(s->stream));
+    }
+    if (phase) *phase = h.phase;
+    if (phase1_pivots) *phase1_pivots = h.p1;
+    return LPX_OK;
+}
+
 int lpx_session_silent_pivots(const lpx_session* s, int* silent) {
     if (!s || !silent) {
         set_error("lpx_session_silent_pivots: bad arguments");
@@ -1462,6 +1615,11 @@ lpx_session* lpx_session_reoptimize(const lpx_session* base, int kind, const dou
         set_error("lpx_session_reoptimize: bad arguments (NULL base or payload, or an unknown kind)");
         return nullptr;
     }
+    if (base->two_phase) {
+        set_error("lpx_session_reoptimize: the base is a two-phase session (its slack layout is not the one "
+                  "re-optimization reads); re-optimization is defined for Primal Simplex results");
+        return nullptr;
+    }
     if (kind == LPX_REOPT_ROW && payload[base->n] != 0.0 && payload[base->n] != 1.0) {
         set_error("lpx_session_reoptimize: the added row's rel must be 0 (<=) or 1 (>=)");
         return nullptr;
@@ -1476,6 +1634,11 @@ int lpx_session_parametric(const lpx_session* base, int kind, const double* payl
                            int* seg_pivots, int* basis, double* tableau) {
     if (!base || !payload || !end || (kind != LPX_PARAM_RHS && kind != LPX_PARAM_COST) || seg_cap < 1) {
         set_error("lpx_session_parametric: bad arguments (NULL base, payload or end, an unknown kind, or seg_cap < 1)");
+        return LPX_E_BAD_ARGS;
+    }
+    if (base->two_phase) {
+        set_error("lpx_session_parametric: the base is a two-phase session (its slack layout is not the one parametric "
+                  "analysis reads); parametric analysis is defined for Primal Simplex results");
         return LPX_E_BAD_ARGS;
     }
     if (!(payload[lpx_param_payload_stride(kind, base->m_in, base->n) - 1] >= 0.0)) {
@@ -1607,8 +1770,8 @@ void* lpx_session_stream(lpx_session* s) { return s ? (void*)s->stream : nullptr
 
 int lpx_session_dims(const lpx_session* s, int* rows, int* cols) {
     if (!s) return LPX_E_BAD_ARGS;
-    if (rows) *rows = s->P.rows;
-    if (cols) *cols = s->P.width;
+    if (rows) *rows = s->two_phase ? s->P.m + 1 : s->P.rows;  // two-phase: lpx_two_phase_dims
+    if (cols) *cols = s->two_phase ? s->tp_ns + 1 : s->P.width;
     return LPX_OK;
 }
 
@@ -1621,6 +1784,16 @@ int lpx_session_read_tableau(lpx_session* s, double* tableau) {
         LPX_CUDA(cudaStreamSynchronize(s->stream));
         if (pipe_current_buffer(s, h)) Tcur = s->P.T1;
     }
+    if (s->two_phase) {
+        // rows 0..m: the columns 0..n+s-1, then the RHS (column W - 1), compact
+        const size_t oc = (size_t)s->tp_ns + 1, pitch = (size_t)s->P.ld * 8;
+        LPX_CUDA(cudaMemcpy2DAsync(tableau, oc * 8, Tcur, pitch, (size_t)s->tp_ns * 8, s->P.m + 1,
+                                   cudaMemcpyDeviceToHost, s->stream));
+        LPX_CUDA(cudaMemcpy2DAsync(tableau + s->tp_ns, oc * 8, Tcur + s->P.width - 1, pitch, 8, s->P.m + 1,
+                                   cudaMemcpyDeviceToHost, s->stream));
+        LPX_CUDA(cudaStreamSynchronize(s->stream));
+        return LPX_OK;
+    }
     LPX_CUDA(cudaMemcpy2DAsync(tableau, (size_t)s->P.width * 8, Tcur, (size_t)s->P.ld * 8, (size_t)s->P.width * 8,
                                s->P.rows, cudaMemcpyDeviceToHost, s->stream));
     LPX_CUDA(cudaStreamSynchronize(s->stream));
@@ -1630,6 +1803,11 @@ int lpx_session_read_tableau(lpx_session* s, double* tableau) {
 int lpx_session_sensitivity(lpx_session* s, double* report) {
     if (!s || !report) {
         set_error("lpx_session_sensitivity: bad arguments");
+        return LPX_E_BAD_ARGS;
+    }
+    if (s->two_phase) {
+        set_error("lpx_session_sensitivity: not defined for a two-phase session (its slack layout is not the one the "
+                  "report reads); the report is defined for Primal Simplex results");
         return LPX_E_BAD_ARGS;
     }
     if (s->dual_model) {

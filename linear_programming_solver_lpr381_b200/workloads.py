@@ -80,6 +80,14 @@ def batch_mixed(count=4096, m=64, n=128, seed=1, sense=1, infeasible=0.0):
     return A, b, c, rel, sense
 
 
+def large_mixed(m=4096, n=8192, seed=5, sense=1):
+    """One large LP with '<=', '>=' and '=' rows built by batch_mixed's rules (its instance 0 at this shape): feasible
+    at an integer x0 >= 0 and bounded.  The two-phase session's workload at C3's shape.  Returns (A, b, c, rel, sense)
+    with A (m, n), b (m,), c (n,)."""
+    A, b, c, rel, sense = batch_mixed(count=1, m=m, n=n, seed=seed, sense=sense)
+    return A[0], b[0], c[0], rel, sense
+
+
 def large_c3(m=4096, n=8192, seed=7):
     """C3: one large dense LP, same integer generator."""
     return lp_integer(m, n, seed)
