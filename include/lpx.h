@@ -606,9 +606,10 @@ int lpx_session_parametric(const lpx_session* base, int kind, const double* payl
  * (m + 2) x (n + s + m + 1), fits, else in global memory), LPX_KERNEL_CTA_SMEM (LPX_E_CAPACITY when it does not fit)
  * or LPX_KERNEL_CTA_GLOBAL; any other value is LPX_E_BAD_ARGS, as are count < 0, m < 1, n < 1, a sense outside 0..1,
  * a rel value outside 0..2, a NULL A / b / c / status and pivots_cap < 0 (checked before any device work).
- * opt.threads (128 / 256 / 512) is honoured.  Scope: no sensitivity, re-optimization or parametric analysis on these
- * results (their slack layout is not the one those definitions read), whether they come from the batched call or from
- * a two-phase session (below). */
+ * opt.threads (128 / 256 / 512) is honoured.  Scope: the sensitivity report of these results is the next section's
+ * ("Sensitivity analysis of a two-phase result"); the Primal Simplex report, re-optimization and parametric analysis
+ * are not defined on them (their slack layout is not the one those definitions read), whether they come from the
+ * batched call or from a two-phase session (below). */
 /* rows / cols of the output tableau: m + 1, n + s + 1 (rel: host pointer, nullable = all LE) */
 int lpx_two_phase_dims(int m, int n, const int* rel, int* rows, int* cols);
 /* Host buffers, strided per LP: A[count][m][n], b[count][m], c[count][n]; rel[m] shared. */
@@ -640,7 +641,8 @@ int lpx_two_phase_solve_batched_dev(int count, int m, int n, int sense, const do
  *                              x[n], z = T[m][W-1].
  *   read_pivots                holds up to max_iterations + m pairs (drive-out pivots can go past the limit).
  *   silent_pivots              0.  lpx_session_profile and close work as on any session.
- *   sensitivity / parametric   LPX_E_BAD_ARGS; lpx_session_reoptimize returns NULL. */
+ *   sensitivity / parametric   LPX_E_BAD_ARGS; lpx_session_reoptimize returns NULL.  The session's report is
+ *                              lpx_session_two_phase_sensitivity (next section). */
 lpx_session* lpx_two_phase_session_open(int m, int n, int sense, const double* A, const int* rel, const double* b,
                                         const double* c, const lpx_options* opt);
 /* A, b, c are DEVICE pointers, rel a host pointer; b is read back once (normalisation and column numbering). */
@@ -650,6 +652,46 @@ lpx_session* lpx_two_phase_session_open_dev(int m, int n, int sense, const doubl
  * iteration limit leave it at 1); 2 from then on.  phase1_pivots: Phase I pivots so far, drive-out pivots included.
  * As of the session's enqueued work (synchronises its stream). */
 int lpx_session_two_phase_info(lpx_session* s, int* phase, int* phase1_pivots);
+
+/* ---- Sensitivity analysis of a two-phase result — NOT the reference's --------------------------------------- */
+/* Shadow prices, slacks / surpluses and RHS / cost ranges of an OPTIMAL two-phase result, for models with '>=' rows,
+ * '=' rows and negative right-hand sides.  Checked against oracle/orc_twophase.cpp bit for bit and against an
+ * independent LP solver.  Notation of the two-phase section: flip_i (b_i < 0 strictly), sigma_i = -1 if flip_i else +1;
+ * slk_i the slack column of row i (-1 for EQ), art_i its artificial column (-1 if none); ns = n + s; T the final
+ * full-width tableau (rows 0..m-1 the constraints, row m the objective in max form, RHS column W-1), basis in internal
+ * column numbers.  Every pivot updates every column, so the unit column of row i, u_i = art_i if art_i >= 0 else
+ * slk_i (the column that started as +e_i of the normalised row), holds B^-1 e_i and T[m][u_i] = y_i at the end.
+ * EPS = 1e-9; FP64 with separate multiply / add / subtract and true division; negation is an exact sign flip.
+ *   shadow[i]  = sigma_i * T[m][u_i], negated again for Min: d(objective as written)/d b_i for the model as given.
+ *   slack[i]   = beta_r if slk_i >= 0 is basic in row r, else +0 (EQ rows: +0).  The surplus of a '>=' row, the
+ *                gap of the normalised row for a flipped one; always >= 0.
+ *   rhs range  : over constraint rows r, g_r = sigma_i * T[r][u_i], beta_r = T[r][W-1], q_r = -(beta_r / g_r).
+ *                basis[r] < ns: g_r > EPS gives a lo candidate q_r, g_r < -EPS a hi candidate.  basis[r] >= ns (an
+ *                artificial left basic in a redundant row, which must stay at zero): |g_r| > EPS gives q_r to BOTH
+ *                sides.  lo = b_i + max, hi = b_i + min, with b_i the model's value; an empty side is -inf / +inf.
+ *   reduced[j] = T[m][j].
+ *   cost range : as the Primal Simplex report, over the non-basic columns k < ns (an artificial never takes part).
+ * Ties: -0.0 equals +0.0, the lowest index wins with its own value.  A result whose status is not LPX_OPTIMAL gets
+ * a record of NaNs.  On all-'<=' models with b >= 0 (no artificial, u_i = n + i, ns = W - 1) every record equals
+ * lpx_primal_solve_sensitivity_batched's bit for bit, for both senses.  Layout and stride: lpx_sensitivity_stride.
+ * Host buffers, shaped as lpx_two_phase_solve_batched without the pivot log and the tableau; every output except status
+ * and report may be NULL.  The tableaux never leave the device: the report is the solve kernel's epilogue.  opt.kernel
+ * and opt.threads as in lpx_two_phase_solve_batched (the same shared-memory fit); the same argument refusals, and a
+ * NULL report is LPX_E_BAD_ARGS, all before any device work. */
+int lpx_two_phase_solve_sensitivity_batched(int count, int m, int n, int sense, const double* A, const int* rel,
+                                            const double* b, const double* c, const lpx_options* opt, int* status,
+                                            int* phase1_pivots, int* n_pivots, int* basis, double* x, double* z,
+                                            double* report, long long* total_pivots);
+/* Same, all pointers are DEVICE pointers (rel too), asynchronous on `stream`; total_pivots as in
+ * lpx_two_phase_solve_batched_dev. */
+int lpx_two_phase_solve_sensitivity_batched_dev(int count, int m, int n, int sense, const double* A, const int* rel,
+                                                const double* b, const double* c, const lpx_options* opt, int* status,
+                                                int* phase1_pivots, int* n_pivots, int* basis, double* x, double* z,
+                                                double* report, unsigned long long* total_pivots, void* stream);
+/* Two-phase session: report is a host buffer of one stride, computed in HBM from the session's tableau, which is only
+ * read.  Synchronous, after the session's enqueued work; NaNs unless the session's status (as of its last step / sync)
+ * is LPX_OPTIMAL.  A session that is not two-phase: LPX_E_BAD_ARGS, the reason in lpx_last_error(). */
+int lpx_session_two_phase_sensitivity(lpx_session* s, double* report);
 
 /* ---- measurement helpers (bench.py) --------------------------------------------------------- */
 /* Unfused FP64 rate (separate DMUL and DADD, the only arithmetic the bit-exactness contract

@@ -41,7 +41,8 @@ EXPORTS = [
     "lpx_cutting_plane_batched_dev", "lpx_param_payload_stride", "lpx_param_segment_stride", "lpx_parametric_dims",
     "lpx_parametric_batched_dev", "lpx_parametric", "lpx_session_parametric", "lpx_two_phase_dims",
     "lpx_two_phase_solve_batched", "lpx_two_phase_solve_batched_dev", "lpx_two_phase_session_open",
-    "lpx_two_phase_session_open_dev", "lpx_session_two_phase_info",
+    "lpx_two_phase_session_open_dev", "lpx_session_two_phase_info", "lpx_two_phase_solve_sensitivity_batched",
+    "lpx_two_phase_solve_sensitivity_batched_dev", "lpx_session_two_phase_sensitivity",
 ]
 
 
@@ -172,6 +173,9 @@ def lib():
     L.lpx_two_phase_dims.argtypes = [C.c_int, C.c_int, C.c_void_p, _ip, _ip]
     L.lpx_two_phase_solve_batched.argtypes = [C.c_int] * 4 + [C.c_void_p] * 9 + [C.c_int] + [C.c_void_p] * 4 + [_llp]
     L.lpx_two_phase_solve_batched_dev.argtypes = [C.c_int] * 4 + [C.c_void_p] * 9 + [C.c_int] + [C.c_void_p] * 6
+    L.lpx_two_phase_solve_sensitivity_batched.argtypes = [C.c_int] * 4 + [C.c_void_p] * 12 + [_llp]
+    L.lpx_two_phase_solve_sensitivity_batched_dev.argtypes = [C.c_int] * 4 + [C.c_void_p] * 14
+    L.lpx_session_two_phase_sensitivity.argtypes = [C.c_void_p, C.c_void_p]
     L.lpx_session_parametric.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 8
     L.lpx_bnb_simplex_batched.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,

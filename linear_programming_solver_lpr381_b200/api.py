@@ -439,14 +439,54 @@ def two_phase_solve_batched_dev(count, m, n, sense, dA, drel, db, dc, dstatus, d
         F.ptr(dphase1), F.ptr(dnpiv), F.ptr(dpivots), pivots_cap, F.ptr(dbasis), F.ptr(dx), F.ptr(dz),
         F.ptr(dtableau), F.ptr(dtotal), F.ptr(stream or 0)))
 
+def two_phase_sensitivity_batched(A, b, c, rel=None, sense=0, max_iterations=10000, kernel=F.KERNEL_AUTO, threads=0):
+    """lpx_two_phase_solve_sensitivity_batched: two_phase_solve_batched without the pivot log and the tableaux, plus
+    the two-phase sensitivity report of every OPTIMAL LP (include/lpx.h, "Sensitivity analysis of a two-phase result";
+    NaN records for the others), computed on the GPU next to the full-width tableaux.  Returns status, phase1_pivots,
+    n_pivots, basis, x, z, total_pivots, `report` (count, 4m + 3n) and its named (count, .) views."""
+    A, b, c, rel = _prep(A, b, c, rel)
+    count, m, n = A.shape
+    opt = F.make_options(max_iterations, kernel, threads)
+    out = dict(status=np.zeros(count, np.int32), phase1_pivots=np.zeros(count, np.int32),
+               n_pivots=np.zeros(count, np.int32), basis=np.zeros((count, m), np.int32), x=np.zeros((count, n)),
+               z=np.zeros(count), report=np.zeros((count, sensitivity_stride(m, n))))
+    total = C.c_longlong()
+    F.check(F.lib().lpx_two_phase_solve_sensitivity_batched(
+        count, m, n, sense, F.ptr(A), F.ptr(rel), F.ptr(b), F.ptr(c), C.byref(opt),
+        *[F.ptr(out[k]) for k in ("status", "phase1_pivots", "n_pivots", "basis", "x", "z", "report")],
+        C.byref(total)))
+    out["total_pivots"] = total.value
+    out.update(split_sensitivity(out["report"], m, n))
+    return out
+
+
+def two_phase_sensitivity(A, b, c, rel=None, sense=0, **kw):
+    """One LP through two_phase_sensitivity_batched: the same fields without the leading count axis."""
+    A = np.asarray(A, dtype=np.float64)
+    r = two_phase_sensitivity_batched(A[None], np.asarray(b, np.float64)[None], np.asarray(c, np.float64)[None], rel,
+                                      sense, **kw)
+    return {k: (v[0] if isinstance(v, np.ndarray) else v) for k, v in r.items()}
+
+
+def two_phase_sensitivity_batched_dev(count, m, n, sense, dA, drel, db, dc, dstatus, dphase1, dnpiv, dbasis, dx, dz,
+                                      dreport, dtotal, stream, max_iterations=10000, kernel=F.KERNEL_AUTO, threads=0):
+    """lpx_two_phase_solve_sensitivity_batched_dev: raw device pointers (ints, 0 / None for the nullable ones),
+    asynchronous on `stream` (a cudaStream_t); dreport receives count x sensitivity_stride(m, n) doubles."""
+    opt = F.make_options(max_iterations, kernel, threads)
+    F.check(F.lib().lpx_two_phase_solve_sensitivity_batched_dev(
+        count, m, n, sense, F.ptr(dA), F.ptr(drel), F.ptr(db), F.ptr(dc), C.byref(opt), F.ptr(dstatus),
+        F.ptr(dphase1), F.ptr(dnpiv), F.ptr(dbasis), F.ptr(dx), F.ptr(dz), F.ptr(dreport), F.ptr(dtotal),
+        F.ptr(stream or 0)))
+
 
 class Session:
     """Large single LP whose tableau lives in HBM (lpx_session_*).  dual=True: DualSimplex.Solve on the model
     (lpx_dual_session_open); the silent ForceDualFeasibility pivots run inside the constructor and `.silent` counts
     them.  A Dual Simplex session has no sensitivity report and cannot be a re-optimization base.  two_phase=True: the
     two-phase Simplex on a model with '>=' rows, '=' rows and negative right-hand sides (lpx_two_phase_session_open);
-    `.rows` x `.cols` is its output tableau, (m + 1) x (n + s + 1), and `two_phase_info()` its progress.  It has no
-    sensitivity report, parametric analysis or re-optimization."""
+    `.rows` x `.cols` is its output tableau, (m + 1) x (n + s + 1), `two_phase_info()` its progress and
+    `two_phase_sensitivity()` its report.  It has no Primal Simplex sensitivity report, parametric analysis or
+    re-optimization."""
 
     def __init__(self, A, b, c, rel=None, sense=0, max_iterations=10000, device_ptrs=False, m=None, n=None,
                  single_cta_select=0, kblock=0, pass_variant=0, dual=False, two_phase=False):
@@ -570,6 +610,13 @@ class Session:
         named views."""
         rep = np.zeros(sensitivity_stride(self.m, self.n))
         F.check(F.lib().lpx_session_sensitivity(self._h, F.ptr(rep)))
+        return dict(report=rep, **split_sensitivity(rep, self.m, self.n))
+
+    def two_phase_sensitivity(self):
+        """lpx_session_two_phase_sensitivity: the two-phase report of this two-phase session's tableau (NaNs unless
+        its status is OPTIMAL): `report` and its named views."""
+        rep = np.zeros(sensitivity_stride(self.m, self.n))
+        F.check(F.lib().lpx_session_two_phase_sensitivity(self._h, F.ptr(rep)))
         return dict(report=rep, **split_sensitivity(rep, self.m, self.n))
 
     def pivots(self, cap):

@@ -183,6 +183,17 @@ namespace Linear_Programming_Solver.Models
             IntPtr b, IntPtr c, ref LpxOptions opt);
         [DllImport(Lib)]
         public static extern int lpx_session_two_phase_info(IntPtr s, out int phase, out int phase1_pivots);
+        // Sensitivity of two-phase results (include/lpx.h; not the reference's): lpx_sensitivity_stride doubles per
+        // LP, NaNs unless OPTIMAL.  Every output except status and report may be null.
+        [DllImport(Lib)]
+        public static extern int lpx_two_phase_solve_sensitivity_batched(int count, int m, int n, int sense,
+            double[] A, int[] rel, double[] b, double[] c, ref LpxOptions opt, int[] status, int[] phase1_pivots,
+            int[] n_pivots, int[] basis, double[] x, double[] z, double[] report, out long total_pivots);
+        [DllImport(Lib)]
+        public static extern int lpx_two_phase_solve_sensitivity_batched_dev(int count, int m, int n, int sense,
+            IntPtr A, IntPtr rel, IntPtr b, IntPtr c, ref LpxOptions opt, IntPtr status, IntPtr phase1_pivots,
+            IntPtr n_pivots, IntPtr basis, IntPtr x, IntPtr z, IntPtr report, IntPtr total_pivots, IntPtr stream);
+        [DllImport(Lib)] public static extern int lpx_session_two_phase_sensitivity(IntPtr s, double[] report);
         // One query against an OPTIMAL session, on the whole GPU (host buffers, synchronous; the base is only read);
         // opt IntPtr.Zero = the base's options (stream_block: breakpoints per HBM pass).  Any output but end may be null.
         [DllImport(Lib)]

@@ -1,6 +1,6 @@
 // lpx_sens.cu — sensitivity report kernels and their entry points: lpx_sensitivity_stride,
-// lpx_sensitivity_batched_dev (final tableaux already on the device) and the session launcher behind
-// lpx_session_sensitivity.  lpx_primal_solve_sensitivity_batched (lpx_cta.cu) runs the batched kernel per chunk.
+// lpx_sensitivity_batched_dev (final tableaux already on the device), the session launcher behind
+// lpx_session_sensitivity, and the two-phase session launcher behind lpx_session_two_phase_sensitivity.  lpx_primal_solve_sensitivity_batched (lpx_cta.cu) runs the batched kernel per chunk.
 #include <algorithm>
 #include <vector>
 
@@ -224,6 +224,90 @@ int sens_session_launch(int m, int n, int mm, size_t ld, int sense, const int* r
     sens_session_row_kernel<<<(n + 7) / 8, 256, 0, stream>>>(S);
     sens_session_col_kernel<<<dim3(cblocks, (unsigned)S.nchunks, 1), 256, 0, stream>>>(S);
     sens_session_combine_kernel<<<cblocks, 256, 0, stream>>>(S);
+    LPX_CUDA(cudaGetLastError());
+    count_launch(4);
+    return LPX_OK;
+}
+
+// ---- two-phase session: the report of "Sensitivity analysis of a two-phase result" on the full-width tableau -------
+// (objective row m, W = the session's width).  info = flip | slk | art, m ints each, as the session's open wrote them.
+
+struct TwoPhaseSensRows {
+    const int* flip;
+    const int* slk;
+    const int* art;
+    int ns;  // n + s: columns from ns to W - 2 are artificials
+};
+
+__global__ void __launch_bounds__(1024) tp_sens_rowof_kernel(SensSession S, int ns) {
+    for (int j = threadIdx.x; j < S.W; j += 1024) S.rowof[j] = j < ns ? -1 : S.m;  // never in a cost range
+    __syncthreads();
+    for (int r = threadIdx.x; r < S.mm; r += 1024) S.rowof[S.basis[r]] = r;
+}
+
+// Column pass over the unit columns u_i: thread per constraint, one chunk of chunk_rows rows per blockIdx.y.  A row
+// whose basic variable is an artificial (a redundant row) bounds both sides.
+__global__ void __launch_bounds__(256) tp_sens_col_kernel(SensSession S, TwoPhaseSensRows R) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= S.m) return;
+    const int u = R.art[i] >= 0 ? R.art[i] : R.slk[i];
+    const bool f = R.flip[i] != 0;
+    const int r0 = blockIdx.y * S.chunk_rows, r1 = min(S.mm, r0 + S.chunk_rows);
+    SensBest lo = sens_empty(), hi = sens_empty();
+    for (int r = r0; r < r1; r++) {
+        const double* Tr = S.T + (size_t)r * S.ld;
+        const double g = sens_sign(Tr[u], f);
+        if (S.basis[r] < R.ns) sens_rhs_candidate(lo, hi, Tr[S.W - 1], g, r);
+        else sens_rhs_candidate_both(lo, hi, Tr[S.W - 1], g, r);
+    }
+    SensBest* p = S.partial + 2 * ((size_t)blockIdx.y * S.m + i);
+    p[0] = lo;
+    p[1] = hi;
+}
+
+// Combine of the chunks in row order, plus shadow price and slack.
+__global__ void __launch_bounds__(256) tp_sens_combine_kernel(SensSession S, TwoPhaseSensRows R) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= S.m) return;
+    SensBest lo = sens_empty(), hi = sens_empty();
+    for (int ch = 0; ch < S.nchunks; ch++) {
+        const SensBest* p = S.partial + 2 * ((size_t)ch * S.m + i);
+        sens_pick<true>(lo, p[0]);
+        sens_pick<false>(hi, p[1]);
+    }
+    const int u = R.art[i] >= 0 ? R.art[i] : R.slk[i];
+    const double* z = S.T + (size_t)S.mm * S.ld;
+    const int rs = R.slk[i] >= 0 ? S.rowof[R.slk[i]] : -1;
+    const double slack = rs >= 0 ? S.T[(size_t)rs * S.ld + S.W - 1] : 0.0;
+    sens_write_constraint(S.report, S.m, i, S.sense, sens_sign(z[u], R.flip[i] != 0), slack, lo, hi, S.b[i]);
+}
+
+int tp_sens_session_launch(int m, int n, int ns, int W, size_t ld, int sense, const int* info, const double* b,
+                           const double* c, const int* basis, const double* T, int* rowof, void* partial,
+                           double* report, cudaStream_t stream) {
+    SensSession S;
+    S.m = m;
+    S.n = n;
+    S.mm = m;
+    S.W = W;
+    S.sense = sense;
+    S.chunk_rows = LPX_SENS_CHUNK_ROWS;
+    S.nchunks = (m + LPX_SENS_CHUNK_ROWS - 1) / LPX_SENS_CHUNK_ROWS;
+    S.ld = (int)ld;
+    S.rmap = nullptr;
+    S.b = b;
+    S.c = c;
+    S.basis = basis;
+    S.T = T;
+    S.rowof = rowof;
+    S.partial = static_cast<SensBest*>(partial);
+    S.report = report;
+    const TwoPhaseSensRows R{info, info + m, info + 2 * m, ns};
+    const unsigned cblocks = (unsigned)((m + 255) / 256);
+    tp_sens_rowof_kernel<<<1, 1024, 0, stream>>>(S, ns);
+    sens_session_row_kernel<<<(n + 7) / 8, 256, 0, stream>>>(S);
+    tp_sens_col_kernel<<<dim3(cblocks, (unsigned)S.nchunks, 1), 256, 0, stream>>>(S, R);
+    tp_sens_combine_kernel<<<cblocks, 256, 0, stream>>>(S, R);
     LPX_CUDA(cudaGetLastError());
     count_launch(4);
     return LPX_OK;

@@ -62,6 +62,23 @@ __device__ __forceinline__ void sens_rhs_candidate(SensBest& lo, SensBest& hi, d
     }
 }
 
+// Two-phase report: row r holds an artificial that stayed basic in a redundant row and must stay at zero, so a
+// direction with |g| > EPS bounds the RHS change on both sides at the same value.
+__device__ __forceinline__ void sens_rhs_candidate_both(SensBest& lo, SensBest& hi, double beta, double g, int r) {
+    if (fabs(g) > LPX_EPS) {
+        SensBest c;
+        c.v = -__ddiv_rn(beta, g);
+        c.i = r;
+        sens_pick<true>(lo, c);
+        sens_pick<false>(hi, c);
+    }
+}
+
+// sigma_i * v of the two-phase report: an exact sign flip when row i was negated (b_i < 0).
+__device__ __forceinline__ double sens_sign(double v, bool flip) {
+    return flip ? __longlong_as_double(__double_as_longlong(v) ^ (long long)0x8000000000000000ULL) : v;
+}
+
 // One non-basic column k of the cost-range row reduction of a basic variable: entry alpha of its row, reduced
 // cost d of column k.
 __device__ __forceinline__ void sens_cost_candidate(SensBest& lo, SensBest& hi, double d, double alpha, int k) {

@@ -527,6 +527,7 @@ struct lpx_session {
     TwoPhaseLa tla{};
     size_t tla_smem = 0;
     int tp_ns = 0;
+    int* tp_info = nullptr;  // device flip | slk | art (m ints each): lpx_session_two_phase_sensitivity reads them
 };
 
 namespace lpx {
@@ -1383,6 +1384,7 @@ static lpx_session* session_two_phase(int m, int n, int sense, const double* dA,
     s->tla_smem = vec_place(len, order, TV_N, dvec, s->tla.gvec, s->tla.soff);
     s->tla.st = dstate;
     s->tla.ns = ns;
+    s->tp_info = dinfo;
     const TwoPhaseRows R{dinfo, dinfo + m, dinfo + 2 * m, dinfo + 3 * m, a};
     TwoPhaseState h0{};
     h0.phase = 1;
@@ -1392,6 +1394,9 @@ static lpx_session* session_two_phase(int m, int n, int sense, const double* dA,
                                    (int)s->tla_smem) == cudaSuccess;
     ok = ok && cudaMemcpyAsync(dinfo, info.data(), info.size() * 4, cudaMemcpyHostToDevice, st) == cudaSuccess;
     ok = ok && cudaMemcpyAsync(dstate, &h0, sizeof h0, cudaMemcpyHostToDevice, st) == cudaSuccess;
+    // the model's b and c, for the sensitivity report
+    ok = ok && cudaMemcpyAsync(s->sens_b, db, (size_t)m * 8, cudaMemcpyDeviceToDevice, st) == cudaSuccess;
+    ok = ok && cudaMemcpyAsync(s->sens_c, dc, (size_t)n * 8, cudaMemcpyDeviceToDevice, st) == cudaSuccess;
     if (ok) {
         // validate with no constraints only resets StreamCtl to RUNNING, 0 pivots, no entering column
         stream_validate_kernel<<<1, 1024, 0, st>>>(P.ctl, nullptr, 0, INT_MAX);
@@ -1842,6 +1847,44 @@ int lpx_session_sensitivity(lpx_session* s, double* report) {
     const double* Tcur = (s->pipe && pipe_current_buffer(s, h)) ? P.T1 : P.T;
     int rc = sens_session_launch(s->m_in, s->n, P.m, (size_t)P.ld, s->sense, s->sens_rmap, s->sens_b, s->sens_c, P.basis,
                                  Tcur, s->sens_rowof, s->sens_partial, s->sens_report, s->stream);
+    if (rc != LPX_OK) return rc;
+    LPX_CUDA(cudaMemcpyAsync(report, s->sens_report, stride * 8, cudaMemcpyDeviceToHost, s->stream));
+    LPX_CUDA(cudaStreamSynchronize(s->stream));
+    return LPX_OK;
+}
+
+int lpx_session_two_phase_sensitivity(lpx_session* s, double* report) {
+    if (!s || !report) {
+        set_error("lpx_session_two_phase_sensitivity: bad arguments");
+        return LPX_E_BAD_ARGS;
+    }
+    if (!s->two_phase) {
+        set_error("lpx_session_two_phase_sensitivity: not a two-phase session (lpx_session_sensitivity reports on "
+                  "Primal Simplex sessions)");
+        return LPX_E_BAD_ARGS;
+    }
+    std::lock_guard<std::recursive_mutex> lk(rt().mu);
+    const StreamParams& P = s->P;
+    const size_t stride = lpx_sensitivity_stride(s->m_in, s->n);
+    StreamCtl h;
+    LPX_CUDA(cudaMemcpyAsync(&h, P.ctl, sizeof h, cudaMemcpyDeviceToHost, s->stream));
+    LPX_CUDA(cudaStreamSynchronize(s->stream));
+    if (h.status != LPX_OPTIMAL) {
+        for (size_t e = 0; e < stride; e++) report[e] = std::numeric_limits<double>::quiet_NaN();
+        return LPX_OK;
+    }
+    if (!s->sens_report) {
+        s->sens_rowof = (int*)sess_alloc(s, (size_t)P.width * 4);
+        s->sens_partial = sess_alloc(s, sens_session_partial_bytes(P.m, P.m));
+        s->sens_report = (double*)sess_alloc(s, stride * 8);
+        if (!s->sens_rowof || !s->sens_partial || !s->sens_report) {
+            s->sens_report = nullptr;
+            return LPX_E_CUDA;
+        }
+    }
+    // a two-phase session runs the blocked protocol on one tableau; it is only read here
+    int rc = tp_sens_session_launch(P.m, s->n, s->tp_ns, P.width, (size_t)P.ld, s->sense, s->tp_info, s->sens_b,
+                                    s->sens_c, P.basis, P.T, s->sens_rowof, s->sens_partial, s->sens_report, s->stream);
     if (rc != LPX_OK) return rc;
     LPX_CUDA(cudaMemcpyAsync(report, s->sens_report, stride * 8, cudaMemcpyDeviceToHost, s->stream));
     LPX_CUDA(cudaStreamSynchronize(s->stream));

@@ -42,5 +42,10 @@ size_t sens_session_partial_bytes(int m, int mm);
 int sens_session_launch(int m, int n, int mm, size_t ld, int sense, const int* rmap, const double* b, const double* c,
                         const int* basis, const double* T, int* rowof, void* partial, double* report,
                         cudaStream_t stream);
+// Two-phase session: the full-width tableau (m + 2 rows, width W, objective row m), info = flip | slk | art (m ints
+// each).  rowof: W ints, partial: sens_session_partial_bytes(m, m).
+int tp_sens_session_launch(int m, int n, int ns, int W, size_t ld, int sense, const int* info, const double* b,
+                           const double* c, const int* basis, const double* T, int* rowof, void* partial,
+                           double* report, cudaStream_t stream);
 
 }  // namespace lpx

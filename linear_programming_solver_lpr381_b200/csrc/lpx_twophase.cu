@@ -6,11 +6,16 @@
 // The loops are written here from the helpers cta_simplex_kernel uses (warp_argmin_below, cta_stage_ratios,
 // warp_margin_scan_staged, cta_pivot) rather than as a branch of that kernel, which keeps its register allocation
 // (DESIGN §4.12 gives the same reason for the cutting-plane kernel).
+//
+// two_phase_sens_kernel is the same solve with the sensitivity report of include/lpx.h ("Sensitivity analysis of a
+// two-phase result") as its epilogue, read from the full-width tableau before the CTA ends: the artificial columns
+// hold B^-1 e_i of the rows whose unit column they are, and the compact output tableau drops them.
 #include <cstring>
 #include <vector>
 
 #include "lpx_cta.cuh"
 #include "lpx_runtime.hpp"
+#include "lpx_sens.cuh"
 
 namespace lpx {
 
@@ -36,8 +41,46 @@ struct TwoPhaseBatch {
     unsigned long long* total_pivots;
 };
 
-template <int THREADS, bool SMEM_T>
-__global__ void __launch_bounds__(THREADS, 1) two_phase_kernel(const TwoPhaseBatch P) {
+// The report of one OPTIMAL LP from its final full-width tableau T (rows ld doubles apart, objective row m, RHS
+// column W - 1).  rowof takes W ints of scratch that is dead after the solve; sbasis / flip / slk / art as the solve
+// left them.  Constraints: one warp per row i, lanes over the rows r (column reduction along the unit column u_i);
+// decision variables: one warp per variable, lanes over the columns (sens_variable_warp).
+template <int THREADS>
+__device__ __forceinline__ void two_phase_report(const double* T, int ld, int m, int n, int ns, int W, int sense,
+                                                 const int* sbasis, const int* flip, const int* slk, const int* art,
+                                                 int* rowof, const double* bi, const double* ci, double* rep) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    constexpr int NW = THREADS / 32;
+    const int rhs = W - 1;
+    for (int j = tid; j < W; j += THREADS) rowof[j] = j < ns ? -1 : m;  // an artificial never enters a cost range
+    __syncthreads();
+    for (int r = tid; r < m; r += THREADS) rowof[sbasis[r]] = r;
+    __syncthreads();
+    const double* z = T + (size_t)m * ld;
+    for (int i = warp; i < m; i += NW) {
+        const int u = art[i] >= 0 ? art[i] : slk[i];
+        const bool f = flip[i] != 0;
+        SensBest lo = sens_empty(), hi = sens_empty();
+        for (int r = lane; r < m; r += 32) {
+            const double* Tr = T + (size_t)r * ld;
+            const double g = sens_sign(Tr[u], f);
+            if (sbasis[r] < ns) sens_rhs_candidate(lo, hi, Tr[rhs], g, r);
+            else sens_rhs_candidate_both(lo, hi, Tr[rhs], g, r);
+        }
+        lo = sens_warp_reduce<true>(lo);
+        hi = sens_warp_reduce<false>(hi);
+        if (lane == 0) {
+            const int rs = slk[i] >= 0 ? rowof[slk[i]] : -1;
+            const double slack = rs >= 0 ? T[(size_t)rs * ld + rhs] : 0.0;
+            sens_write_constraint(rep, m, i, sense, sens_sign(z[u], f), slack, lo, hi, bi[i]);
+        }
+    }
+    for (int j = warp; j < n; j += NW) sens_variable_warp(T, ld, W, m, n, m, j, sense, rowof, ci[j], rep);
+}
+
+// REPORT: write the sensitivity record of LP p to report + p * (4m + 3n) (NaNs unless OPTIMAL).
+template <int THREADS, bool SMEM_T, bool REPORT>
+__device__ __forceinline__ void two_phase_body(const TwoPhaseBatch& P, double* report) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     constexpr int NW = THREADS / 32;
@@ -238,12 +281,32 @@ __global__ void __launch_bounds__(THREADS, 1) two_phase_kernel(const TwoPhaseBat
             To[k] = T[(size_t)i * ld + (j < ns ? j : rhs)];
         }
     }
+    if constexpr (REPORT) {
+        double* rep = report + (size_t)p * (4 * (size_t)m + 3 * (size_t)n);
+        if (status != LPX_OPTIMAL) {
+            for (int e = tid; e < 4 * m + 3 * n; e += THREADS) rep[e] = sens_nan();
+        } else {
+            // prow (max_width + 2 doubles) is dead once the solve has stopped: rowof's W ints fit in it
+            two_phase_report<THREADS>(T, ld, m, n, ns, W, P.sense, sbasis, flip, slk, art, reinterpret_cast<int*>(prow),
+                                      bi, ci, rep);
+        }
+    }
     if (tid == 0) {
         P.status[p] = status;
         if (P.phase1) P.phase1[p] = p1;
         if (P.n_pivots) P.n_pivots[p] = n_piv;
         if (P.total_pivots && n_piv) atomicAdd(P.total_pivots, (unsigned long long)n_piv);
     }
+}
+
+template <int THREADS, bool SMEM_T>
+__global__ void __launch_bounds__(THREADS, 1) two_phase_kernel(const TwoPhaseBatch P) {
+    two_phase_body<THREADS, SMEM_T, false>(P, nullptr);
+}
+
+template <int THREADS, bool SMEM_T>
+__global__ void __launch_bounds__(THREADS, 1) two_phase_sens_kernel(const TwoPhaseBatch P, double* report) {
+    two_phase_body<THREADS, SMEM_T, true>(P, report);
 }
 
 static int slack_count(int m, const int* rel) {
@@ -271,20 +334,28 @@ static int check_args(int count, int m, int n, int sense, int pivots_cap, const 
 }
 
 template <int THREADS, bool SMEM_T>
-static int launch_two_phase_variant(const TwoPhaseBatch& P, int count, size_t smem, cudaStream_t stream) {
-    auto kfn = two_phase_kernel<THREADS, SMEM_T>;
-    LPX_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kfn<<<count, THREADS, smem, stream>>>(P);
+static int launch_two_phase_variant(const TwoPhaseBatch& P, double* report, int count, size_t smem,
+                                    cudaStream_t stream) {
+    if (report) {
+        auto kfn = two_phase_sens_kernel<THREADS, SMEM_T>;
+        LPX_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kfn<<<count, THREADS, smem, stream>>>(P, report);
+    } else {
+        auto kfn = two_phase_kernel<THREADS, SMEM_T>;
+        LPX_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kfn<<<count, THREADS, smem, stream>>>(P);
+    }
     LPX_CUDA(cudaGetLastError());
     count_launch();
     return LPX_OK;
 }
 
-// Everything on the device already; s (slack columns) known on the host, arguments checked.
+// Everything on the device already; s (slack columns) known on the host, arguments checked.  report (nullable): run the
+// report builds, whose epilogue needs no shared memory beyond the solve's carve, so the fit decision is the same.
 static int two_phase_launch(int count, int m, int n, int sense, int s, const double* A, const int* rel,
                             const double* b, const double* c, const lpx_options& o, int* status, int* phase1,
                             int* n_pivots, int* pivots, int pivots_cap, int* basis, double* x, double* z,
-                            double* tableau, unsigned long long* total_pivots, cudaStream_t stream) {
+                            double* tableau, unsigned long long* total_pivots, double* report, cudaStream_t stream) {
     // the width takes a = m artificials: a depends on each LP's b, while rel is shared by the batch
     const int rows = m + 2, max_width = n + s + m + 1;
     const bool fits = cta_fits_smem(rows, max_width);
@@ -333,13 +404,13 @@ static int two_phase_launch(int count, int m, int n, int sense, int s, const dou
     if (threads != 128 && threads != 256 && threads != 512)  // as cta_launch chooses (lpx_cta.cu)
         threads = (!smem_T || tsize >= 8192) ? 512 : 256;
     if (smem_T) {
-        if (threads == 128) return launch_two_phase_variant<128, true>(P, count, smem, stream);
-        if (threads == 256) return launch_two_phase_variant<256, true>(P, count, smem, stream);
-        return launch_two_phase_variant<512, true>(P, count, smem, stream);
+        if (threads == 128) return launch_two_phase_variant<128, true>(P, report, count, smem, stream);
+        if (threads == 256) return launch_two_phase_variant<256, true>(P, report, count, smem, stream);
+        return launch_two_phase_variant<512, true>(P, report, count, smem, stream);
     }
-    if (threads == 128) return launch_two_phase_variant<128, false>(P, count, smem, stream);
-    if (threads == 256) return launch_two_phase_variant<256, false>(P, count, smem, stream);
-    return launch_two_phase_variant<512, false>(P, count, smem, stream);
+    if (threads == 128) return launch_two_phase_variant<128, false>(P, report, count, smem, stream);
+    if (threads == 256) return launch_two_phase_variant<256, false>(P, report, count, smem, stream);
+    return launch_two_phase_variant<512, false>(P, report, count, smem, stream);
 }
 
 }  // namespace lpx
@@ -385,7 +456,7 @@ int lpx_two_phase_solve_batched_dev(int count, int m, int n, int sense, const do
         ns = slack_count(m, hrel.data());
     }
     return two_phase_launch(count, m, n, sense, ns, A, rel, b, c, o, status, phase1_pivots, n_pivots, pivots,
-                            pivots_cap, basis, x, z, tableau, total_pivots, s);
+                            pivots_cap, basis, x, z, tableau, total_pivots, nullptr, s);
 }
 
 int lpx_two_phase_solve_batched(int count, int m, int n, int sense, const double* A, const int* rel, const double* b,
@@ -429,7 +500,7 @@ int lpx_two_phase_solve_batched(int count, int m, int n, int sense, const double
     LPX_CUDA(cudaMemsetAsync(dtot, 0, 8, s));
     rc = two_phase_launch(count, m, n, sense, ns, dA, rel ? drel : nullptr, db, dc, o, dst, phase1_pivots ? dp1 : nullptr,
                           n_pivots ? dnp : nullptr, cap ? dpiv : nullptr, (int)cap, basis ? dbasis : nullptr,
-                          x ? dx : nullptr, z ? dz : nullptr, dT, dtot, s);
+                          x ? dx : nullptr, z ? dz : nullptr, dT, dtot, nullptr, s);
     if (rc != LPX_OK) return rc;
     auto down = [&](void* dst_h, const void* src, size_t bytes) {
         return dst_h ? cudaMemcpyAsync(dst_h, src, bytes, cudaMemcpyDeviceToHost, s) : cudaSuccess;
@@ -443,6 +514,94 @@ int lpx_two_phase_solve_batched(int count, int m, int n, int sense, const double
     LPX_CUDA(down(x, dx, cnt * n * 8));
     LPX_CUDA(down(z, dz, cnt * 8));
     LPX_CUDA(down(tableau, dT, cnt * tsize * 8));
+    LPX_CUDA(down(&htot, dtot, 8));
+    LPX_CUDA(cudaStreamSynchronize(s));
+    if (total_pivots) *total_pivots = (long long)htot;
+    return LPX_OK;
+}
+
+int lpx_two_phase_solve_sensitivity_batched_dev(int count, int m, int n, int sense, const double* A, const int* rel,
+                                                const double* b, const double* c, const lpx_options* opt, int* status,
+                                                int* phase1_pivots, int* n_pivots, int* basis, double* x, double* z,
+                                                double* report, unsigned long long* total_pivots, void* stream) {
+    lpx_options o;
+    lpx_default_options(&o);
+    if (opt) o = *opt;
+    int rc = check_args(count, m, n, sense, 0, nullptr, o);
+    if (rc != LPX_OK) return rc;
+    if (!A || !b || !c || !status || !report) {
+        set_error("lpx_two_phase_solve_sensitivity_batched_dev: A, b, c, status and report must not be NULL");
+        return LPX_E_BAD_ARGS;
+    }
+    if ((rc = ensure_device()) != LPX_OK) return rc;
+    std::lock_guard<std::recursive_mutex> lk(rt().mu);
+    cudaStream_t s = (cudaStream_t)stream;
+    int ns = m;
+    if (rel) {
+        std::vector<int> hrel(m);
+        LPX_CUDA(cudaMemcpyAsync(hrel.data(), rel, (size_t)m * 4, cudaMemcpyDeviceToHost, s));
+        LPX_CUDA(cudaStreamSynchronize(s));
+        if ((rc = check_args(count, m, n, sense, 0, hrel.data(), o)) != LPX_OK) return rc;
+        ns = slack_count(m, hrel.data());
+    }
+    return two_phase_launch(count, m, n, sense, ns, A, rel, b, c, o, status, phase1_pivots, n_pivots, nullptr, 0, basis,
+                            x, z, nullptr, total_pivots, report, s);
+}
+
+int lpx_two_phase_solve_sensitivity_batched(int count, int m, int n, int sense, const double* A, const int* rel,
+                                            const double* b, const double* c, const lpx_options* opt, int* status,
+                                            int* phase1_pivots, int* n_pivots, int* basis, double* x, double* z,
+                                            double* report, long long* total_pivots) {
+    lpx_options o;
+    lpx_default_options(&o);
+    if (opt) o = *opt;
+    int rc = check_args(count, m, n, sense, 0, rel, o);
+    if (rc != LPX_OK) return rc;
+    if (!A || !b || !c || !status || !report) {
+        set_error("lpx_two_phase_solve_sensitivity_batched: A, b, c, status and report must not be NULL");
+        return LPX_E_BAD_ARGS;
+    }
+    if ((rc = ensure_device()) != LPX_OK) return rc;
+    Runtime& r = rt();
+    std::lock_guard<std::recursive_mutex> lk(r.mu);
+    cudaStream_t s = r.stream;
+    if (total_pivots) *total_pivots = 0;
+    if (count == 0) return LPX_OK;
+    const int ns = slack_count(m, rel);
+    const size_t cnt = (size_t)count, stride = 4 * (size_t)m + 3 * (size_t)n;
+
+    double* dA = ws_dev_as<double>(WS_A, cnt * m * n);
+    double* db = ws_dev_as<double>(WS_B, cnt * m);
+    double* dc = ws_dev_as<double>(WS_C, cnt * n);
+    int* drel = ws_dev_as<int>(WS_REL, m);
+    // ints: status, phase1, n_pivots | basis;  doubles: x | z | report
+    int* di = ws_dev_as<int>(WS_TP_INT, 3 * cnt + cnt * m);
+    double* dd = ws_dev_as<double>(WS_TP_DBL, cnt * n + cnt + cnt * stride);
+    unsigned long long* dtot = ws_dev_as<unsigned long long>(WS_TOTAL, 1);
+    if (!dA || !db || !dc || !drel || !di || !dd || !dtot) return LPX_E_CUDA;
+    int *dst = di, *dp1 = di + cnt, *dnp = di + 2 * cnt, *dbasis = di + 3 * cnt;
+    double *dx = dd, *dz = dd + cnt * n, *drep = dz + cnt;
+
+    LPX_CUDA(cudaMemcpyAsync(dA, A, cnt * m * n * 8, cudaMemcpyHostToDevice, s));
+    LPX_CUDA(cudaMemcpyAsync(db, b, cnt * m * 8, cudaMemcpyHostToDevice, s));
+    LPX_CUDA(cudaMemcpyAsync(dc, c, cnt * n * 8, cudaMemcpyHostToDevice, s));
+    if (rel) LPX_CUDA(cudaMemcpyAsync(drel, rel, (size_t)m * 4, cudaMemcpyHostToDevice, s));
+    LPX_CUDA(cudaMemsetAsync(dtot, 0, 8, s));
+    rc = two_phase_launch(count, m, n, sense, ns, dA, rel ? drel : nullptr, db, dc, o, dst, phase1_pivots ? dp1 : nullptr,
+                          n_pivots ? dnp : nullptr, nullptr, 0, basis ? dbasis : nullptr, x ? dx : nullptr,
+                          z ? dz : nullptr, nullptr, dtot, drep, s);
+    if (rc != LPX_OK) return rc;
+    auto down = [&](void* dst_h, const void* src, size_t bytes) {
+        return dst_h ? cudaMemcpyAsync(dst_h, src, bytes, cudaMemcpyDeviceToHost, s) : cudaSuccess;
+    };
+    unsigned long long htot = 0;
+    LPX_CUDA(down(status, dst, cnt * 4));
+    LPX_CUDA(down(phase1_pivots, dp1, cnt * 4));
+    LPX_CUDA(down(n_pivots, dnp, cnt * 4));
+    LPX_CUDA(down(basis, dbasis, cnt * m * 4));
+    LPX_CUDA(down(x, dx, cnt * n * 8));
+    LPX_CUDA(down(z, dz, cnt * 8));
+    LPX_CUDA(down(report, drep, cnt * stride * 8));
     LPX_CUDA(down(&htot, dtot, 8));
     LPX_CUDA(cudaStreamSynchronize(s));
     if (total_pivots) *total_pivots = (long long)htot;

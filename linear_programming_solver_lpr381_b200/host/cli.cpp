@@ -13,6 +13,8 @@
 //                                           value along a RHS or cost direction (parametric_host.cpp; not the reference's)
 //   lpr381 --two-phase [input]               this project's "Two-Phase Simplex" block: models with '>=' rows, '=' rows
 //                                           and negative right-hand sides (two_phase_host.cpp; not the reference's)
+//   lpr381 --two-phase-sensitivity [input]   the "Two-Phase Simplex" block, then this project's "Two-Phase Sensitivity
+//                                           Analysis" block (shadow prices, slacks, ranges, b.y; sensitivity_host.cpp)
 #include <cstdio>
 #include <fstream>
 #include <iostream>
@@ -25,7 +27,7 @@ using namespace lpr381;
 
 int main(int argc, char** argv) {
     int arg = 1;
-    bool as_export = false, sensitivity = false, bad_what_if = false, two_phase = false;
+    bool as_export = false, sensitivity = false, bad_what_if = false, two_phase = false, two_phase_sens = false;
     std::vector<std::string> what_if, parametric;
     for (; arg < argc; arg++) {
         const std::string a = argv[arg];
@@ -33,6 +35,7 @@ int main(int argc, char** argv) {
         else if (a == "--crlf") NewLine() = "\r\n";
         else if (a == "--sensitivity") sensitivity = true;
         else if (a == "--two-phase") two_phase = true;
+        else if (a == "--two-phase-sensitivity") two_phase_sens = true;
         else if (a == "--what-if") {
             if (++arg < argc) what_if.push_back(argv[arg]);
             else bad_what_if = true;
@@ -41,9 +44,11 @@ int main(int argc, char** argv) {
             else bad_what_if = true;
         } else break;
     }
-    if (two_phase) {
-        if (sensitivity || !what_if.empty() || !parametric.empty() || bad_what_if || as_export || argc - arg > 1) {
-            std::fprintf(stderr, "usage: lpr381 [--crlf] --two-phase [input.txt]  (no algorithm, no other analysis)\n");
+    if (two_phase || two_phase_sens) {
+        if (sensitivity || !what_if.empty() || !parametric.empty() || bad_what_if || as_export || argc - arg > 1 ||
+            (two_phase && two_phase_sens)) {
+            std::fprintf(stderr, "usage: lpr381 [--crlf] --two-phase [input.txt]  (no algorithm, no other analysis)\n"
+                                 "       lpr381 [--crlf] --two-phase-sensitivity [input.txt]\n");
             return 2;
         }
         std::stringstream in;
@@ -58,7 +63,10 @@ int main(int argc, char** argv) {
             in << std::cin.rdbuf();
         }
         try {
-            std::cout << TwoPhaseText(LPParser::ParseFromText(in.str()));
+            const LPProblem problem = LPParser::ParseFromText(in.str());
+            std::string out = TwoPhaseText(problem);
+            if (two_phase_sens) out += NewLine() + TwoPhaseSensitivityText(problem);
+            std::cout << out;
         } catch (const LpException& e) {
             std::fprintf(stderr, "Error: %s\n", e.what());
             return 1;
@@ -69,6 +77,7 @@ int main(int argc, char** argv) {
         std::fprintf(stderr, "usage: lpr381 [--export] [--crlf] [--sensitivity] [--what-if \"<spec>\"]... \"<algorithm>\" "
                              "[input.txt]\n"
                              "       lpr381 [--crlf] --two-phase [input.txt]\n"
+                             "       lpr381 [--crlf] --two-phase-sensitivity [input.txt]\n"
                              "  --sensitivity (\"Primal Simplex\" only): this project's sensitivity report, not the "
                              "reference's\n"
                              "  --what-if (\"Primal Simplex\" only): rhs <i> <b_i> | cost <j> <c_j> | row <constraint> | "

@@ -130,6 +130,9 @@ std::string WhatIfText(const LPProblem& problem, const std::vector<std::string>&
 std::string ParametricText(const LPProblem& problem, const std::vector<std::string>& specs);
 // `lpr381 --two-phase`: the model solved by the two-phase Simplex (two_phase_host.cpp)
 std::string TwoPhaseText(const LPProblem& problem);
+// `lpr381 --two-phase-sensitivity`: the two-phase sensitivity report in SensitivityText's line formats, then the dual
+// objective b.y and the objective as written (sensitivity_host.cpp); the status message when not OPTIMAL.
+std::string TwoPhaseSensitivityText(const LPProblem& problem);
 
 // Environment.NewLine of the host ("\n"; the reference's Windows build uses "\r\n")
 std::string& NewLine();
